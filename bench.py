@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg5|cfg4|cfg3|cfg2]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   (N > 1)
   python bench.py --impl reference ...        the reference's CPU implementation on host cores
+  python bench.py ... --dump-outputs DIR      also write what the last timed step computed, DIR/<name>.npy
 
 A "step" is one hourly record advanced for every buoy of this rank (one launch of
 k_advect_step = the body of si3_part_tracker.py:378-493 incl. the lat/lon update).
@@ -25,10 +26,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree and writes nothing into it
 
 SEED_BOX = int(os.environ.get("SITRACK_BENCH_SEED_BOX", "0")) or None   # diagnostic only
 B_ALG = 83.0          # algorithmic bytes per buoy-step (SURVEY.md §8d): 25 state in + 25 out + 33 row
 D2H_PER_BUOY = 33     # y,x f8 + lat,lon f8 + mask i1
+# --dump-outputs keeps at most this many buoys (a fixed sample): 44 B each as written (y,x and lat,lon f8, mask f4,
+# buoy index f8), 44 MB at most, which leaves room under 64 MB for the per-step alive counts
+DUMP_BUOYS = 1_000_000
 WORKLOADS = {
     "cfg5": dict(grid="arctic12", buoys=12_500_000, kind="dense", nrec_res=8,
                  label="cfg5-share: synthetic 1/12deg-class C-grid 1700x1475, 12.5M buoys/GPU (100M on 8 GPUs)"),
@@ -272,6 +277,7 @@ def run_ours(args):
         t1.record(stream)
         barrier()
         launches["n"] = nsteps
+        launches["n_alive"] = na[nwarm:]
         return t0.elapsed_time(t1), int(na[nwarm:].sum().item())
 
     # -- value: K steps, records and state resident in HBM --------------------------------------
@@ -281,6 +287,9 @@ def run_ours(args):
     gpu_launches = launches["n"]                      # k_advect_step launches inside the timed region
     sampler.stop()
     clocks = sampler.summary()
+    if args.dump_outputs and rank == 0:
+        b = (W + K - 1) % NBV                         # the row buffers of the last timed step
+        dump_outputs(args.dump_outputs, o_yx[b], ll_of(b), o_mk[b], launches["n_alive"], eng.perm_t)
 
     def reduce_max_sum(ms_, bs_):
         if world == 1:
@@ -590,6 +599,37 @@ def nP_max(nP, dist, dev):
     return int(t.item())
 
 
+def dump_outputs(out_dir, yx, latlon, mask, n_alive, perm=None):
+    """What a caller of st_step receives from the last timed step, for comparing two builds output for output:
+    the trajectory row (y,x km and lat,lon degrees, f8; the mask as f4) of a fixed sample of at most DUMP_BUOYS
+    buoys, that sample's indices in the order the buoys were handed to the product, and the alive count of
+    every timed step (f8).  perm: the engine's storage order (set_buoys_dev(sort=True) keeps the rows cell-major,
+    row r is buoy perm[r]); the sample is read back in the caller's order, so that it does not depend on how the
+    product lays the buoys out."""
+    import torch
+    nP = yx.shape[0]
+    if nP > DUMP_BUOYS:
+        idx = np.sort(np.random.default_rng(0).choice(nP, DUMP_BUOYS, replace=False))
+    else:
+        idx = np.arange(nP)
+    rows = torch.from_numpy(idx).to(yx.device)
+    if perm is not None:                                # the caller's buoy i is stored in row inv[i]
+        inv = torch.empty_like(perm)
+        inv[perm] = torch.arange(nP, device=perm.device, dtype=perm.dtype)
+        rows = inv.index_select(0, rows)
+    out = {"buoy": idx.astype(np.float64),
+           "yx": yx.index_select(0, rows).cpu().numpy(),
+           "mask": mask.index_select(0, rows).cpu().numpy().astype(np.float32),
+           "n_alive": n_alive.cpu().numpy().astype(np.float64)}
+    if latlon is not None:
+        out["latlon"] = latlon.index_select(0, rows).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log("outputs of the last timed step: %s in %s (%.1f MB)"
+        % (", ".join(sorted(out)), out_dir, sum(a.nbytes for a in out.values()) / 1e6))
+
+
 # ---------------------------------------------------------------------------------------------
 # CPU baselines (oracle/ is only ever the thing timed here, never on the product path)
 # ---------------------------------------------------------------------------------------------
@@ -772,7 +812,15 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=2000, help="buoys in the Python cpu_baseline sample")
     ap.add_argument("--cpu-records", type=int, default=100)
     ap.add_argument("--ref-buoys-per-core", type=int, default=2000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's trajectory row (a fixed sample of at most "
+                         "%d buoys, rank 0's shard) and the alive count of every timed step as DIR/<name>.npy"
+                         % DUMP_BUOYS)
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         args.steps = 100 if args.steps is None else args.steps
         args.warmup = 3 if args.warmup is None else max(args.warmup, 1)

@@ -174,6 +174,39 @@ def gold_survive(sit, g, ic):
     return dict(sv_jT=jT, sv_iT=iT, sv_kill=res)
 
 
+def gold_host(sit):
+    """host_ref.npz: inputs and answers of the host-side surface (tests/test_host_logic.py): time span, index
+    update, seeding helpers, time strings.  The inputs are drawn as the tests drew them next to the imported
+    reference; `sit` is the module whose answers are stored (main() passes the reference)."""
+    rng = np.random.default_rng(0)
+    out = {}
+    t = 850608000 + 1800 + 3600 * np.arange(240)
+    span = []
+    for _ in range(50):
+        seed = int(850608000 + rng.integers(0, 200) * 3600 + rng.integers(0, 3600))
+        stop = int(seed + rng.integers(1, 30) * 3600) if rng.random() < 0.7 else 0           # 0: no iStop
+        span.append([seed, stop] + [int(v) for v in quiet(sit.GetTimeSpan, 3600., t, seed, t[0], t[-1],
+                                                            iStop=stop or None)])
+    out["span"] = np.array(span, np.int64)                  # seed, stop -> Nt, kt0, ktN, itM0, itMN
+    updt = [(rng.integers(5, 50, (2, 4)), rng.integers(5, 50, 2)) for _ in range(8)]
+    out["updt_V"], out["updt_ji"] = np.array([u[0] for u in updt]), np.array([u[1] for u in updt])
+    res = [sit.UpdtInd4NewCell(k + 1, V.copy(), ji.copy()) for k, (V, ji) in enumerate(updt)]
+    out["updt_V_out"], out["updt_ji_out"] = np.array([r[0] for r in res]), np.array([r[1] for r in res])
+    out["debug_seeding"] = sit.debugSeeding()
+    x = rng.uniform(0, 360, 20)
+    out["degE"], out["degWE"], out["degWE_270"] = x, sit.degE_to_degWE(x), sit.degE_to_degWE(270.)
+    it = np.array([0, 850608000, 861494399]); prec = np.array(list("smhD"))
+    out["clock_epoch"], out["clock_precision"] = it, prec
+    out["clock"] = np.array([[sit.epoch2clock(int(a), precision=str(p)) for p in prec] for a in it])
+    msk = (rng.random((40, 30)) > 0.2).astype('i1'); lat = rng.uniform(50, 90, (40, 30))
+    lon = rng.uniform(0, 360, (40, 30)); ic = rng.random((40, 30))
+    out.update(nemo_msk=msk, nemo_lat=lat, nemo_lon=lon, nemo_ic=ic)
+    out["nemo_khss1"] = sit.nemoSeed(msk, lat, lon, ic, khss=1)
+    out["nemo_khss3"] = sit.nemoSeed(msk, lat, lon, ic, khss=3)
+    out["nemo_F"] = quiet(sit.nemoSeed, msk, lat, lon, ic, khss=1, platF=lat + 0.1, plonF=lon + 0.1)
+    return out
+
+
 def grid_arrays(g):
     keys = ["Yt", "Xt", "Yf", "Xf", "Yu", "Xu", "Yv", "Xv", "latT", "lonT", "tmask", "ResKM"]
     return {"g_" + k: g[k] for k in keys}
@@ -244,6 +277,7 @@ def main():
     np.savez_compressed(os.path.join(GOLD, "nearest_box.npz"), pt=np.array(nb_pt), ji_prv=np.array(nb_prv),
                         np_box_r=np.array(nb_r), out=np.array(nb_out))
     print("nearest_box: %d cases, %d not found" % (len(nb_out), int((np.array(nb_out)[:, 0] < 0).sum())))
+    np.savez_compressed(os.path.join(GOLD, "host_ref.npz"), **gold_host(sit))
 
     # ---- tracking on the 'tiny' grid, 48 records ---------------------------------------
     ids_t, SG_t, SC_t = synth.hss_seeds(tiny, IC[0], khss=2)
