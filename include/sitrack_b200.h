@@ -256,6 +256,20 @@ int  st_gather_timed_out(st_ctx *ctx, int *timed_out);
 int  st_gather_set_mode(st_ctx *ctx, int mode);
 int  st_gather_destroy(st_ctx *ctx);
 
+/* ---- sea-ice deformation: strain rates of buoy triangles (RGPS-style) ---------------------
+ * ASYNC.  For nT triangles tri_dev (nT,3) int32 (buoy indices, 16-byte aligned; each triangle anticlockwise
+ * in the (x,y) plane) between two trajectory rows dt_days days apart -- positions yx0_dev, yx1_dev (nP,2) f8
+ * [y,x] km and masks m0_dev, m1_dev (nP) i1 -- writes out_dev (6,nT) f4, one plane per output:
+ *   divergence ux+vy, shear sqrt((ux-vy)^2+(uy+vx)^2), vorticity vx-uy [1/day], area [km^2, on the projection
+ *   plane, at mid-time], y_ctr, x_ctr [km, mid-time centroid];
+ * the velocity gradient is the line integral over the triangle's edges of the velocities (x1-x0)/dt at the
+ * mid-time positions (x0+x1)/2 (Lindsay & Stern 2003).  A triangle with a vertex of mask 0 at either end, or a
+ * signed area that is not positive at either end or at mid-time, gets -9999 in every output.  Computed in f8,
+ * rounded once to f4; bit-identical to oracle/deform_ref.py (DESIGN.md section 10).  Indices are not
+ * range-checked on the device.  ctx may be NULL: the current device, errors through st_last_error(NULL).     */
+int  st_deform_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, const double *yx0_dev, const int8_t *m0_dev,
+                   const double *yx1_dev, const int8_t *m1_dev, double dt_days, float *out_dev, void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

@@ -55,6 +55,11 @@ def __argument_parsing__():
                         help='small clouds: one kernel launch per record (streaming) instead of one per chunk of records')
     parser.add_argument('--rows', default='f4', choices=['f4', 'f8'],
                         help='dtype of the trajectory rows copied off the GPU: f4 = the dtype the output files store (default), f8 = full in-memory arrays as upstream')
+    parser.add_argument('--deform', type=float, default=None, metavar='HOURS',
+                        help='also compute sea-ice deformation (divergence, shear, vorticity) of buoy triangles over '
+                             'windows of HOURS (a multiple of the model time step) on the GPU, into ./nc/..._deformation_...')
+    parser.add_argument('--deform-maxedge', type=float, default=None, metavar='KM',
+                        help='with --deform: drop triangles with an edge longer than KM (default: twice the median edge)')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -114,17 +119,33 @@ def record_windows(zTpos, nP, kstrt, kstop, ztime_model, iTmA, iTmB):
     return z1st, zLst
 
 
+def deform_records(hours, world):
+    """--deform HOURS -> records per deformation window (None without the flag); ERROR and exit when it is not a
+    positive multiple of the model time step, or under torchrun (triangles would cross the ranks' shards)."""
+    if hours is None:
+        return None
+    if world > 1:
+        print('ERROR: --deform is not available with several processes (WORLD_SIZE > 1): triangles would cross ranks')
+        exit(0)
+    n = hours * 3600. / rdt
+    if not (hours > 0 and abs(n - round(n)) < 1e-9 and round(n) >= 1):
+        print('ERROR: --deform HOURS must be a positive multiple of the model time step (%g h), got %g' % (rdt / 3600., hours))
+        exit(0)
+    return int(round(n))
+
+
 def main():
     print('\n##########################################################')
     print('#            SITRACK ICE PARTICULES TRACKER              #')
     print('#                 (sitrack_b200 engine)                  #')
     print('##########################################################\n')
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
+    args = __argument_parsing__()
+    ndeform = deform_records(args.deform, world)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
         dist.init_process_group("gloo")
-    args = __argument_parsing__()
     cf_uv, cf_mm, fNCseed, jrecSeed, cdate_stop, CONF = args.fsi3, args.fmmm, args.fsdg, args.krec, args.dend, args.ncnf
     lUse2DTime = not args.fxdt
     if args.device is not None:
@@ -260,6 +281,24 @@ def main():
     # small clouds are launch-bound: a whole chunk of records per launch (k_advect_multi, 4 us per record instead of
     # 11 us) and the rows of the chunk come back together; large clouds stream row by row
     small = world == 1 and physics is None and nP <= 262144 and nP * (Nt + 1) * 17 < 2e9 and not args.no_chunk
+    deform = None
+    if ndeform:
+        # strain rates of buoy triangles, window by window on the GPU; the mesh is built from the seeds in the order the
+        # files use (after --sort), so its vertices index the tracking file's `buoy` axis
+        nwin = Nt // ndeform
+        if nwin < 1:
+            print('ERROR: --deform window (%d records) is longer than the run (%d records)!' % (ndeform, Nt))
+            exit(0)
+        tri = sit.TriangulateCloud(xPosC0, max_edge_km=args.deform_maxedge)
+        if tri.shape[0] == 0:
+            print('ERROR: --deform: no triangle left in the mesh of the buoys!')
+            exit(0)
+        print(' *** --deform: %d triangles, %d windows of %d records' % (tri.shape[0], nwin, ndeform))
+        cf_def = './nc/' + corgn + '_deformation_' + SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + hstr(vTime[nwin * ndeform]) + csfkm + ext
+        dwriter = sit.DeformationWriter(cf_def, nwin, tri, IDs, corigin=corgn)
+        deform = dict(tri=tri, every=ndeform,
+                      sink=lambda w, out: dwriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], out))
+        small = False                                             # windows close inside the streaming record loop
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
         res = eng.track(record, Nt, kstrt=kstrt, pos0=xPosC0, posG0=xPosG0, rec_first=z1st, chunk=nchunk,
@@ -268,8 +307,10 @@ def main():
             keep_row(k, res['posC'][k + 1], res['posG'][k + 1], res['mask'][k + 1])
     else:
         res = eng.track(record, Nt, kstrt=kstrt, rec_first=cut(z1st), sink=sink,
-                        row_dtype='f8' if physics else args.rows, physics=physics)
+                        row_dtype='f8' if physics else args.rows, physics=physics, deform=deform)
     eng.close()
+    if deform:
+        dwriter.close()
     ds.close()
     n_alive = res['n_alive']
     if world > 1:

@@ -8,6 +8,7 @@ from .util import *          # noqa: F401,F403
 from .ncio import *          # noqa: F401,F403
 from .tracking import *      # noqa: F401,F403
 from .locate import *        # noqa: F401,F403
+from .deform import *        # noqa: F401,F403
 from . import config                      # noqa: F401
 from .engine import TrackEngine          # noqa: F401
 from ._lib import SitrackCudaError       # noqa: F401

@@ -1136,6 +1136,21 @@ int st_track_record_host_f4(st_ctx* c, int jrec, const float* u, const float* v,
     return track_record_host_impl(c, jrec, u, v, ic, out_yx, out_latlon, out_mask, n_alive, 1);
 }
 
+// ---- deformation of buoy triangles (st_deform.cu) ------------------------------------------------
+int st_deform_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double* yx0, const int8_t* m0, const double* yx1,
+                  const int8_t* m1, double dt_days, float* out, void* stream)
+{
+    if (nT < 0) return fail(c, ST_EINVAL, "st_deform_dev: nT < 0");
+    if (nT == 0) return ST_OK;
+    if (!tri || !yx0 || !m0 || !yx1 || !m1 || !out) return fail(c, ST_EINVAL, "st_deform_dev: NULL argument");
+    if ((uintptr_t)tri % 16 || (uintptr_t)yx0 % 16 || (uintptr_t)yx1 % 16)
+        return fail(c, ST_EINVAL, "st_deform_dev: tri, yx0 and yx1 must be 16-byte aligned");
+    if (!(dt_days > 0.0)) return fail(c, ST_EINVAL, "st_deform_dev: dt_days must be positive");
+    if (c) CU(c, cudaSetDevice(c->device));
+    CU(c, launch_deform(nT, tri, (const pt*)yx0, m0, (const pt*)yx1, m1, dt_days, out, (cudaStream_t)stream));
+    return ST_OK;
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

@@ -161,4 +161,10 @@ cudaError_t launch_geom_survive(long long n, const int32_t* ji, int Nj, int Ni, 
 cudaError_t launch_haversine(long long n, double plat, double plon, const double* lat, const double* lon,
                              double* out, cudaStream_t st);
 
+// ---- strain rates of buoy triangles between two trajectory rows (st_deform.cu) -------------
+// k_deform: tri (nT,3) buoy indices (16-byte aligned), yx0/yx1 (nP) positions and m0/m1 (nP) masks at the two ends
+// of the window, dt in days; out = six (nT) f4 planes [divergence | shear | vorticity | area | y_ctr | x_ctr].
+cudaError_t launch_deform(long long nT, const int32_t* tri, const pt* yx0, const int8_t* m0, const pt* yx1,
+                          const int8_t* m1, double dt, float* out, cudaStream_t st);
+
 }  // namespace st

@@ -241,6 +241,7 @@ class TrackEngine:
         rf = None if rec_first is None else as_c(rec_first, np.int32)
         rl = None if rec_last is None else as_c(rec_last, np.int32)
         self.perm = None
+        self.perm_t = None
         if sort and pos.shape[0] > 1:
             perm = np.argsort(cell[:, 0].astype(np.int64) * self.Ni + cell[:, 1], kind="stable")
             pos, cell = as_c(pos[perm], np.float64), as_c(cell[perm], np.int32)
@@ -426,7 +427,7 @@ class TrackEngine:
 
     # -- the record loop ---------------------------------------------------------------
     def track(self, records, nrec, kstrt=0, pos0=None, posG0=None, rec_first=None, want_latlon=True,
-              sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None):
+              sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None):
         """The record loop (si3_part_tracker.py:361-496), pipelined.
 
         records: callable k -> (u, v, ic) arrays (Nj,Ni) for record index k (0-based
@@ -440,6 +441,12 @@ class TrackEngine:
         physics = dict(scheme=, interp=, max_hops=) switches every record to st_step_ext (f8 rows only).
         row_dtype "f4" moves the rows in the output file's dtype (ncio.py:153-159: 17 B per buoy
         instead of 33 B over PCIe, values = the f8 rows cast to f4); the state stays f8 on the device.
+        deform = dict(tri=(nT,3) triangles of buoys in the caller's order (anticlockwise, e.g. TriangulateCloud),
+        every=n, sink=callable or None): strain rates of the triangles (sitrack_b200.deform) over the windows of
+        rows [w*n, (w+1)*n], computed on the device from the f8 positions as each window closes (a trailing partial
+        window is dropped; row 0 is the state handed to set_buoys, masked like the returned series' row 0).
+        sink(w, out) receives a dict of (nT,) f4 arrays in the caller's triangle order; with sink None the
+        list of them is returned under "deform".  Not with the chunked season path (chunk > 1, sink=None).
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -456,7 +463,10 @@ class TrackEngine:
                 raise ValueError("physics modes write f8 rows")
             chunk = None
         if chunk and chunk > 1 and sink is None:
+            if deform is not None:
+                raise ValueError("deform runs on the streaming record loop: not with chunk > 1 and sink=None")
             return self._track_chunked(get, nrec, kstrt, pos0, posG0, rec_first, want_latlon, int(chunk), rdt)
+        dfm = None if deform is None else _DeformRun(self, torch, dev, deform, rec_first, kstrt, row_f4=rdt == torch.float32)
         self.record_slots(2)
         stg = [self.staging(0), self.staging(1)]
         s_in, s_cmp, s_out = (torch.cuda.Stream(dev) for _ in range(3))
@@ -533,25 +543,111 @@ class TrackEngine:
                         l.copy_(d_ll[b], non_blocking=True)
                     m.copy_(d_mk[b], non_blocking=True)
                 ev_out[k] = torch.cuda.Event(); ev_out[k].record(s_out)
+                if dfm is not None:
+                    dfm.after_step(k, d_yx[b], d_mk[b], s_cmp, s_out)
             for k in range(max(0, nrec - NB), nrec):
                 if keep:
                     ev_out[k].synchronize()
                 else:
                     drain(k)
+            if dfm is not None:
+                dfm.finish()
         finally:
             if chain:
                 self.set_row_chain(False)                  # state up to date again (synchronises)
         torch.cuda.synchronize(dev)
         pool.shutdown()
         n_alive = d_na.cpu().numpy()
+        extra = {} if dfm is None or dfm.collected is None else dict(deform=dfm.collected)
         if not keep:
-            return dict(n_alive=n_alive)
+            return dict(n_alive=n_alive, **extra)
         posC, posG, mask = posC.numpy(), posG.numpy(), mask.numpy()
         if perm is not None:                                # engine order -> the caller's order
             inv = np.empty_like(perm); inv[perm] = np.arange(perm.size)
             posC, posG, mask = posC[:, inv], posG[:, inv], mask[:, inv]
         _finish_rows(posC, posG, mask, pos0, posG0, rec_first, kstrt)
-        return dict(posC=posC, posG=posG, mask=mask, n_alive=n_alive)
+        return dict(posC=posC, posG=posG, mask=mask, n_alive=n_alive, **extra)
+
+
+class _DeformRun:
+    """track(deform=...): the anchor row of the open window on the device, k_deform when a window closes, its
+    outputs to the host on the output stream.
+
+    Positions are f8: with f8 rows the row itself (read only, so row chaining is unaffected), with f4 rows the
+    device state (steps with f4 rows do not chain, so it is current after every step).  Triangles are mapped into
+    engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs go back to the
+    caller's triangle order on the host."""
+
+    def __init__(self, eng, torch, dev, spec, rec_first, kstrt, row_f4):
+        from . import deform as D
+        self.eng, self.torch, self.row_f4, self.D = eng, torch, row_f4, D
+        self.every = int(spec["every"])
+        if self.every < 1:
+            raise ValueError("deform: every must be >= 1 record")
+        self.sink = spec.get("sink")
+        self.collected = [] if self.sink is None else None
+        nP = eng.nP
+        tri = D.check_mesh(spec["tri"], nP)
+        perm = eng.perm
+        if perm is None and getattr(eng, "perm_t", None) is not None:      # set_buoys_dev(sort=True)
+            perm = eng.perm_t.cpu().numpy()
+        m0 = np.ones(nP, np.int8) if rec_first is None else (np.asarray(rec_first) - kstrt == 0).astype(np.int8)
+        if perm is not None:                                                # caller's order -> engine slots
+            if perm.shape != (nP,):
+                raise ValueError("deform: the engine's buoy permutation does not match its %d buoys" % nP)
+            inv = np.empty_like(perm); inv[perm] = np.arange(perm.size)
+            tri = inv[tri].astype(np.int32)
+            m0 = m0[perm]
+        tri, self.inv = D.sort_mesh(tri)
+        self.nT = tri.shape[0]
+        self.dt = self.every * eng.rdt / 86400.0
+        self.tri_t = torch.from_numpy(tri).to(dev)
+        p = C.c_void_p()
+        check(eng.L.st_state_device_ptrs(eng.h, C.byref(p), None, None), eng.h)
+        self.state_pos = _tensor_from_ptr(torch, p.value, (nP, 2), torch.float64, 8, eng.device)
+        # the anchor: row 0 (on torch's current stream; track's streams wait for it)
+        self.a_yx = self.state_pos.clone()
+        self.a_mk = torch.from_numpy(m0).to(dev)
+        self.d_out = [torch.empty((6, max(self.nT, 1)), dtype=torch.float32, device=dev) for _ in range(2)]
+        self.h_out = [torch.empty((6, max(self.nT, 1)), dtype=torch.float32).pin_memory() for _ in range(2)]
+        self.ev_out = []
+        self.drained = 0
+
+    def after_step(self, k, yx_row, mk_row, s_cmp, s_out):
+        """Step k has been queued on s_cmp: row k+1 closes window w when k+1 = (w+1)*every."""
+        if (k + 1) % self.every:
+            return
+        torch, w = self.torch, (k + 1) // self.every - 1
+        b = w % 2
+        if w >= 2:
+            s_cmp.wait_event(self.ev_out[w - 2])                   # d_out[b] has reached the host
+        yx = self.state_pos if self.row_f4 else yx_row
+        self.D.launch(self.eng.L, self.eng.h, self.nT, self.tri_t, self.a_yx, self.a_mk, yx, mk_row, self.dt,
+                      self.d_out[b], s_cmp)
+        with torch.cuda.stream(s_cmp):                              # row (w+1)*every anchors the next window
+            self.a_yx.copy_(yx)
+            self.a_mk.copy_(mk_row)
+        ev = torch.cuda.Event(); ev.record(s_cmp)
+        if w >= 2:
+            self._drain(w - 2)                                      # h_out[b] is free again
+        s_out.wait_event(ev)
+        with torch.cuda.stream(s_out):
+            self.h_out[b].copy_(self.d_out[b], non_blocking=True)
+        self.ev_out.append(torch.cuda.Event()); self.ev_out[w].record(s_out)
+
+    def _drain(self, w):
+        self.ev_out[w].synchronize()
+        o = self.h_out[w % 2].numpy()[:, :self.nT][:, self.inv]     # a copy, in the caller's triangle order
+        out = {n: o[j] for j, n in enumerate(self.D.DEFORM_NAMES)}
+        if self.sink is None:
+            self.collected.append(out)
+        else:
+            self.sink(w, out)
+        self.drained = w + 1
+
+    def finish(self):
+        for w in range(self.drained, len(self.ev_out)):
+            self._drain(w)
 
 
 def _finish_rows(posC, posG, mask, pos0, posG0, rec_first, kstrt):

@@ -21,7 +21,7 @@ from .util import epoch2clock as e2c
 
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
-           "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter"]
+           "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -223,6 +223,93 @@ class CloudBuoyWriter:
             with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
                 for fn in sorted(os.listdir(self._tmp)):
                     z.write(os.path.join(self._tmp, fn), arcname=fn)         # streamed from disk, like np.savez's members
+            shutil.rmtree(self._tmp, ignore_errors=True)
+        print('      ===> ' + self.cf_out + ' saved!')
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DeformationWriter:
+    """Window-by-window writer of the strain rates of buoy triangles (sitrack_b200.deform, TrackEngine.track's
+    `deform`).  Dimensions time (windows), triangle, vertex = 3; variables
+      time_start, time_end (time) i4          first and last date of each window [tunits]
+      vertices (triangle,vertex) i4           indices into the `buoy` axis of the tracking file
+      id_vertices (triangle,vertex) i8        IDs of those buoys
+      divergence, shear, vorticity (time,triangle) f4 [day-1]; area f4 [km2]; y_ctr, x_ctr f4 [km]
+    each output with `units` and the fill value `fillVal` for invalid triangles.  netCDF4 when available and the
+    name does not end in .npz; otherwise an .npz with the same variables, plus `<name>_units` (0-d strings) and
+    `FillValue` members for the attributes, assembled from on-disk .npy members like CloudBuoyWriter's."""
+
+    def __init__(self, cf_out, ntime, tri, pIDs, tunits=tunits_default, fillVal=FillValue, corigin=None):
+        from .deform import DEFORM_NAMES, DEFORM_UNITS
+        print('\n *** [DeformationWriter]: About to generate file: ' + cf_out + ' ...')
+        tri = np.asarray(tri).reshape(-1, 3)
+        self.ntime, self.nT = int(ntime), tri.shape[0]
+        self.names = DEFORM_NAMES
+        ids = np.asarray(pIDs).astype('i8')[tri] if self.nT else np.zeros((0, 3), 'i8')
+        nc = None
+        if not str(cf_out).endswith(".npz"):
+            try:
+                import netCDF4 as nc
+            except ImportError:
+                cf_out += ".npz"
+                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
+        self.cf_out, self._nc = cf_out, nc
+        if nc is None:
+            import tempfile
+            self._tmp = tempfile.mkdtemp(prefix=".deform_", dir=os.path.dirname(os.path.abspath(cf_out)) or ".")
+            mm = lambda n, dt, shp: np.lib.format.open_memmap(os.path.join(self._tmp, n + ".npy"), mode='w+', dtype=dt, shape=shp)
+            self._v = {n: mm(n, 'f4', (self.ntime, self.nT)) for n in self.names}
+            self._v['time_start'] = mm('time_start', 'i4', (self.ntime,))
+            self._v['time_end'] = mm('time_end', 'i4', (self.ntime,))
+            mm('vertices', 'i4', (self.nT, 3))[:] = tri
+            mm('id_vertices', 'i8', (self.nT, 3))[:] = ids
+            for n in self.names:
+                np.save(os.path.join(self._tmp, n + "_units.npy"), np.array(DEFORM_UNITS[n]))
+            np.save(os.path.join(self._tmp, "FillValue.npy"), np.float32(fillVal))
+        else:
+            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
+            f.createDimension('time', None)
+            f.createDimension('triangle', self.nT)
+            f.createDimension('vertex', 3)
+            self._v = {}
+            for n in ('time_start', 'time_end'):
+                self._v[n] = f.createVariable(n, 'i4', ('time',)); self._v[n].units = tunits
+            f.createVariable('vertices', 'i4', ('triangle', 'vertex'))[:] = tri
+            vid = f.createVariable('id_vertices', 'i8', ('triangle', 'vertex')); vid.units = 'ID of buoy'
+            vid[:] = ids
+            zkw = dict(zlib=True, complevel=9)
+            for n in self.names:
+                self._v[n] = f.createVariable(n, 'f4', ('time', 'triangle'), fill_value=fillVal, **zkw)
+                self._v[n].units = DEFORM_UNITS[n]
+            if corigin:
+                f.Origin = corigin
+            f.About = 'Sea-ice deformation rates of buoy triangles'
+            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+
+    def write(self, jw, time_start, time_end, out):
+        """Window jw: out = dict of (nT,) arrays over the six outputs."""
+        self._v['time_start'][jw] = time_start
+        self._v['time_end'][jw] = time_end
+        for n in self.names:
+            self._v[n][jw, :] = np.asarray(out[n], dtype=np.float32)
+
+    def close(self):
+        if self._nc is not None:
+            self._f.close()
+        else:
+            import shutil
+            import zipfile
+            for v in self._v.values():
+                v.flush()
+            self._v = {}
+            with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
+                for fn in sorted(os.listdir(self._tmp)):
+                    z.write(os.path.join(self._tmp, fn), arcname=fn)
             shutil.rmtree(self._tmp, ignore_errors=True)
         print('      ===> ' + self.cf_out + ' saved!')
 
