@@ -270,6 +270,33 @@ int  st_gather_destroy(st_ctx *ctx);
 int  st_deform_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, const double *yx0_dev, const int8_t *m0_dev,
                    const double *yx1_dev, const int8_t *m1_dev, double dt_days, float *out_dev, void *stream);
 
+/* ---- deformation coarse-grained over material boxes, and per-scale statistics ------------------
+ * A hierarchy of `levels` (1..20) box levels over the nT triangles (DESIGN.md section 11, sit.BoxHierarchy):
+ * tri_dev (nT,3) int32 is the mesh in hierarchy order (sorted by the Morton code of each triangle's level-1 box),
+ * tri_off_dev (level_nbox[0]+1) int64 the level-1 boxes' ranges of it, child_off_dev the ranges of children of the
+ * boxes of levels 2..levels, concatenated ((level_nbox[l]+1) each; may be NULL when levels = 1).  level_nbox and
+ * min_area (HOST, levels): boxes per level and the area [km^2] from which a box counts (cover * L^2).
+ * st_deform_scales_scratch_bytes gives the size of the scratch buffer st_deform_scales_dev needs (box sums and
+ * moment partials); allocate it once per hierarchy.
+ * ASYNC st_deform_scales_dev: between two rows dt_days apart (positions and masks as st_deform_dev), per box the sums
+ * over its valid triangles of 2A and of the edge line integrals (f8, in a fixed order without atomics; an invalid
+ * triangle adds +0.0); per box divergence, shear, vorticity, eps_tot = sqrt(div^2 + shear^2), L_eff = sqrt(area),
+ * centroid.  Per scale s (0 = the triangles themselves, s = the boxes of level s):
+ *   moments_dev (levels+1, 4) f8   sums of L_eff, eps_tot, eps_tot^2, eps_tot^3 over the valid cells;
+ *   hist_dev (levels+1, 3, nedge+1) int64   counts of eps_tot, |div|, shear [1/day] binned on edges_dev (nedge f8,
+ *                                           ascending) by searchsorted(edges, v, side="right").
+ * boxes_dev, if not NULL, (7, sum level_nbox) f4 planes divergence, shear, vorticity, eps_tot, L_eff, y_ctr, x_ctr
+ * of every box, -9999 where invalid.  Bit-identical to oracle/deform_scale_ref.py and run to run.  No host
+ * synchronisation, no allocation; indices and ranges are not checked on the device.                          */
+int  st_deform_scales_scratch_bytes(int64_t nT, int levels, const int64_t *level_nbox, const double *min_area,
+                                    int nedge, int64_t *bytes);
+int  st_deform_scales_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, const double *yx0_dev,
+                          const int8_t *m0_dev, const double *yx1_dev, const int8_t *m1_dev, double dt_days,
+                          int levels, const int64_t *level_nbox, const double *min_area, const int64_t *tri_off_dev,
+                          const int64_t *child_off_dev, int nedge, const double *edges_dev, void *scratch_dev,
+                          int64_t scratch_bytes, double *moments_dev, int64_t *hist_dev, float *boxes_dev,
+                          void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

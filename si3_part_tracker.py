@@ -60,6 +60,10 @@ def __argument_parsing__():
                              'windows of HOURS (a multiple of the model time step) on the GPU, into ./nc/..._deformation_...')
     parser.add_argument('--deform-maxedge', type=float, default=None, metavar='KM',
                         help='with --deform: drop triangles with an edge longer than KM (default: twice the median edge)')
+    parser.add_argument('--deform-scales', type=float, nargs=2, default=None, metavar=('L0_KM', 'LEVELS'),
+                        help='with --deform: also coarse-grain the triangles over LEVELS levels of material boxes of side '
+                             'L0_KM * 2^s and write per-scale statistics (n, means of L_eff and eps_tot^q, histograms) '
+                             'of every window into ./nc/..._deformation-scaling_...')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -134,6 +138,24 @@ def deform_records(hours, world):
     return int(round(n))
 
 
+def deform_scales_args(scales, hours):
+    """--deform-scales L0_KM LEVELS -> (L0_km, levels) or None; ERROR and exit without --deform, with L0 <= 0, or
+    with LEVELS not an integer in 1..20."""
+    if scales is None:
+        return None
+    L0, lev = scales
+    if hours is None:
+        print('ERROR: --deform-scales needs --deform HOURS')
+        exit(0)
+    if not L0 > 0:
+        print('ERROR: --deform-scales L0_KM must be positive, got %g' % L0)
+        exit(0)
+    if lev != int(lev) or not 1 <= lev <= sit.MAX_LEVELS:
+        print('ERROR: --deform-scales LEVELS must be an integer in 1..%d, got %g' % (sit.MAX_LEVELS, lev))
+        exit(0)
+    return L0, int(lev)
+
+
 def main():
     print('\n##########################################################')
     print('#            SITRACK ICE PARTICULES TRACKER              #')
@@ -142,6 +164,7 @@ def main():
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     args = __argument_parsing__()
     ndeform = deform_records(args.deform, world)
+    dscales = deform_scales_args(args.deform_scales, args.deform)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
@@ -294,10 +317,19 @@ def main():
             print('ERROR: --deform: no triangle left in the mesh of the buoys!')
             exit(0)
         print(' *** --deform: %d triangles, %d windows of %d records' % (tri.shape[0], nwin, ndeform))
-        cf_def = './nc/' + corgn + '_deformation_' + SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + hstr(vTime[nwin * ndeform]) + csfkm + ext
+        cf_tail = SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + hstr(vTime[nwin * ndeform]) + csfkm + ext
+        cf_def = './nc/' + corgn + '_deformation_' + cf_tail
         dwriter = sit.DeformationWriter(cf_def, nwin, tri, IDs, corigin=corgn)
         deform = dict(tri=tri, every=ndeform,
                       sink=lambda w, out: dwriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], out))
+        if dscales:
+            # boxes over the same mesh and seeds; only per-scale statistics leave the GPU
+            H = sit.BoxHierarchy(xPosC0, tri, *dscales)
+            print(' *** --deform-scales: %d levels of boxes from %g km, %s boxes' % (H.levels, H.L0_km, H.nbox.tolist()))
+            cf_sc = './nc/' + corgn + '_deformation-scaling_' + cf_tail
+            swriter = sit.DeformationScalingWriter(cf_sc, nwin, H.scale_km, H.bin_edges, corigin=corgn)
+            deform.update(scales=H, scale_sink=lambda w, st: swriter.write(w, vTime[w * ndeform],
+                                                                          vTime[(w + 1) * ndeform], st))
         small = False                                             # windows close inside the streaming record loop
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
@@ -311,6 +343,8 @@ def main():
     eng.close()
     if deform:
         dwriter.close()
+        if dscales:
+            swriter.close()
     ds.close()
     n_alive = res['n_alive']
     if world > 1:

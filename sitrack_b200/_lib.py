@@ -75,6 +75,9 @@ SIGNATURES = {
     "st_gather_destroy": (c_int, [vp]),
     "st_gather_set_mode": (c_int, [vp, c_int]),
     "st_deform_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, vp, c_dbl, vp, vp]),
+    "st_deform_scales_scratch_bytes": (c_int, [c_i64, c_int, vp, vp, c_int, vp]),
+    "st_deform_scales_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, vp, c_dbl, c_int, vp, vp, vp, vp, c_int, vp, vp, c_i64,
+                                     vp, vp, vp, vp]),
     "st_xy2latlon": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_latlon2xy": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_xy2latlon_dev": (c_int, [c_i64, vp, vp, c_dbl, c_dbl, vp]),

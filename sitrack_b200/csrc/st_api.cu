@@ -1151,6 +1151,61 @@ int st_deform_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double* yx0, 
     return ST_OK;
 }
 
+// ---- deformation coarse-grained over a box hierarchy, and its statistics (st_deform_scale.cu) ------
+static int scale_plan_checked(st_ctx* c, const char* who, int64_t nT, int levels, const int64_t* level_nbox,
+                              const double* min_area, int nedge, ScalePlan* p, long long* bytes)
+{
+    if (levels < 1 || levels > SC_MAX_LEVELS) return fail(c, ST_EINVAL, std::string(who) + ": levels must be in 1..20");
+    if (!level_nbox || !min_area) return fail(c, ST_EINVAL, std::string(who) + ": NULL argument");
+    if (nedge < 1 || nedge > SC_MAX_EDGES) return fail(c, ST_EINVAL, std::string(who) + ": nedge must be in 1..4096");
+    if (nT < 1 || nT > INT32_MAX) return fail(c, ST_EINVAL, std::string(who) + ": nT must be in 1..2^31-1");
+    for (int l = 0; l < levels; ++l) {
+        if (level_nbox[l] < 1 || level_nbox[l] > (l ? level_nbox[l - 1] : nT))
+            return fail(c, ST_EINVAL, std::string(who) + ": level_nbox must be >= 1 and non-increasing, level 1 <= nT");
+        if (!(min_area[l] > 0.0)) return fail(c, ST_EINVAL, std::string(who) + ": min_area must be positive");
+    }
+    static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
+    *bytes = scale_plan(levels, reinterpret_cast<const long long*>(level_nbox), min_area, nedge, p);
+    return ST_OK;
+}
+
+int st_deform_scales_scratch_bytes(int64_t nT, int levels, const int64_t* level_nbox, const double* min_area,
+                                   int nedge, int64_t* bytes)
+{
+    ScalePlan p; long long b = 0;
+    if (!bytes) return fail(nullptr, ST_EINVAL, "st_deform_scales_scratch_bytes: NULL argument");
+    const int rc = scale_plan_checked(nullptr, "st_deform_scales_scratch_bytes", nT, levels, level_nbox, min_area, nedge, &p, &b);
+    if (rc != ST_OK) return rc;
+    *bytes = b;
+    return ST_OK;
+}
+
+int st_deform_scales_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double* yx0, const int8_t* m0,
+                         const double* yx1, const int8_t* m1, double dt_days, int levels, const int64_t* level_nbox,
+                         const double* min_area, const int64_t* tri_off, const int64_t* child_off, int nedge,
+                         const double* edges, void* scratch, int64_t scratch_bytes, double* moments, int64_t* hist,
+                         float* boxes, void* stream)
+{
+    ScalePlan p; long long need = 0;
+    const int rc = scale_plan_checked(c, "st_deform_scales_dev", nT, levels, level_nbox, min_area, nedge, &p, &need);
+    if (rc != ST_OK) return rc;
+    if (!tri || !yx0 || !m0 || !yx1 || !m1 || !tri_off || (levels > 1 && !child_off) || !edges || !scratch ||
+        !moments || !hist)
+        return fail(c, ST_EINVAL, "st_deform_scales_dev: NULL argument");
+    if ((uintptr_t)tri % 16 || (uintptr_t)yx0 % 16 || (uintptr_t)yx1 % 16)
+        return fail(c, ST_EINVAL, "st_deform_scales_dev: tri, yx0 and yx1 must be 16-byte aligned");
+    if ((uintptr_t)tri_off % 8 || (uintptr_t)child_off % 8 || (uintptr_t)edges % 8 || (uintptr_t)scratch % 8 ||
+        (uintptr_t)moments % 8 || (uintptr_t)hist % 8 || (uintptr_t)boxes % 4)
+        return fail(c, ST_EINVAL, "st_deform_scales_dev: tri_off, child_off, edges, scratch, moments and hist must be 8-byte aligned");
+    if (scratch_bytes < need) return fail(c, ST_EINVAL, "st_deform_scales_dev: scratch_bytes is smaller than st_deform_scales_scratch_bytes");
+    if (!(dt_days > 0.0)) return fail(c, ST_EINVAL, "st_deform_scales_dev: dt_days must be positive");
+    if (c) CU(c, cudaSetDevice(c->device));
+    CU(c, launch_deform_scales(p, tri, reinterpret_cast<const long long*>(tri_off),
+                               reinterpret_cast<const long long*>(child_off), (const pt*)yx0, m0, (const pt*)yx1, m1,
+                               dt_days, edges, scratch, moments, hist, boxes, (cudaStream_t)stream));
+    return ST_OK;
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

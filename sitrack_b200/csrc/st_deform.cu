@@ -12,35 +12,11 @@
 // stages its 256 index triples through shared memory with 16-byte loads); positions and masks are gathered
 // through the read-only path.  The caller sorts the triangles by their smallest vertex once, so that a warp's
 // gathers stay within a few lines of a cell-major cloud.
-#include "st_kernels.h"
+#include "st_deform.cuh"
 
 namespace st {
 
 constexpr int DEF_BLOCK = 256;
-
-__device__ __forceinline__ pt ld_ro_pt(const pt* __restrict__ a, int i)
-{
-    const double2 v = __ldg(reinterpret_cast<const double2*>(a + i));
-    pt r; r.y = v.x; r.x = v.y; return r;
-}
-
-// 2A = (X0 Y1 - X1 Y0) + (X1 Y2 - X2 Y1) + (X2 Y0 - X0 Y2), left to right
-__device__ __forceinline__ double twice_area(double X0, double X1, double X2, double Y0, double Y1, double Y2)
-{
-    const double t01 = __dsub_rn(__dmul_rn(X0, Y1), __dmul_rn(X1, Y0));
-    const double t12 = __dsub_rn(__dmul_rn(X1, Y2), __dmul_rn(X2, Y1));
-    const double t20 = __dsub_rn(__dmul_rn(X2, Y0), __dmul_rn(X0, Y2));
-    return __dadd_rn(__dadd_rn(t01, t12), t20);
-}
-
-// sum over the edges 0->1, 1->2, 2->0 of (F_{i+1} + F_i)(Z_{i+1} - Z_i), left to right
-__device__ __forceinline__ double edge_sum(double F0, double F1, double F2, double Z0, double Z1, double Z2)
-{
-    const double e01 = __dmul_rn(__dadd_rn(F1, F0), __dsub_rn(Z1, Z0));
-    const double e12 = __dmul_rn(__dadd_rn(F2, F1), __dsub_rn(Z2, Z1));
-    const double e20 = __dmul_rn(__dadd_rn(F0, F2), __dsub_rn(Z0, Z2));
-    return __dadd_rn(__dadd_rn(e01, e12), e20);
-}
 
 // out: six (nT) f4 planes [divergence | shear | vorticity | area | y_ctr | x_ctr]
 __global__ void __launch_bounds__(DEF_BLOCK) k_deform(long long nT, const int* __restrict__ tri,

@@ -167,4 +167,31 @@ cudaError_t launch_haversine(long long n, double plat, double plon, const double
 cudaError_t launch_deform(long long nT, const int32_t* tri, const pt* yx0, const int8_t* m0, const pt* yx1,
                           const int8_t* m1, double dt, float* out, cudaStream_t st);
 
+// ---- coarse-grained deformation over a hierarchy of material boxes, and its statistics (st_deform_scale.cu) ----
+constexpr int SC_MAX_LEVELS = 20;
+constexpr int SC_MAX_EDGES = 4096;
+
+// Shapes of one hierarchy, passed by value.  Box records of all levels are concatenated (level 1 first); child
+// offsets of levels >= 2 likewise; moment partials: scale s (0 = triangles) owns blocks [blk0[s], blk0[s+1]).
+struct ScalePlan {
+    int levels, nedge, nbin;                    // nbin = nedge + 1 counts per histogram
+    long long nbox_all;
+    long long nbox[SC_MAX_LEVELS];
+    long long box0[SC_MAX_LEVELS];              // first box of each level
+    long long child0[SC_MAX_LEVELS];            // level l >= 1 (0-based): its (nbox[l]+1) offsets start here
+    double min_area[SC_MAX_LEVELS];             // a box is valid when its area >= min_area (cover * L^2)
+    int blk0[SC_MAX_LEVELS + 2];
+};
+
+// Fills *p; returns the scratch bytes launch_deform_scales needs (box sums + moment partials).
+long long scale_plan(int levels, const long long* nbox, const double* min_area, int nedge, ScalePlan* p);
+// tri (nT,3) buoy indices in hierarchy order; tri_off (nbox[0]+1) level-1 ranges; child_off the concatenated child
+// ranges of levels >= 2; edges (nedge) f8 ascending.  Writes mom (levels+1, 4) f8 = sums of L_eff, eps_tot,
+// eps_tot^2, eps_tot^3, hist (levels+1, 3, nedge+1) counts of eps_tot, |div|, shear, and, when out is not NULL,
+// seven (nbox_all) f4 planes of box outputs.
+cudaError_t launch_deform_scales(const ScalePlan& p, const int32_t* tri, const long long* tri_off,
+                                 const long long* child_off, const pt* yx0, const int8_t* m0, const pt* yx1,
+                                 const int8_t* m1, double dt, const double* edges, void* scratch, double* mom,
+                                 int64_t* hist, float* out, cudaStream_t st);
+
 }  // namespace st

@@ -447,6 +447,10 @@ class TrackEngine:
         window is dropped; row 0 is the state handed to set_buoys, masked like the returned series' row 0).
         sink(w, out) receives a dict of (nT,) f4 arrays in the caller's triangle order; with sink None the
         list of them is returned under "deform".  Not with the chunked season path (chunk > 1, sink=None).
+        deform may also hold scales=BoxHierarchy (built on the same tri and buoys) and scale_sink=callable or None:
+        as each window closes the deformation of its boxes is reduced on the device to per-scale statistics
+        (sitrack_b200.deform_scales), and only those reach the host: scale_sink(w, stats), or with scale_sink None
+        the list of them under "deform_scales".  They do not depend on the order the buoys are stored in.
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -559,6 +563,8 @@ class TrackEngine:
         pool.shutdown()
         n_alive = d_na.cpu().numpy()
         extra = {} if dfm is None or dfm.collected is None else dict(deform=dfm.collected)
+        if dfm is not None and dfm.scale_collected is not None:
+            extra["deform_scales"] = dfm.scale_collected
         if not keep:
             return dict(n_alive=n_alive, **extra)
         posC, posG, mask = posC.numpy(), posG.numpy(), mask.numpy()
@@ -576,7 +582,8 @@ class _DeformRun:
     Positions are f8: with f8 rows the row itself (read only, so row chaining is unaffected), with f4 rows the
     device state (steps with f4 rows do not chain, so it is current after every step).  Triangles are mapped into
     engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs go back to the
-    caller's triangle order on the host."""
+    caller's triangle order on the host.  With `scales`, the box hierarchy pass runs on the same rows after k_deform
+    and before the anchor copy; its statistics go to the host on the output stream alongside the triangles'."""
 
     def __init__(self, eng, torch, dev, spec, rec_first, kstrt, row_f4):
         from . import deform as D
@@ -598,6 +605,19 @@ class _DeformRun:
             inv = np.empty_like(perm); inv[perm] = np.arange(perm.size)
             tri = inv[tri].astype(np.int32)
             m0 = m0[perm]
+        self.scales = None
+        H = spec.get("scales")
+        if H is not None:
+            from . import deform_scales as DS
+            if not isinstance(H, DS.BoxHierarchy) or not H.matches(spec["tri"], nP):
+                raise ValueError("deform: scales must be a BoxHierarchy built on the same mesh (tri) and %d buoys" % nP)
+            # triangles keep the hierarchy's order (mapped to engine slots only): the sums do not depend on `perm`
+            self.scales = DS._DevicePlan(torch, dev, H, tri)
+            self.d_st = [self.scales.outputs() for _ in range(2)]
+            self.h_st = [self.scales.outputs(pin=True) for _ in range(2)]
+            self.DS, self.H = DS, H
+        self.scale_sink = spec.get("scale_sink")
+        self.scale_collected = [] if H is not None and self.scale_sink is None else None
         tri, self.inv = D.sort_mesh(tri)
         self.nT = tri.shape[0]
         self.dt = self.every * eng.rdt / 86400.0
@@ -624,6 +644,8 @@ class _DeformRun:
         yx = self.state_pos if self.row_f4 else yx_row
         self.D.launch(self.eng.L, self.eng.h, self.nT, self.tri_t, self.a_yx, self.a_mk, yx, mk_row, self.dt,
                       self.d_out[b], s_cmp)
+        if self.scales is not None:
+            self.scales.launch(self.eng.h, self.a_yx, self.a_mk, yx, mk_row, self.dt, *self.d_st[b], None, s_cmp)
         with torch.cuda.stream(s_cmp):                              # row (w+1)*every anchors the next window
             self.a_yx.copy_(yx)
             self.a_mk.copy_(mk_row)
@@ -633,6 +655,9 @@ class _DeformRun:
         s_out.wait_event(ev)
         with torch.cuda.stream(s_out):
             self.h_out[b].copy_(self.d_out[b], non_blocking=True)
+            if self.scales is not None:
+                for h, d in zip(self.h_st[b], self.d_st[b]):
+                    h.copy_(d, non_blocking=True)
         self.ev_out.append(torch.cuda.Event()); self.ev_out[w].record(s_out)
 
     def _drain(self, w):
@@ -643,6 +668,12 @@ class _DeformRun:
             self.collected.append(out)
         else:
             self.sink(w, out)
+        if self.scales is not None:
+            st = self.DS.stats_dict(self.H, *(h.numpy() for h in self.h_st[w % 2]))
+            if self.scale_sink is None:
+                self.scale_collected.append(st)
+            else:
+                self.scale_sink(w, st)
         self.drained = w + 1
 
     def finish(self):

@@ -21,7 +21,8 @@ from .util import epoch2clock as e2c
 
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
-           "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter"]
+           "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter",
+           "DeformationScalingWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -311,6 +312,92 @@ class DeformationWriter:
                 for fn in sorted(os.listdir(self._tmp)):
                     z.write(os.path.join(self._tmp, fn), arcname=fn)
             shutil.rmtree(self._tmp, ignore_errors=True)
+        print('      ===> ' + self.cf_out + ' saved!')
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DeformationScalingWriter:
+    """Window-by-window writer of the per-scale statistics of coarse-grained deformation (sitrack_b200.deform_scales,
+    TrackEngine.track's `deform` with `scales`).  Dimensions time (windows), scale, bin, bin_edge; variables
+      time_start, time_end (time) i4                       first and last date of each window [tunits]
+      scale_km (scale) f8                                  box side [km]; fillVal for the triangles (scale 0)
+      bin_edges (bin_edge) f8                              histogram edges [day-1]
+      n (time,scale) i8                                    cells (boxes or triangles) that count
+      L_eff, eps_tot, eps_tot2, eps_tot3 (time,scale) f8   means of sqrt(area) [km] and of eps_tot^q [day-q],
+                                                           fillVal where n = 0
+      hist_total, hist_divergence, hist_shear (time,scale,bin) i8   counts of eps_tot, |div|, shear per bin,
+                                                           bin k = [edge k-1, edge k), underflow and overflow first/last
+    with `units` on every variable.  netCDF4 when available and the name does not end in .npz; otherwise an .npz
+    with the same variables, plus `<name>_units` (0-d strings) and `FillValue` members for the attributes."""
+
+    MEANS = (("L_eff", "sum_L_eff", "km"), ("eps_tot", "sum_eps_tot", "day-1"), ("eps_tot2", "sum_eps_tot2", "day-2"),
+             ("eps_tot3", "sum_eps_tot3", "day-3"))
+    HISTS = ("hist_total", "hist_divergence", "hist_shear")
+
+    def __init__(self, cf_out, ntime, scale_km, bin_edges, tunits=tunits_default, fillVal=FillValue, corigin=None):
+        print('\n *** [DeformationScalingWriter]: About to generate file: ' + cf_out + ' ...')
+        scale_km, bin_edges = np.asarray(scale_km, 'f8'), np.asarray(bin_edges, 'f8')
+        self.ntime, self.ns, self.nbin = int(ntime), scale_km.size, bin_edges.size + 1
+        self.fill = fillVal
+        units = dict(time_start=tunits, time_end=tunits, scale_km='km', bin_edges='day-1', n='1',
+                     **{n: u for n, _, u in self.MEANS}, **{h: '1' for h in self.HISTS})
+        nc = None
+        if not str(cf_out).endswith(".npz"):
+            try:
+                import netCDF4 as nc
+            except ImportError:
+                cf_out += ".npz"
+                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
+        self.cf_out, self._nc = cf_out, nc
+        shapes = dict(time_start=('i4', ('time',)), time_end=('i4', ('time',)), n=('i8', ('time', 'scale')),
+                      **{n: ('f8', ('time', 'scale')) for n, _, _ in self.MEANS},
+                      **{h: ('i8', ('time', 'scale', 'bin')) for h in self.HISTS})
+        if nc is None:
+            size = dict(time=self.ntime, scale=self.ns, bin=self.nbin)
+            self._v = {n: np.zeros([size[d] for d in dims], dt) for n, (dt, dims) in shapes.items()}
+            self._v['scale_km'], self._v['bin_edges'] = scale_km, bin_edges
+            self._units = units
+        else:
+            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
+            f.createDimension('time', None)
+            f.createDimension('scale', self.ns)
+            f.createDimension('bin', self.nbin)
+            f.createDimension('bin_edge', bin_edges.size)
+            self._v = {}
+            for n, (dt, dims) in shapes.items():
+                self._v[n] = f.createVariable(n, dt, dims, **(dict(fill_value=fillVal) if dt == 'f8' else {}))
+            f.createVariable('scale_km', 'f8', ('scale',))[:] = scale_km
+            f.createVariable('bin_edges', 'f8', ('bin_edge',))[:] = bin_edges
+            for n, u in units.items():
+                f.variables[n].units = u
+            if corigin:
+                f.Origin = corigin
+            f.About = 'Per-scale statistics of sea-ice deformation coarse-grained over material boxes of buoy triangles'
+            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+
+    def write(self, jw, time_start, time_end, stats):
+        """Window jw: stats = the dict of sitrack_b200.CoarseGrainedRates / track(deform=dict(scales=...))."""
+        n = np.asarray(stats['n'], 'i8')
+        self._v['time_start'][jw] = time_start
+        self._v['time_end'][jw] = time_end
+        self._v['n'][jw, :] = n
+        with np.errstate(all='ignore'):
+            for name, key, _ in self.MEANS:
+                self._v[name][jw, :] = np.where(n > 0, np.asarray(stats[key], 'f8') / np.maximum(n, 1), self.fill)
+        for h in self.HISTS:
+            self._v[h][jw, :, :] = np.asarray(stats[h], 'i8')
+
+    def close(self):
+        if self._nc is not None:
+            self._f.close()
+        else:
+            extra = {n + '_units': np.array(u) for n, u in self._units.items()}
+            np.savez(self.cf_out, FillValue=np.float64(self.fill), **self._v, **extra)
         print('      ===> ' + self.cf_out + ' saved!')
 
     def __enter__(self):

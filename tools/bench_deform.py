@@ -14,6 +14,13 @@ loop runs after each window (device-to-device, f8 positions + mask) and the two-
 it replaces are timed the same way.  Byte model from shapes: 12 B of indices + 24 B of outputs per triangle,
 2 x (16 + 1) B of positions and masks per buoy.  A random sample of triangles is checked bit for bit against
 oracle/deform_ref.py.
+
+The coarse-graining pass (st_deform_scales_dev: level-1 box sums with the triangles' statistics, one parent pass per
+level, box statistics, final reduction) is timed the same way on the same rows, for --L0 km boxes and --levels
+levels, with statistics only (no box planes), as the record loop runs it.  Byte model: 12 B of indices per
+triangle, 2 x 17 B per buoy, 8 B of level-1 ranges per level-1 box and 64 B box records (written once, read by the
+parent and statistics passes).  The level-1 outputs of a random sample of boxes are checked bit for bit against
+oracle/deform_scale_ref.py, and two passes must give the same statistics bit for bit.
 """
 import argparse
 import json
@@ -79,6 +86,49 @@ def time_loop(torch, fn, seconds, warm=20):
     return e0.elapsed_time(e1) * 1e3 / n, n                          # us per call
 
 
+def scales(torch, a, rng, yx0, yx1, m0, m1, tri, dt, g, us_deform):
+    """Time and check the coarse-graining pass on the same rows."""
+    import time
+    from sitrack_b200 import deform_scales as DS
+    from oracle import deform_scale_ref as O
+    t0 = time.perf_counter()
+    H = DS.BoxHierarchy(yx0, tri, a.L0, a.levels)
+    t_build = time.perf_counter() - t0
+    nP, nT = yx0.shape[0], tri.shape[0]
+    plan = DS._DevicePlan(torch, torch.device("cuda", torch.cuda.current_device()), H, tri)
+    mom, hist = plan.outputs()
+    yx0_t, yx1_t, m0_t, m1_t = g(yx0), g(yx1), g(m0), g(m1)
+    s = torch.cuda.current_stream()
+    run = lambda: plan.launch(None, yx0_t, m0_t, yx1_t, m1_t, dt, mom, hist, None, s)
+    us, n = time_loop(torch, run, a.seconds)
+    m1_, h1_ = mom.cpu().numpy(), hist.cpu().numpy()
+    run()
+    same = bool(np.array_equal(m1_, mom.cpu().numpy()) and np.array_equal(h1_, hist.cpu().numpy()))
+    # level-1 outputs of a sample of boxes against the oracle (the box planes of one more pass)
+    boxes_t = torch.empty((7, int(H.nbox.sum())), dtype=torch.float32, device="cuda")
+    plan.launch(None, yx0_t, m0_t, yx1_t, m1_t, dt, mom, hist, boxes_t, s)
+    planes = boxes_t[:, :int(H.nbox[0])].cpu().numpy()
+    pick = np.sort(rng.choice(int(H.nbox[0]), min(20000, int(H.nbox[0])), replace=False))
+    lo, hi = H.tri_off[pick], H.tri_off[pick + 1]
+    ts = np.concatenate([H.order[i:j] for i, j in zip(lo, hi)])
+    off = np.r_[0, np.cumsum(hi - lo)]
+    T, _, _ = O.triangle_terms(yx0, yx1, m0, m1, tri[ts], dt)
+    o, ok = O.box_outputs(O.level1_sums(T, off), H.min_area[0])
+    with np.errstate(all="ignore"):
+        exact = all(np.array_equal(planes[j, pick], np.where(ok, o[k], O.FillValue).astype(np.float32))
+                    for j, k in enumerate(O.BOX_NAMES))
+    nb = H.nbox.astype(np.int64)
+    nball = int(nb.sum())
+    bytes_model = nT * 12 + nP * 2 * 17 + int(nb[0]) * 8 + 64 * (2 * nball + nball - int(nb[0]))
+    peak, _ = hbm_peak()
+    gbs = bytes_model / (us * 1e-6) / 1e9
+    return dict(us_per_window=round(us, 2), passes_timed=n, vs_k_deform=round(us / us_deform, 3), L0_km=a.L0,
+                levels=a.levels, boxes_per_level=nb.tolist(), host_build_s=round(t_build, 2),
+                bytes_model=dict(total=bytes_model, achieved_gbs=round(gbs, 1), frac_of_peak=round(gbs / peak, 4)),
+                n_per_scale=h1_[:, 0].sum(1).tolist(), sample_boxes=int(pick.size),
+                sample_boxes_bit_identical=bool(exact), run_to_run_identical=same)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--ny", type=int, default=3531)
@@ -86,6 +136,8 @@ def main():
     ap.add_argument("--seconds", type=float, default=1.0)
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--L0", type=float, default=12.0)
+    ap.add_argument("--levels", type=int, default=6)
     a = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -106,7 +158,7 @@ def main():
     us, n = time_loop(torch, run, a.seconds)
     # correctness on a random sample (the oracle is numpy: a sample, not all 25 M)
     out = out_t.cpu().numpy()
-    pick = np.sort(rng.choice(nT, 200000, replace=False))
+    pick = np.sort(rng.choice(nT, min(200000, nT), replace=False))
     ref = R.deform(yx0, yx1, m0, m1, tri[pick], dt)
     exact = all(np.array_equal(out[j, pick], ref[k]) for j, k in enumerate(R.NAMES))
     # the anchor copy after each window, and what moving two f8 rows to the host costs instead
@@ -120,6 +172,7 @@ def main():
     def d2h():
         h0.copy_(yx0_t, non_blocking=True); h1.copy_(yx1_t, non_blocking=True)
     us_d2h, n_d2h = time_loop(torch, d2h, a.seconds / 2, warm=3)
+    sc = scales(torch, a, rng, yx0, yx1, m0, m1, tri, dt, g, us)
     bytes_model = nT * (12 + 24) + nP * 2 * (16 + 1)
     peak, peak_src = hbm_peak()
     gbs = bytes_model / (us * 1e-6) / 1e9
@@ -133,14 +186,14 @@ def main():
                valid_fraction=float((out[0] != -9999.0).mean()),
                workload="jittered 3 km lattice %dx%d, 2 triangles per square, sorted by smallest vertex; "
                         "inputs larger than L2, no flush" % (a.ny, a.nx),
-               card=card_info(torch, dev))
+               scales=sc, card=card_info(torch, dev))
     line = json.dumps(res)
     print(line)
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
             f.write(line + "\n")
-    return 0 if exact else 1
+    return 0 if exact and sc["sample_boxes_bit_identical"] and sc["run_to_run_identical"] else 1
 
 
 if __name__ == "__main__":
