@@ -297,6 +297,41 @@ int  st_deform_scales_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, const
                           int64_t scratch_bytes, double *moments_dev, int64_t *hist_dev, float *boxes_dev,
                           void *stream);
 
+/* ---- deformation coarse-grained over a fixed Eulerian grid, rebuilt every window ----------------
+ * A grid of nj x ni (1..2^20 each) level-1 cells of side L0 km from the origin (oy, ox) km (DESIGN.md section 12,
+ * sit.EulerianGrid): cell (bj, bi) covers [oy + bj L0, oy + (bj+1) L0) x [ox + bi L0, ox + (bi+1) L0); level s
+ * (1..levels, levels 1..20) has side L0 2^(s-1), key (bj, bi) >> (s-1), nj_s = ((nj-1) >> (s-1)) + 1 rows and ni_s
+ * likewise.  tri_dev (nT,3) int32 is the mesh in the caller's triangle order (buoy indices as stored on the device).
+ * st_deform_grid_scratch_bytes gives the scratch st_deform_grid_dev needs (box records, moment partials, sort
+ * buffers, CUB's temporary storage, segmentation arrays); it checks its arguments before any CUDA call and then
+ * needs a device (CUB's size query).
+ * ASYNC st_deform_grid_dev: between two rows dt_days apart (positions and masks as st_deform_dev) a triangle is binned
+ * when it is valid by st_deform_dev's rule and its mid-time centroid lies in the grid (floor((Yc - oy)/L0) in
+ * [0, nj) compared in f8; NaN and inf never are).  Binned triangles are sorted stably by the Morton code of their
+ * level-1 key (ties in the caller's order) on the device; each level's boxes are the runs of that order, and the
+ * sums, box outputs, cover rule (area >= min_area[s], HOST (levels)), moments_dev and hist_dev are those of
+ * st_deform_scales_dev over these boxes (scale 0 = the binned triangles).  fields_dev (sum_s 7 nj_s ni_s) f4: per
+ * level, seven (nj_s, ni_s) planes divergence, shear, vorticity, eps_tot, L_eff, y_ctr, x_ctr, -9999 where a cell
+ * has no binned triangle or does not count; nbox_dev (levels) int64 the boxes per level.  The front of the scratch
+ * holds the f8 box records (8 doubles per box: a2, Nux, Nuy, Nvx, Nvy, NY, NX, pad), level s from the prefix sum of
+ * the bounds min(nT, nj_s ni_s).  Launch shapes depend on (nT, nj, ni, levels) only: bit-identical run to run.  No
+ * host synchronisation, no allocation; indices are not checked on the device.  Refuses nT < 1, dt_days <= 0 or
+ * NaN, a non-finite origin, L0 <= 0 and writes nothing then.                                               */
+int  st_deform_grid_scratch_bytes(int64_t nT, int levels, int nj, int ni, int nedge, int64_t *bytes);
+int  st_deform_grid_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, const double *yx0_dev, const int8_t *m0_dev,
+                        const double *yx1_dev, const int8_t *m1_dev, double dt_days, int levels, int nj, int ni,
+                        double oy, double ox, double L0, const double *min_area, int nedge, const double *edges_dev,
+                        void *scratch_dev, int64_t scratch_bytes, double *moments_dev, int64_t *hist_dev,
+                        float *fields_dev, int64_t *nbox_dev, void *stream);
+/* The same pass stopped after stage `upto` (1 cell keys, 2 sort, 3 segmentation, 4 everything = st_deform_grid_dev),
+ * for timing the stages with events; below 4 the outputs are not written.                                   */
+int  st_deform_grid_stages_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, const double *yx0_dev,
+                               const int8_t *m0_dev, const double *yx1_dev, const int8_t *m1_dev, double dt_days,
+                               int levels, int nj, int ni, double oy, double ox, double L0, const double *min_area,
+                               int nedge, const double *edges_dev, void *scratch_dev, int64_t scratch_bytes,
+                               double *moments_dev, int64_t *hist_dev, float *fields_dev, int64_t *nbox_dev, int upto,
+                               void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

@@ -64,6 +64,11 @@ def __argument_parsing__():
                         help='with --deform: also coarse-grain the triangles over LEVELS levels of material boxes of side '
                              'L0_KM * 2^s and write per-scale statistics (n, means of L_eff and eps_tot^q, histograms) '
                              'of every window into ./nc/..._deformation-scaling_...')
+    parser.add_argument('--deform-grid', type=float, nargs=2, default=None, metavar=('L0_KM', 'LEVELS'),
+                        help='with --deform: also coarse-grain the triangles over the fixed cells of a grid of side L0_KM * 2^s '
+                             '(LEVELS levels) covering the model\'s T-points, binned every window by mid-time centroid, and '
+                             'write per-level fields into ./nc/..._deformation-grid_... and per-scale statistics into '
+                             './nc/..._deformation-grid-scaling_...')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -156,6 +161,36 @@ def deform_scales_args(scales, hours):
     return L0, int(lev)
 
 
+def deform_grid_args(grid, hours):
+    """--deform-grid L0_KM LEVELS -> (L0_km, levels) or None; ERROR and exit without --deform, with L0 <= 0, or with
+    LEVELS not an integer in 1..20."""
+    if grid is None:
+        return None
+    L0, lev = grid
+    if hours is None:
+        print('ERROR: --deform-grid needs --deform HOURS')
+        exit(0)
+    if not L0 > 0:
+        print('ERROR: --deform-grid L0_KM must be positive, got %g' % L0)
+        exit(0)
+    if lev != int(lev) or not 1 <= lev <= sit.MAX_LEVELS:
+        print('ERROR: --deform-grid LEVELS must be an integer in 1..%d, got %g' % (sit.MAX_LEVELS, lev))
+        exit(0)
+    return L0, int(lev)
+
+
+def deform_grid_over(Yt, Xt, L0, levels):
+    """The EulerianGrid of side L0 covering the T-points (Yt, Xt) km: origin floor(min / L0) L0 and
+    floor((max - origin) / L0) + 1 cells per axis; ERROR and exit when that is more than 2^20 cells a side."""
+    origin = np.array([np.floor(np.min(Yt) / L0) * L0, np.floor(np.min(Xt) / L0) * L0])
+    shape = [int(np.floor((np.max(A) - o) / L0)) + 1 for A, o in ((Yt, origin[0]), (Xt, origin[1]))]
+    if max(shape) > sit.MAX_GRID_SIDE:
+        print('ERROR: --deform-grid L0_KM = %g gives %d x %d cells over the model grid, more than %d a side'
+              % (L0, shape[0], shape[1], sit.MAX_GRID_SIDE))
+        exit(0)
+    return sit.EulerianGrid(origin, L0, shape, levels)
+
+
 def main():
     print('\n##########################################################')
     print('#            SITRACK ICE PARTICULES TRACKER              #')
@@ -165,6 +200,7 @@ def main():
     args = __argument_parsing__()
     ndeform = deform_records(args.deform, world)
     dscales = deform_scales_args(args.deform_scales, args.deform)
+    dgrid = deform_grid_args(args.deform_grid, args.deform)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
@@ -197,6 +233,7 @@ def main():
     imaskt, xlatT, xlonT, xYt, xXt, xYf, xXf, xResKM = sit.GetModelGrid(cf_mm)
     xYv, xXv, xYu, xXu = sit.GetModelUVGrid(cf_mm) if args.uvstrategy == 1 else (None, None, None, None)
     (Nj, Ni) = np.shape(imaskt)
+    G = deform_grid_over(xYt, xXt, *dgrid) if dgrid else None
 
     ds = sit.open_dataset(cf_uv)
     vU, vV, vIC = ds.variables['u_ice'], ds.variables['v_ice'], ds.variables['siconc']
@@ -330,6 +367,18 @@ def main():
             swriter = sit.DeformationScalingWriter(cf_sc, nwin, H.scale_km, H.bin_edges, corigin=corgn)
             deform.update(scales=H, scale_sink=lambda w, st: swriter.write(w, vTime[w * ndeform],
                                                                           vTime[(w + 1) * ndeform], st))
+        if G is not None:
+            # fixed cells over the model grid, membership rebuilt every window; only fields and statistics leave the GPU
+            print(' *** --deform-grid: %d levels of cells from %g km, %d x %d level-1 cells from (%g, %g) km'
+                  % (G.levels, G.L0_km, G.shape[0], G.shape[1], G.origin[0], G.origin[1]))
+            gwriter = sit.DeformationGridWriter('./nc/' + corgn + '_deformation-grid_' + cf_tail, nwin, G, corigin=corgn)
+            gswriter = sit.DeformationScalingWriter('./nc/' + corgn + '_deformation-grid-scaling_' + cf_tail, nwin,
+                                                    G.scale_km, G.bin_edges, corigin=corgn)
+
+            def grid_sink(w, fields, st):
+                gwriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], fields)
+                gswriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], st)
+            deform.update(grid=G, grid_sink=grid_sink)
         small = False                                             # windows close inside the streaming record loop
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
@@ -345,6 +394,9 @@ def main():
         dwriter.close()
         if dscales:
             swriter.close()
+        if G is not None:
+            gwriter.close()
+            gswriter.close()
     ds.close()
     n_alive = res['n_alive']
     if world > 1:

@@ -78,6 +78,11 @@ SIGNATURES = {
     "st_deform_scales_scratch_bytes": (c_int, [c_i64, c_int, vp, vp, c_int, vp]),
     "st_deform_scales_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, vp, c_dbl, c_int, vp, vp, vp, vp, c_int, vp, vp, c_i64,
                                      vp, vp, vp, vp]),
+    "st_deform_grid_scratch_bytes": (c_int, [c_i64, c_int, c_int, c_int, c_int, vp]),
+    "st_deform_grid_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, vp, c_dbl, c_int, c_int, c_int, c_dbl, c_dbl, c_dbl, vp,
+                                   c_int, vp, vp, c_i64, vp, vp, vp, vp, vp]),
+    "st_deform_grid_stages_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, vp, c_dbl, c_int, c_int, c_int, c_dbl, c_dbl, c_dbl,
+                                          vp, c_int, vp, vp, c_i64, vp, vp, vp, vp, c_int, vp]),
     "st_xy2latlon": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_latlon2xy": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_xy2latlon_dev": (c_int, [c_i64, vp, vp, c_dbl, c_dbl, vp]),

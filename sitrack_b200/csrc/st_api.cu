@@ -1206,6 +1206,60 @@ int st_deform_scales_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double
     return ST_OK;
 }
 
+// ---- deformation coarse-grained over a fixed Eulerian grid, rebuilt every window (st_deform_grid.cu) ----
+int st_deform_grid_scratch_bytes(int64_t nT, int levels, int nj, int ni, int nedge, int64_t* bytes)
+{
+    if (!bytes) return fail(nullptr, ST_EINVAL, "st_deform_grid_scratch_bytes: NULL argument");
+    GridPlan g;
+    if (const char* why = grid_plan(nT, levels, nj, ni, nullptr, nedge, &g))
+        return fail(nullptr, ST_EINVAL, std::string("st_deform_grid_scratch_bytes: ") + why);
+    CU(nullptr, grid_plan_cub(&g));
+    *bytes = g.bytes;
+    return ST_OK;
+}
+
+int st_deform_grid_stages_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double* yx0, const int8_t* m0,
+                              const double* yx1, const int8_t* m1, double dt_days, int levels, int nj, int ni,
+                              double oy, double ox, double L0, const double* min_area, int nedge, const double* edges,
+                              void* scratch, int64_t scratch_bytes, double* moments, int64_t* hist, float* fields,
+                              int64_t* nbox, int upto, void* stream)
+{
+    if (upto < GR_STAGE_KEY || upto > GR_STAGE_ALL) return fail(c, ST_EINVAL, "st_deform_grid_stages_dev: upto must be in 1..4");
+    GridPlan g;
+    if (const char* why = grid_plan(nT, levels, nj, ni, min_area, nedge, &g))
+        return fail(c, ST_EINVAL, std::string("st_deform_grid_dev: ") + why);
+    if (!tri || !yx0 || !m0 || !yx1 || !m1 || !min_area || !edges || !scratch || !moments || !hist || !fields || !nbox)
+        return fail(c, ST_EINVAL, "st_deform_grid_dev: NULL argument");
+    if ((uintptr_t)tri % 4 || (uintptr_t)yx0 % 16 || (uintptr_t)yx1 % 16 || (uintptr_t)scratch % 256 ||
+        (uintptr_t)edges % 8 || (uintptr_t)moments % 8 || (uintptr_t)hist % 8 || (uintptr_t)nbox % 8 ||
+        (uintptr_t)fields % 4)
+        return fail(c, ST_EINVAL, "st_deform_grid_dev: yx0 and yx1 must be 16-byte aligned, scratch 256-byte, "
+                                  "edges, moments, hist and nbox 8-byte, tri and fields 4-byte");
+    for (int l = 0; l < levels; ++l)
+        if (!(min_area[l] > 0.0)) return fail(c, ST_EINVAL, "st_deform_grid_dev: min_area must be positive");
+    if (!(isfinite(L0) && L0 > 0.0)) return fail(c, ST_EINVAL, "st_deform_grid_dev: L0 must be finite and positive");
+    if (!isfinite(oy) || !isfinite(ox)) return fail(c, ST_EINVAL, "st_deform_grid_dev: the origin must be finite");
+    if (!(dt_days > 0.0)) return fail(c, ST_EINVAL, "st_deform_grid_dev: dt_days must be positive");
+    if (c) CU(c, cudaSetDevice(c->device));
+    CU(c, grid_plan_cub(&g));
+    if (scratch_bytes < g.bytes)
+        return fail(c, ST_EINVAL, "st_deform_grid_dev: scratch_bytes is smaller than st_deform_grid_scratch_bytes");
+    CU(c, launch_deform_grid(g, tri, (const pt*)yx0, m0, (const pt*)yx1, m1, dt_days, oy, ox, L0, edges, scratch,
+                             moments, hist, fields, reinterpret_cast<long long*>(nbox), upto, (cudaStream_t)stream));
+    return ST_OK;
+}
+
+int st_deform_grid_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double* yx0, const int8_t* m0,
+                       const double* yx1, const int8_t* m1, double dt_days, int levels, int nj, int ni, double oy,
+                       double ox, double L0, const double* min_area, int nedge, const double* edges, void* scratch,
+                       int64_t scratch_bytes, double* moments, int64_t* hist, float* fields, int64_t* nbox,
+                       void* stream)
+{
+    return st_deform_grid_stages_dev(c, nT, tri, yx0, m0, yx1, m1, dt_days, levels, nj, ni, oy, ox, L0, min_area,
+                                     nedge, edges, scratch, scratch_bytes, moments, hist, fields, nbox, GR_STAGE_ALL,
+                                     stream);
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

@@ -16,6 +16,9 @@
 //
 // Kernels, all on the caller's stream: k_scale_l1 (level-1 box sums + scale-0 statistics), k_scale_parent (one
 // launch per coarser level), k_scale_stats (box outputs, validity, statistics of every level), k_scale_final.
+// DEV = false: box counts from the ScalePlan (material boxes, built on the host).  DEV = true: box counts from device
+// memory (dnbox, Eulerian boxes segmented on the device, st_deform_grid.cu); the ScalePlan then holds upper bounds of
+// them, so launch grids, box record layout and moment partials depend on the bounds only.
 #include "st_deform.cuh"
 
 namespace st {
@@ -103,19 +106,21 @@ __device__ __forceinline__ void stats_flush(StatAcc a, int blk, int scale, int n
 }
 
 // Level-1 box sums (one warp per box, boxes grid-strided over the warps) and the scale-0 statistics.
+template <bool DEV>
 __global__ void __launch_bounds__(SC_BLOCK) k_scale_l1(ScalePlan p, const long long* __restrict__ tri_off,
                                                        const int* __restrict__ tri,
                                                        const pt* __restrict__ yx0, const int8_t* __restrict__ m0,
                                                        const pt* __restrict__ yx1, const int8_t* __restrict__ m1,
                                                        double dt, const double* __restrict__ edges,
                                                        double* __restrict__ box, double* __restrict__ part,
-                                                       unsigned long long* __restrict__ hist)
+                                                       unsigned long long* __restrict__ hist,
+                                                       const long long* __restrict__ dnbox)
 {
     double* e; int* cnt;
     stats_smem_init(edges, p.nedge, p.nbin, e, cnt);
     const int lane = threadIdx.x & 31;
     StatAcc st; st.zero();
-    const long long nbox = p.nbox[0];
+    const long long nbox = DEV ? dnbox[0] : p.nbox[0];
     for (long long b = (long long)blockIdx.x * SC_WARPS + (threadIdx.x >> 5); b < nbox; b += (long long)gridDim.x * SC_WARPS) {
         const long long t1 = tri_off[b + 1];
         double acc[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
@@ -168,11 +173,13 @@ __global__ void __launch_bounds__(SC_BLOCK) k_scale_l1(ScalePlan p, const long l
 }
 
 // Level s+1 from level s: thread per parent box, ((c0 + c1) + c2) + c3 over its children in Morton order.
+template <bool DEV>
 __global__ void __launch_bounds__(SC_BLOCK) k_scale_parent(long long n, const long long* __restrict__ coff,
-                                                           const double* __restrict__ child, double* __restrict__ parent)
+                                                           const double* __restrict__ child, double* __restrict__ parent,
+                                                           const long long* __restrict__ dn)
 {
     const long long i = (long long)blockIdx.x * SC_BLOCK + threadIdx.x;
-    if (i >= n) return;
+    if (i >= (DEV ? *dn : n)) return;
     double acc[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     const long long c1 = coff[i + 1];
     for (long long c = coff[i]; c < c1; ++c) {
@@ -185,10 +192,11 @@ __global__ void __launch_bounds__(SC_BLOCK) k_scale_parent(long long n, const lo
 
 // Box outputs, validity and statistics of every level >= 1; the blocks [blk0[s], blk0[s+1]) serve scale s.
 // out (optional): seven f4 planes over all boxes [divergence | shear | vorticity | total | L_eff | y_ctr | x_ctr].
+template <bool DEV>
 __global__ void __launch_bounds__(SC_BLOCK) k_scale_stats(ScalePlan p, const double* __restrict__ box,
                                                           const double* __restrict__ edges, double* __restrict__ part,
                                                           unsigned long long* __restrict__ hist, float* __restrict__ out,
-                                                          long long nbox_all)
+                                                          long long nbox_all, const long long* __restrict__ dnbox)
 {
     double* e; int* cnt;
     stats_smem_init(edges, p.nedge, p.nbin, e, cnt);
@@ -196,7 +204,7 @@ __global__ void __launch_bounds__(SC_BLOCK) k_scale_stats(ScalePlan p, const dou
     int s = 1;
     while (s < p.levels && gb >= p.blk0[s + 1]) ++s;
     const int lv = s - 1;
-    const long long nb = p.nbox[lv], first = p.box0[lv];
+    const long long nb = DEV ? dnbox[lv] : p.nbox[lv], first = p.box0[lv];
     const long long stride = (long long)(p.blk0[s + 1] - p.blk0[s]) * SC_BLOCK;
     const double thr = p.min_area[lv];
     StatAcc st; st.zero();
@@ -283,10 +291,11 @@ long long scale_plan(int levels, const long long* nbox, const double* min_area, 
 
 size_t scale_smem(const ScalePlan& p) { return (size_t)p.nedge * sizeof(double) + (size_t)3 * p.nbin * sizeof(int); }
 
-cudaError_t launch_deform_scales(const ScalePlan& p, const int32_t* tri, const long long* tri_off,
+template <bool DEV>
+static cudaError_t launch_scales(const ScalePlan& p, const int32_t* tri, const long long* tri_off,
                                  const long long* child_off, const pt* yx0, const int8_t* m0, const pt* yx1,
                                  const int8_t* m1, double dt, const double* edges, void* scratch, double* mom,
-                                 int64_t* hist, float* out, cudaStream_t st)
+                                 int64_t* hist, float* out, const long long* dnbox, cudaStream_t st)
 {
     double* box = static_cast<double*>(scratch);
     double* part = box + SC_BOX * p.nbox_all;
@@ -295,17 +304,37 @@ cudaError_t launch_deform_scales(const ScalePlan& p, const int32_t* tri, const l
     cudaError_t e = cudaMemsetAsync(hist, 0, sizeof(int64_t) * 3 * (size_t)p.nbin * (p.levels + 1), st);
     if (e != cudaSuccess) return e;
     if (smem > 48 * 1024) {
-        if ((e = cudaFuncSetAttribute(k_scale_l1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess ||
-            (e = cudaFuncSetAttribute(k_scale_stats, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+        if ((e = cudaFuncSetAttribute(k_scale_l1<DEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess ||
+            (e = cudaFuncSetAttribute(k_scale_stats<DEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
             return e;
     }
-    k_scale_l1<<<p.blk0[1], SC_BLOCK, smem, st>>>(p, tri_off, tri, yx0, m0, yx1, m1, dt, edges, box, part, h);
+    k_scale_l1<DEV><<<p.blk0[1], SC_BLOCK, smem, st>>>(p, tri_off, tri, yx0, m0, yx1, m1, dt, edges, box, part, h, dnbox);
     for (int l = 1; l < p.levels; ++l)
-        k_scale_parent<<<(unsigned)((p.nbox[l] + SC_BLOCK - 1) / SC_BLOCK), SC_BLOCK, 0, st>>>(
-            p.nbox[l], child_off + p.child0[l], box + SC_BOX * p.box0[l - 1], box + SC_BOX * p.box0[l]);
-    k_scale_stats<<<p.blk0[p.levels + 1] - p.blk0[1], SC_BLOCK, smem, st>>>(p, box, edges, part, h, out, p.nbox_all);
+        k_scale_parent<DEV><<<(unsigned)((p.nbox[l] + SC_BLOCK - 1) / SC_BLOCK), SC_BLOCK, 0, st>>>(
+            p.nbox[l], child_off + p.child0[l], box + SC_BOX * p.box0[l - 1], box + SC_BOX * p.box0[l],
+            DEV ? dnbox + l : nullptr);
+    k_scale_stats<DEV><<<p.blk0[p.levels + 1] - p.blk0[1], SC_BLOCK, smem, st>>>(p, box, edges, part, h, out,
+                                                                                 p.nbox_all, dnbox);
     k_scale_final<<<p.levels + 1, SC_BLOCK, 0, st>>>(p, part, mom);
     return cudaGetLastError();
+}
+
+cudaError_t launch_deform_scales(const ScalePlan& p, const int32_t* tri, const long long* tri_off,
+                                 const long long* child_off, const pt* yx0, const int8_t* m0, const pt* yx1,
+                                 const int8_t* m1, double dt, const double* edges, void* scratch, double* mom,
+                                 int64_t* hist, float* out, cudaStream_t st)
+{
+    return launch_scales<false>(p, tri, tri_off, child_off, yx0, m0, yx1, m1, dt, edges, scratch, mom, hist, out,
+                                nullptr, st);
+}
+
+cudaError_t launch_deform_scales_devcount(const ScalePlan& p, const int32_t* tri, const long long* tri_off,
+                                          const long long* child_off, const pt* yx0, const int8_t* m0, const pt* yx1,
+                                          const int8_t* m1, double dt, const double* edges, void* scratch, double* mom,
+                                          int64_t* hist, float* out, const long long* dnbox, cudaStream_t st)
+{
+    return launch_scales<true>(p, tri, tri_off, child_off, yx0, m0, yx1, m1, dt, edges, scratch, mom, hist, out,
+                               dnbox, st);
 }
 
 }  // namespace st

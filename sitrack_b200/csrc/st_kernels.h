@@ -193,5 +193,49 @@ cudaError_t launch_deform_scales(const ScalePlan& p, const int32_t* tri, const l
                                  const long long* child_off, const pt* yx0, const int8_t* m0, const pt* yx1,
                                  const int8_t* m1, double dt, const double* edges, void* scratch, double* mom,
                                  int64_t* hist, float* out, cudaStream_t st);
+// The same pass with the box counts in device memory (dnbox, levels); p.nbox then holds upper bounds of them, which
+// fix the launch grids, the box record layout and the moment partials.
+cudaError_t launch_deform_scales_devcount(const ScalePlan& p, const int32_t* tri, const long long* tri_off,
+                                          const long long* child_off, const pt* yx0, const int8_t* m0, const pt* yx1,
+                                          const int8_t* m1, double dt, const double* edges, void* scratch, double* mom,
+                                          int64_t* hist, float* out, const long long* dnbox, cudaStream_t st);
+
+// ---- coarse-grained deformation over a fixed Eulerian grid, rebuilt every window (st_deform_grid.cu) ----
+constexpr int GR_MAX_SIDE = 1 << 20;           // level-1 cells a side
+
+// Shapes of one grid pass (host only): per-level bounds, field offsets and the scratch layout, in bytes from the
+// front of the scratch.  Layout (every region 256-byte aligned):
+//   box    8 * sum(bound) f8 box records, level s at box0[s] (the ScalePlan's; as st_deform_scale.cu), then the
+//          moment partials 4 * blk0[levels+1] f8;
+//   planes 7 * sum(bound) f4 box outputs (k_scale_stats' planes over the bounds);
+//   code   sum(bound) u64 Morton codes of the boxes' keys at their own level, level s at box0[s];
+//   off    level-1 ranges of the sorted triangles (bound[0]+1) i8, then the child ranges of levels 2.. (bound+1 each);
+//   nbin   1 i8, the number of binned triangles;
+//   flag, pos  nT i4 run-head flags and their exclusive scan;
+//   kin, kout  nT u64 sort keys;  vin, vout  nT i4 sort values (caller's triangle index);
+//   tri    3 * nT i4, the binned triangles' rows in hierarchy order;
+//   cub    temporary storage of the sort and the scans.
+struct GridPlan {
+    ScalePlan sp;                               // nbox = the bounds min(nT, nj_s * ni_s)
+    long long nT;
+    int levels, nj, ni, end_bit;
+    int nj_s[SC_MAX_LEVELS], ni_s[SC_MAX_LEVELS];
+    long long field0[SC_MAX_LEVELS + 1];        // f4 offset of each level's seven planes in the field buffer
+    long long o_box, o_planes, o_code, o_off, o_nbin, o_flag, o_pos, o_kin, o_kout, o_vin, o_vout, o_tri, o_cub;
+    size_t cub_bytes;
+    long long bytes;
+};
+
+// Fills *g (shapes, layout without CUB's part); 0 on success, else the argument that is out of range.
+const char* grid_plan(long long nT, int levels, int nj, int ni, const double* min_area, int nedge, GridPlan* g);
+// CUB's temporary storage (a device query); completes g->cub_bytes and g->bytes.
+cudaError_t grid_plan_cub(GridPlan* g);
+// tri (nT,3) caller's triangle order; fields sum_s 7 nj_s ni_s f4; nbox (levels) i8 out.  upto < GR_STAGE_ALL
+// stops after that stage (stage timing only: the outputs are then not written).
+enum { GR_STAGE_KEY = 1, GR_STAGE_SORT = 2, GR_STAGE_SEGMENT = 3, GR_STAGE_ALL = 4 };
+cudaError_t launch_deform_grid(const GridPlan& g, const int32_t* tri, const pt* yx0, const int8_t* m0, const pt* yx1,
+                               const int8_t* m1, double dt, double oy, double ox, double L0, const double* edges,
+                               void* scratch, double* mom, int64_t* hist, float* fields, long long* nbox,
+                               int upto, cudaStream_t st);
 
 }  // namespace st

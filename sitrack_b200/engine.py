@@ -451,6 +451,11 @@ class TrackEngine:
         as each window closes the deformation of its boxes is reduced on the device to per-scale statistics
         (sitrack_b200.deform_scales), and only those reach the host: scale_sink(w, stats), or with scale_sink None
         the list of them under "deform_scales".  They do not depend on the order the buoys are stored in.
+        deform may also hold grid=EulerianGrid and grid_sink=callable or None, with or without scales: as each window
+        closes its triangles are binned into the grid's fixed cells by their mid-time centroid and coarse-grained on
+        the device (sitrack_b200.deform_grid); only the fields and statistics reach the host: grid_sink(w, fields,
+        stats), or with grid_sink None the list of (fields, stats) under "deform_grid".  They do not depend on the
+        order the buoys are stored in either.
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -565,6 +570,8 @@ class TrackEngine:
         extra = {} if dfm is None or dfm.collected is None else dict(deform=dfm.collected)
         if dfm is not None and dfm.scale_collected is not None:
             extra["deform_scales"] = dfm.scale_collected
+        if dfm is not None and dfm.grid_collected is not None:
+            extra["deform_grid"] = dfm.grid_collected
         if not keep:
             return dict(n_alive=n_alive, **extra)
         posC, posG, mask = posC.numpy(), posG.numpy(), mask.numpy()
@@ -583,7 +590,9 @@ class _DeformRun:
     device state (steps with f4 rows do not chain, so it is current after every step).  Triangles are mapped into
     engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs go back to the
     caller's triangle order on the host.  With `scales`, the box hierarchy pass runs on the same rows after k_deform
-    and before the anchor copy; its statistics go to the host on the output stream alongside the triangles'."""
+    and before the anchor copy; its statistics go to the host on the output stream alongside the triangles'.  With
+    `grid`, the Eulerian grid pass follows on the same rows, over the triangles in the caller's order (mapped to
+    engine slots), and its fields and statistics go to the host the same way."""
 
     def __init__(self, eng, torch, dev, spec, rec_first, kstrt, row_f4):
         from . import deform as D
@@ -618,6 +627,20 @@ class _DeformRun:
             self.DS, self.H = DS, H
         self.scale_sink = spec.get("scale_sink")
         self.scale_collected = [] if H is not None and self.scale_sink is None else None
+        self.grid = None
+        G = spec.get("grid")
+        if G is not None:
+            from . import deform_grid as DG
+            if not isinstance(G, DG.EulerianGrid):
+                raise ValueError("deform: grid must be an EulerianGrid")
+            # caller's triangle order (mapped to engine slots only): ties of the sort, hence the sums, do not depend
+            # on `perm`
+            self.grid = DG._GridPlan(torch, dev, G, tri)
+            self.d_gr = [self.grid.outputs() for _ in range(2)]
+            self.h_gr = [self.grid.outputs(pin=True) for _ in range(2)]
+            self.DG, self.G = DG, G
+        self.grid_sink = spec.get("grid_sink")
+        self.grid_collected = [] if G is not None and self.grid_sink is None else None
         tri, self.inv = D.sort_mesh(tri)
         self.nT = tri.shape[0]
         self.dt = self.every * eng.rdt / 86400.0
@@ -646,6 +669,8 @@ class _DeformRun:
                       self.d_out[b], s_cmp)
         if self.scales is not None:
             self.scales.launch(self.eng.h, self.a_yx, self.a_mk, yx, mk_row, self.dt, *self.d_st[b], None, s_cmp)
+        if self.grid is not None:
+            self.grid.launch(self.eng.h, self.a_yx, self.a_mk, yx, mk_row, self.dt, *self.d_gr[b], s_cmp)
         with torch.cuda.stream(s_cmp):                              # row (w+1)*every anchors the next window
             self.a_yx.copy_(yx)
             self.a_mk.copy_(mk_row)
@@ -657,6 +682,9 @@ class _DeformRun:
             self.h_out[b].copy_(self.d_out[b], non_blocking=True)
             if self.scales is not None:
                 for h, d in zip(self.h_st[b], self.d_st[b]):
+                    h.copy_(d, non_blocking=True)
+            if self.grid is not None:
+                for h, d in zip(self.h_gr[b], self.d_gr[b]):
                     h.copy_(d, non_blocking=True)
         self.ev_out.append(torch.cuda.Event()); self.ev_out[w].record(s_out)
 
@@ -674,6 +702,13 @@ class _DeformRun:
                 self.scale_collected.append(st)
             else:
                 self.scale_sink(w, st)
+        if self.grid is not None:
+            mom, hist, fields, _ = (h.numpy() for h in self.h_gr[w % 2])
+            fl, st = self.DG.split_fields(self.G, fields), self.DG.stats_dict(self.G, mom, hist)
+            if self.grid_sink is None:
+                self.grid_collected.append((fl, st))
+            else:
+                self.grid_sink(w, fl, st)
         self.drained = w + 1
 
     def finish(self):

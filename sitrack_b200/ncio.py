@@ -22,7 +22,7 @@ from .util import epoch2clock as e2c
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
            "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter",
-           "DeformationScalingWriter"]
+           "DeformationScalingWriter", "DeformationGridWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -398,6 +398,113 @@ class DeformationScalingWriter:
         else:
             extra = {n + '_units': np.array(u) for n, u in self._units.items()}
             np.savez(self.cf_out, FillValue=np.float64(self.fill), **self._v, **extra)
+        print('      ===> ' + self.cf_out + ' saved!')
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DeformationGridWriter:
+    """Window-by-window writer of deformation coarse-grained over the cells of a fixed Eulerian grid
+    (sitrack_b200.deform_grid, TrackEngine.track's `deform` with `grid`).  Dimensions time (windows) and, per level
+    s = 1..levels, y<s>, x<s>; variables
+      time_start, time_end (time) i4                       first and last date of each window [tunits]
+      y<s> (y<s>), x<s> (x<s>) f8                          cell-centre coordinates [km] on the tracking plane
+      <name>_<s> (time,y<s>,x<s>) f4                       divergence, shear, vorticity, total [day-1], L_eff [km],
+                                                           y_ctr, x_ctr [km]; fillVal where the cell does not count
+    with `units` on every variable and the attributes L_km (cell side per level), cover and origin ([y, x] km of the
+    grid's corner); corigin, if given, as `Origin`.  netCDF4 when available and the name does not end in .npz;
+    otherwise an .npz with the same variables, plus `L_km`, `cover`, `origin`, `<name>_units` (0-d strings) and
+    `FillValue` members, assembled from on-disk .npy members like DeformationWriter's."""
+
+    UNITS = dict(divergence='day-1', shear='day-1', vorticity='day-1', total='day-1', L_eff='km', y_ctr='km',
+                 x_ctr='km')
+
+    def __init__(self, cf_out, ntime, G, tunits=tunits_default, fillVal=FillValue, corigin=None):
+        from .deform_scales import BOX_NAMES
+        print('\n *** [DeformationGridWriter]: About to generate file: ' + cf_out + ' ...')
+        self.ntime, self.levels, self.names = int(ntime), G.levels, BOX_NAMES
+        self.var = lambda n, s: '%s_%d' % (n, s + 1)
+        nc = None
+        if not str(cf_out).endswith(".npz"):
+            try:
+                import netCDF4 as nc
+            except ImportError:
+                cf_out += ".npz"
+                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
+        self.cf_out, self._nc = cf_out, nc
+        units = dict(time_start=tunits, time_end=tunits)
+        for s in range(G.levels):
+            units['y%d' % (s + 1)] = units['x%d' % (s + 1)] = 'km'
+            units.update({self.var(n, s): self.UNITS[n] for n in self.names})
+        if nc is None:
+            import tempfile
+            self._tmp = tempfile.mkdtemp(prefix=".deform_grid_", dir=os.path.dirname(os.path.abspath(cf_out)) or ".")
+            mm = lambda n, dt, shp: np.lib.format.open_memmap(os.path.join(self._tmp, n + ".npy"), mode='w+', dtype=dt, shape=shp)
+            self._v = {'time_start': mm('time_start', 'i4', (self.ntime,)), 'time_end': mm('time_end', 'i4', (self.ntime,))}
+            for s, (nj, ni) in enumerate(G.shapes):
+                y, x = G.centres(s)
+                np.save(os.path.join(self._tmp, 'y%d.npy' % (s + 1)), y)
+                np.save(os.path.join(self._tmp, 'x%d.npy' % (s + 1)), x)
+                for n in self.names:
+                    self._v[self.var(n, s)] = mm(self.var(n, s), 'f4', (self.ntime, nj, ni))
+            for n, u in units.items():
+                np.save(os.path.join(self._tmp, n + "_units.npy"), np.array(u))
+            np.save(os.path.join(self._tmp, "L_km.npy"), np.asarray(G.L_km, 'f8'))
+            np.save(os.path.join(self._tmp, "cover.npy"), np.float64(G.cover))
+            np.save(os.path.join(self._tmp, "origin.npy"), np.asarray(G.origin, 'f8'))
+            np.save(os.path.join(self._tmp, "FillValue.npy"), np.float32(fillVal))
+        else:
+            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
+            f.createDimension('time', None)
+            self._v = {}
+            for n in ('time_start', 'time_end'):
+                self._v[n] = f.createVariable(n, 'i4', ('time',))
+            zkw = dict(zlib=True, complevel=9)
+            for s, (nj, ni) in enumerate(G.shapes):
+                dy, dx = 'y%d' % (s + 1), 'x%d' % (s + 1)
+                f.createDimension(dy, nj)
+                f.createDimension(dx, ni)
+                y, x = G.centres(s)
+                self._v[dy] = f.createVariable(dy, 'f8', (dy,)); self._v[dy][:] = y
+                self._v[dx] = f.createVariable(dx, 'f8', (dx,)); self._v[dx][:] = x
+                for n in self.names:
+                    self._v[self.var(n, s)] = f.createVariable(self.var(n, s), 'f4', ('time', dy, dx),
+                                                               fill_value=fillVal, **zkw)
+            for n, u in units.items():
+                self._v[n].units = u
+            f.L_km = np.asarray(G.L_km, 'f8')
+            f.cover = float(G.cover)
+            f.origin = np.asarray(G.origin, 'f8')
+            if corigin:
+                f.Origin = corigin
+            f.About = 'Sea-ice deformation of buoy triangles coarse-grained over the cells of a fixed grid'
+            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+
+    def write(self, jw, time_start, time_end, fields):
+        """Window jw: fields = per level dicts of (nj_s, ni_s) planes (sitrack_b200.GriddedRates, track's grid_sink)."""
+        self._v['time_start'][jw] = time_start
+        self._v['time_end'][jw] = time_end
+        for s in range(self.levels):
+            for n in self.names:
+                self._v[self.var(n, s)][jw, :, :] = np.asarray(fields[s][n], dtype=np.float32)
+
+    def close(self):
+        if self._nc is not None:
+            self._f.close()
+        else:
+            import shutil
+            import zipfile
+            for v in self._v.values():
+                v.flush()
+            self._v = {}
+            with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
+                for fn in sorted(os.listdir(self._tmp)):
+                    z.write(os.path.join(self._tmp, fn), arcname=fn)
+            shutil.rmtree(self._tmp, ignore_errors=True)
         print('      ===> ' + self.cf_out + ' saved!')
 
     def __enter__(self):

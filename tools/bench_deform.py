@@ -21,6 +21,13 @@ levels, with statistics only (no box planes), as the record loop runs it.  Byte 
 triangle, 2 x 17 B per buoy, 8 B of level-1 ranges per level-1 box and 64 B box records (written once, read by the
 parent and statistics passes).  The level-1 outputs of a random sample of boxes are checked bit for bit against
 oracle/deform_scale_ref.py, and two passes must give the same statistics bit for bit.
+
+The Eulerian grid pass (st_deform_grid_dev: cell keys, device radix sort, segmentation, the same box passes, field
+scatter) is timed the same way in the same run, on a grid of --L0 km cells and --levels levels covering the lattice
+at mid-time, with its statistics and dense fields as the record loop runs it.  The cumulative stages (keys; keys +
+sort; keys + sort + segmentation; the whole pass) are timed as well through st_deform_grid_stages_dev, so key, sort
+and segmentation times are differences of event timings.  The fields of a random sample of level-1 cells are
+checked bit for bit against oracle/deform_grid_ref.py, and two passes must give the same statistics and fields.
 """
 import argparse
 import json
@@ -129,6 +136,70 @@ def scales(torch, a, rng, yx0, yx1, m0, m1, tri, dt, g, us_deform):
                 sample_boxes_bit_identical=bool(exact), run_to_run_identical=same)
 
 
+def grid(torch, a, rng, yx0, yx1, m0, m1, tri, dt, g, us_deform, us_scales):
+    """Time and check the Eulerian grid pass on the same rows."""
+    import ctypes as C
+    import sitrack_b200 as sit
+    from sitrack_b200 import deform_grid as DG
+    from sitrack_b200._lib import check
+    from oracle import deform_scale_ref as O
+    from oracle import deform_grid_ref as OG
+    L0 = a.L0
+    mid = 0.5 * (yx0 + yx1)
+    origin = np.floor(mid.min(0) / L0) * L0
+    shape = tuple(int(n) for n in np.floor((mid.max(0) - origin) / L0) + 1)
+    G = sit.EulerianGrid(origin, L0, shape, a.levels)
+    plan = DG._GridPlan(torch, torch.device("cuda", torch.cuda.current_device()), G, tri)
+    mom, hist, fields, nbox = plan.outputs()
+    yx0_t, yx1_t, m0_t, m1_t = g(yx0), g(yx1), g(m0), g(m1)
+    s = torch.cuda.current_stream()
+    L = plan.L
+
+    def stages(upto):
+        check(L.st_deform_grid_stages_dev(
+            None, int(plan.tri_t.shape[0]), plan.tri_t.data_ptr(), yx0_t.data_ptr(), m0_t.data_ptr(), yx1_t.data_ptr(),
+            m1_t.data_ptr(), float(dt), G.levels, G.shape[0], G.shape[1], float(G.origin[0]), float(G.origin[1]),
+            G.L0_km, plan.min_area.ctypes.data, G.bin_edges.size, plan.edges_t.data_ptr(), plan.scratch.data_ptr(),
+            plan.scratch_bytes, mom.data_ptr(), hist.data_ptr(), fields.data_ptr(), nbox.data_ptr(), upto,
+            C.c_void_p(s.cuda_stream)))
+    run = lambda: plan.launch(None, yx0_t, m0_t, yx1_t, m1_t, dt, mom, hist, fields, nbox, s)
+    us, n = time_loop(torch, run, a.seconds)
+    cum = [time_loop(torch, lambda u=u: stages(u), a.seconds / 2)[0] for u in (1, 2, 3)]
+    run()
+    m1_, h1_, f1_, nb = mom.cpu().numpy(), hist.cpu().numpy(), fields.cpu().numpy(), nbox.cpu().numpy()
+    run()
+    same = bool(np.array_equal(m1_, mom.cpu().numpy()) and np.array_equal(h1_, hist.cpu().numpy()) and
+                np.array_equal(f1_.view(np.uint32), fields.cpu().numpy().view(np.uint32)))
+    # level-1 cells of a sample of binned triangles' cells against the oracle, bit for bit
+    fl = DG.split_fields(G, f1_)
+    parts = [OG.eulerian_binning(yx0, yx1, m0, m1, tri[i:i + 2 ** 21], G.origin, L0, G.shape)
+             for i in range(0, tri.shape[0], 2 ** 21)]                # in slices: host memory
+    binned, key = np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
+    cell = key[:, 0] * G.shape[1] + key[:, 1]
+    cells = np.unique(cell[binned])
+    pick = np.sort(rng.choice(cells, min(20000, cells.size), replace=False))
+    sel = np.flatnonzero(binned & np.isin(cell, pick))
+    sel = sel[np.argsort(cell[sel], kind="stable")]                 # caller's order within each cell
+    cs = cell[sel]
+    st = np.flatnonzero(np.r_[True, cs[1:] != cs[:-1]])
+    off = np.r_[st, cs.size]
+    T, _, _ = O.triangle_terms(yx0, yx1, m0, m1, tri[sel], dt)
+    o, ok = O.box_outputs(O.level1_sums(T, off), G.min_area[0])
+    ucell = cs[st]
+    with np.errstate(all="ignore"):
+        exact = all(np.array_equal(fl[0][k].ravel()[ucell], np.where(ok, o[k], O.FillValue).astype(np.float32))
+                    for k in O.BOX_NAMES)
+    stage = dict(key_us=round(cum[0], 2), sort_us=round(cum[1] - cum[0], 2), segmentation_us=round(cum[2] - cum[1], 2),
+                 boxes_stats_fields_us=round(us - cum[2], 2))
+    return dict(us_per_window=round(us, 2), passes_timed=n, vs_k_deform=round(us / us_deform, 3),
+                vs_lagrangian_pass=round(us / us_scales, 3), goal_2x_lagrangian_met=bool(us <= 2.0 * us_scales),
+                stages_cumulative_us=[round(c, 2) for c in cum], stages=stage, L0_km=L0, levels=a.levels,
+                origin_km=G.origin.tolist(), shape=list(G.shape), boxes_per_level=nb.tolist(),
+                n_per_scale=h1_[:, 0].sum(1).tolist(), binned_triangles=int(binned.sum()),
+                field_words=G.field_size(), sample_cells=int(pick.size), sample_cells_bit_identical=bool(exact),
+                run_to_run_identical=same)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--ny", type=int, default=3531)
@@ -173,6 +244,7 @@ def main():
         h0.copy_(yx0_t, non_blocking=True); h1.copy_(yx1_t, non_blocking=True)
     us_d2h, n_d2h = time_loop(torch, d2h, a.seconds / 2, warm=3)
     sc = scales(torch, a, rng, yx0, yx1, m0, m1, tri, dt, g, us)
+    gr = grid(torch, a, rng, yx0, yx1, m0, m1, tri, dt, g, us, sc["us_per_window"])
     bytes_model = nT * (12 + 24) + nP * 2 * (16 + 1)
     peak, peak_src = hbm_peak()
     gbs = bytes_model / (us * 1e-6) / 1e9
@@ -186,14 +258,15 @@ def main():
                valid_fraction=float((out[0] != -9999.0).mean()),
                workload="jittered 3 km lattice %dx%d, 2 triangles per square, sorted by smallest vertex; "
                         "inputs larger than L2, no flush" % (a.ny, a.nx),
-               scales=sc, card=card_info(torch, dev))
+               scales=sc, grid=gr, card=card_info(torch, dev))
     line = json.dumps(res)
     print(line)
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
             f.write(line + "\n")
-    return 0 if exact and sc["sample_boxes_bit_identical"] and sc["run_to_run_identical"] else 1
+    return 0 if (exact and sc["sample_boxes_bit_identical"] and sc["run_to_run_identical"] and
+                 gr["sample_cells_bit_identical"] and gr["run_to_run_identical"]) else 1
 
 
 if __name__ == "__main__":
