@@ -332,6 +332,31 @@ int  st_deform_grid_stages_dev(st_ctx *ctx, int64_t nT, const int32_t *tri_dev, 
                                double *moments_dev, int64_t *hist_dev, float *fields_dev, int64_t *nbox_dev, int upto,
                                void *stream);
 
+/* ---- two-particle (pair) dispersion over time lags, and per-(lag, class) statistics ----------
+ * nQ (1..2^31-1) pairs pairs_dev (nQ,2) int32 of buoy indices (8-byte aligned; not range-checked on the device) between
+ * the closing row yx1_dev, m1_dev and nact origin rows yx0[o], m0[o] (HOST arrays of device pointers) that lie lag[o]
+ * (HOST, distinct, 1..lags) steps of dt_days days before it (DESIGN.md section 13, oracle/dispersion_ref.py).  Per pair
+ * and origin, valid when both buoys have mask != 0 in both rows, in f8: r0 = |p_a - p_b| at the origin, r1 at the
+ * closing row, dr = r1 - r0, dD2 = |(p_a - p_b)_1 - (p_a - p_b)_0|^2, stretch rate s = |dr| / (r0 lag dt_days) [day-1];
+ * separation class searchsorted(r_edges, r0, side="right") over nclass_edges (1..63) ascending f8 edges, stretch bin
+ * the same over nedge (1..4096) bins.  Outputs, zeroed and then written for the active lags only:
+ *   hist_dev (lags, nclass_edges+1, nedge+1) int64   counts of s (exact);
+ *   sums_dev (lags, nclass_edges+1, 4) f8            sums of r0, dr, dr^2, dD2 over the valid pairs;
+ *   per_pair_dev, if not NULL (nact = 1 only), (4, nQ) f8 r0, r1, dr, dD2, -9999 for invalid pairs.
+ * The sums use no floating-point atomics and a launch grid that depends on nQ only: bit-identical run to run and
+ * between one call over several origins and one call per origin.  The shared-memory counters limit the shapes:
+ * nact (nclass_edges+1)(nedge+1) ints plus (nclass_edges + nedge + 4 (nclass_edges+1)(nact + 16)) doubles must fit in
+ * 227 KB.  st_dispersion_scratch_bytes checks (nQ, lags, classes, bins) for nact = lags on the host, before any CUDA
+ * call, and gives the scratch (block partials) to allocate once.  ASYNC st_dispersion_dev: no host synchronisation,
+ * no allocation; refuses nQ < 1, dt_days <= 0 or NaN, nact outside 1..lags and shapes past the limit, and writes
+ * nothing then.                                                                                               */
+int  st_dispersion_scratch_bytes(int64_t nQ, int lags, int nclass_edges, int nedge, int64_t *bytes);
+int  st_dispersion_dev(st_ctx *ctx, int64_t nQ, const int32_t *pairs_dev, const double *yx1_dev, const int8_t *m1_dev,
+                       int nact, const double *const *yx0, const int8_t *const *m0, const int *lag, double dt_days,
+                       int lags, int nclass_edges, const double *r_edges_dev, int nedge, const double *bins_dev,
+                       void *scratch_dev, int64_t scratch_bytes, int64_t *hist_dev, double *sums_dev,
+                       double *per_pair_dev, void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

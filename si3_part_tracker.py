@@ -69,6 +69,13 @@ def __argument_parsing__():
                              '(LEVELS levels) covering the model\'s T-points, binned every window by mid-time centroid, and '
                              'write per-level fields into ./nc/..._deformation-grid_... and per-scale statistics into '
                              './nc/..._deformation-grid-scaling_...')
+    parser.add_argument('--dispersion', type=float, nargs=2, default=None, metavar=('HOURS', 'LAGS'),
+                        help='also compute two-particle dispersion of buoy pairs on the GPU: origins every HOURS (a multiple '
+                             'of the model time step), lags of 1..LAGS windows, per-lag and per-separation-class statistics '
+                             'of every window into ./nc/..._dispersion_...')
+    parser.add_argument('--dispersion-pairs', type=float, nargs=3, default=None, metavar=('N', 'R_MIN_KM', 'R_MAX_KM'),
+                        help='with --dispersion: N random draws of pairs at log-uniform separations in [R_MIN_KM, R_MAX_KM] '
+                             '(default: one draw per buoy, 10 to 1000 km)')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -179,6 +186,37 @@ def deform_grid_args(grid, hours):
     return L0, int(lev)
 
 
+def dispersion_args(disp, pairs, world):
+    """--dispersion HOURS LAGS [--dispersion-pairs N R_MIN_KM R_MAX_KM] -> (records per window, lags, N or None,
+    r_min, r_max) or None; ERROR and exit when HOURS is not a positive multiple of the model time step, LAGS is not an
+    integer in 1..MAX_LAGS, N < 1, R_MIN <= 0 or R_MAX <= R_MIN, --dispersion-pairs comes without --dispersion, or under
+    torchrun (pairs would cross the ranks' shards)."""
+    if disp is None:
+        if pairs is not None:
+            print('ERROR: --dispersion-pairs needs --dispersion HOURS LAGS')
+            exit(0)
+        return None
+    hours, lags = disp
+    if world > 1:
+        print('ERROR: --dispersion is not available with several processes (WORLD_SIZE > 1): pairs would cross ranks')
+        exit(0)
+    n = hours * 3600. / rdt
+    if not (hours > 0 and abs(n - round(n)) < 1e-9 and round(n) >= 1):
+        print('ERROR: --dispersion HOURS must be a positive multiple of the model time step (%g h), got %g' % (rdt / 3600., hours))
+        exit(0)
+    if lags != int(lags) or not 1 <= lags <= sit.MAX_LAGS:
+        print('ERROR: --dispersion LAGS must be an integer in 1..%d, got %g' % (sit.MAX_LAGS, lags))
+        exit(0)
+    N, r_min, r_max = (None, 10.0, 1000.0) if pairs is None else pairs
+    if N is not None and (N != int(N) or N < 1):
+        print('ERROR: --dispersion-pairs N must be a positive integer, got %g' % N)
+        exit(0)
+    if not (r_min > 0 and r_max > r_min and np.isfinite(r_max)):
+        print('ERROR: --dispersion-pairs needs 0 < R_MIN_KM < R_MAX_KM, got %g %g' % (r_min, r_max))
+        exit(0)
+    return int(round(n)), int(lags), None if N is None else int(N), r_min, r_max
+
+
 def deform_grid_over(Yt, Xt, L0, levels):
     """The EulerianGrid of side L0 covering the T-points (Yt, Xt) km: origin floor(min / L0) L0 and
     floor((max - origin) / L0) + 1 cells per axis; ERROR and exit when that is more than 2^20 cells a side."""
@@ -201,6 +239,7 @@ def main():
     ndeform = deform_records(args.deform, world)
     dscales = deform_scales_args(args.deform_scales, args.deform)
     dgrid = deform_grid_args(args.deform_grid, args.deform)
+    dspa = dispersion_args(args.dispersion, args.dispersion_pairs, world)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
@@ -226,6 +265,9 @@ def main():
     Nt, kstrt, kstop, iTmA, iTmB = sit.GetTimeSpan(rdt, ztime_model, idateSeedA, idateModA, idateModB, iStop=date_stop)
     if Nt < 1:
         print(' QUITTING since no matching model records!')
+        exit(0)
+    if dspa and Nt // dspa[0] < 1:
+        print('ERROR: --dispersion window (%d records) is longer than the run (%d records)!' % (dspa[0], Nt))
         exit(0)
     for cd in ['seed', 'nc', 'npz']:
         makedirs(cd, exist_ok=True)
@@ -380,6 +422,24 @@ def main():
                 gswriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], st)
             deform.update(grid=G, grid_sink=grid_sink)
         small = False                                             # windows close inside the streaming record loop
+    dispersion = None
+    if dspa:
+        # pairs over the seeds in the order the files use (after --sort); only statistics leave the GPU
+        nd, lags, npair, r_min, r_max = dspa
+        nwd = Nt // nd
+        pairs = sit.SeparationPairs(xPosC0, r_min, r_max, nP if npair is None else npair, seed=0)
+        if pairs.shape[0] == 0:
+            print('ERROR: --dispersion: no pair of distinct buoys was drawn!')
+            exit(0)
+        print(' *** --dispersion: %d pairs at %g to %g km, %d windows of %d records, lags 1..%d'
+              % (pairs.shape[0], r_min, r_max, nwd, nd, lags))
+        cf_dsp = './nc/' + corgn + '_dispersion_' + SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + \
+            hstr(vTime[nwd * nd]) + csfkm + ext
+        pwriter = sit.DispersionWriter(cf_dsp, nwd, np.arange(1, lags + 1) * (nd * rdt / 86400.), sit.DEFAULT_R_EDGES,
+                                       sit.DEFAULT_BIN_EDGES, corigin=corgn)
+        dispersion = dict(pairs=pairs, every=nd, lags=lags,
+                          sink=lambda w, st: pwriter.write(w, vTime[w * nd], vTime[(w + 1) * nd], st))
+        small = False
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
         res = eng.track(record, Nt, kstrt=kstrt, pos0=xPosC0, posG0=xPosG0, rec_first=z1st, chunk=nchunk,
@@ -388,7 +448,8 @@ def main():
             keep_row(k, res['posC'][k + 1], res['posG'][k + 1], res['mask'][k + 1])
     else:
         res = eng.track(record, Nt, kstrt=kstrt, rec_first=cut(z1st), sink=sink,
-                        row_dtype='f8' if physics else args.rows, physics=physics, deform=deform)
+                        row_dtype='f8' if physics else args.rows, physics=physics, deform=deform,
+                        dispersion=dispersion)
     eng.close()
     if deform:
         dwriter.close()
@@ -397,6 +458,8 @@ def main():
         if G is not None:
             gwriter.close()
             gswriter.close()
+    if dispersion:
+        pwriter.close()
     ds.close()
     n_alive = res['n_alive']
     if world > 1:

@@ -83,6 +83,9 @@ SIGNATURES = {
                                    c_int, vp, vp, c_i64, vp, vp, vp, vp, vp]),
     "st_deform_grid_stages_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, vp, c_dbl, c_int, c_int, c_int, c_dbl, c_dbl, c_dbl,
                                           vp, c_int, vp, vp, c_i64, vp, vp, vp, vp, c_int, vp]),
+    "st_dispersion_scratch_bytes": (c_int, [c_i64, c_int, c_int, c_int, vp]),
+    "st_dispersion_dev": (c_int, [vp, c_i64, vp, vp, vp, c_int, vp, vp, vp, c_dbl, c_int, c_int, vp, c_int, vp, vp,
+                                  c_i64, vp, vp, vp, vp]),
     "st_xy2latlon": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_latlon2xy": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_xy2latlon_dev": (c_int, [c_i64, vp, vp, c_dbl, c_dbl, vp]),

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libsitrack_b200.so")
-SOURCES = ["st_api.cu", "st_advect.cu", "st_locate.cu", "st_geom.cu", "st_ext.cu", "st_deform.cu", "st_deform_scale.cu", "st_deform_grid.cu"]
+SOURCES = ["st_api.cu", "st_advect.cu", "st_locate.cu", "st_geom.cu", "st_ext.cu", "st_deform.cu", "st_deform_scale.cu", "st_deform_grid.cu", "st_disperse.cu"]
 HEADERS = ["st_device.cuh", "st_kernels.h", "st_deform.cuh", "st_persist.cuh", "st_pipe.cuh", "st_warp.cuh", "st_cert.cuh", "st_experiments.cuh", os.path.join("..", "..", "include", "sitrack_b200.h")]
 
 NVCC_FLAGS = [

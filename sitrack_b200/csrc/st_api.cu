@@ -1260,6 +1260,63 @@ int st_deform_grid_dev(st_ctx* c, int64_t nT, const int32_t* tri, const double* 
                                      stream);
 }
 
+// ---- pair dispersion over time lags, and its statistics (st_disperse.cu) ----------------------------
+static const char* disp_check(int64_t nQ, int lags, int nclass_edges, int nedge, int nact)
+{
+    if (nQ < 1 || nQ > INT32_MAX) return "nQ must be in 1..2^31-1";
+    if (lags < 1 || lags > DS_MAX_LAGS) return "lags must be in 1..64";
+    if (nclass_edges < 1 || nclass_edges > DS_MAX_CLASS_EDGES) return "nclass_edges must be in 1..63";
+    if (nedge < 1 || nedge > SC_MAX_EDGES) return "nedge must be in 1..4096";
+    if (nact < 1 || nact > lags) return "the number of active lags must be in 1..lags";
+    if (disp_smem(nact, nclass_edges, nedge) > DS_MAX_SMEM)
+        return "lags x classes x bins need more than the 227 KB of shared memory a block may have";
+    return nullptr;
+}
+
+int st_dispersion_scratch_bytes(int64_t nQ, int lags, int nclass_edges, int nedge, int64_t* bytes)
+{
+    if (!bytes) return fail(nullptr, ST_EINVAL, "st_dispersion_scratch_bytes: NULL argument");
+    if (const char* why = disp_check(nQ, lags, nclass_edges, nedge, lags))
+        return fail(nullptr, ST_EINVAL, std::string("st_dispersion_scratch_bytes: ") + why);
+    *bytes = disp_scratch_bytes(nQ, lags, nclass_edges);
+    return ST_OK;
+}
+
+int st_dispersion_dev(st_ctx* c, int64_t nQ, const int32_t* pairs, const double* yx1, const int8_t* m1, int nact,
+                      const double* const* yx0, const int8_t* const* m0, const int* lag, double dt_days, int lags,
+                      int nclass_edges, const double* r_edges, int nedge, const double* bins, void* scratch,
+                      int64_t scratch_bytes, int64_t* hist, double* sums, double* per_pair, void* stream)
+{
+    if (const char* why = disp_check(nQ, lags, nclass_edges, nedge, nact))
+        return fail(c, ST_EINVAL, std::string("st_dispersion_dev: ") + why);
+    if (!(dt_days > 0.0)) return fail(c, ST_EINVAL, "st_dispersion_dev: dt_days must be positive");
+    if (!pairs || !yx1 || !m1 || !yx0 || !m0 || !lag || !r_edges || !bins || !scratch || !hist || !sums)
+        return fail(c, ST_EINVAL, "st_dispersion_dev: NULL argument");
+    if (per_pair && nact != 1) return fail(c, ST_EINVAL, "st_dispersion_dev: per_pair needs exactly one active lag");
+    if ((uintptr_t)pairs % 8 || (uintptr_t)yx1 % 16 || (uintptr_t)r_edges % 8 || (uintptr_t)bins % 8 ||
+        (uintptr_t)scratch % 8 || (uintptr_t)hist % 8 || (uintptr_t)sums % 8 || (uintptr_t)per_pair % 8)
+        return fail(c, ST_EINVAL, "st_dispersion_dev: rows must be 16-byte aligned, pairs, edges, scratch and outputs "
+                                  "8-byte");
+    DispOrigins og = {};
+    og.nact = nact;
+    for (int o = 0; o < nact; ++o) {
+        if (!yx0[o] || !m0[o]) return fail(c, ST_EINVAL, "st_dispersion_dev: NULL origin row");
+        if ((uintptr_t)yx0[o] % 16) return fail(c, ST_EINVAL, "st_dispersion_dev: rows must be 16-byte aligned");
+        if (lag[o] < 1 || lag[o] > lags) return fail(c, ST_EINVAL, "st_dispersion_dev: lag numbers must be in 1..lags");
+        for (int p = 0; p < o; ++p)
+            if (lag[p] == lag[o]) return fail(c, ST_EINVAL, "st_dispersion_dev: a lag number appears twice");
+        og.yx[o] = (const pt*)yx0[o];
+        og.m[o] = m0[o];
+        og.lag[o] = lag[o];
+    }
+    if (scratch_bytes < disp_scratch_bytes(nQ, lags, nclass_edges))
+        return fail(c, ST_EINVAL, "st_dispersion_dev: scratch_bytes is smaller than st_dispersion_scratch_bytes");
+    if (c) CU(c, cudaSetDevice(c->device));
+    CU(c, launch_dispersion(og, nQ, pairs, (const pt*)yx1, m1, dt_days, lags, nclass_edges, r_edges, nedge, bins,
+                            scratch, hist, sums, per_pair, (cudaStream_t)stream));
+    return ST_OK;
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

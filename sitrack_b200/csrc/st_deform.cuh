@@ -1,5 +1,6 @@
 // st_deform.cuh -- the per-triangle arithmetic that k_deform (st_deform.cu) and the coarse-graining kernels
-// (st_deform_scale.cu) share, so that both spell every sum in the oracle's order from one definition.
+// (st_deform_scale.cu) share, so that both spell every sum in the oracle's order from one definition; the gather of
+// an f8 position and the histogram bin rule, shared with the pair-dispersion kernel (st_disperse.cu) as well.
 #pragma once
 #include "st_kernels.h"
 
@@ -9,6 +10,18 @@ __device__ __forceinline__ pt ld_ro_pt(const pt* __restrict__ a, int i)
 {
     const double2 v = __ldg(reinterpret_cast<const double2*>(a + i));
     pt r; r.y = v.x; r.x = v.y; return r;
+}
+
+// bin of v on ascending edges e[0..ne): searchsorted(e, v, side="right"), so ne + 1 bins with underflow and overflow
+__device__ __forceinline__ int bin_right(const double* __restrict__ e, int ne, double v)
+{
+    if (v != v) return ne;                                      // NaN sorts last, as numpy's searchsorted
+    int lo = 0, hi = ne;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (e[mid] <= v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
 }
 
 // 2A = (X0 Y1 - X1 Y0) + (X1 Y2 - X2 Y1) + (X2 Y0 - X0 Y2), left to right

@@ -29,17 +29,6 @@ constexpr int SC_GRID = 1184;          // fixed (not the SM count): the moment p
                                        // same on every device
 constexpr int SC_BOX = 8;              // doubles per box record: a2, ux, uy, vx, vy, NY, NX sums + padding
 
-__device__ __forceinline__ int bin_right(const double* __restrict__ e, int ne, double v)
-{
-    if (v != v) return ne;                                      // NaN sorts last, as numpy's searchsorted
-    int lo = 0, hi = ne;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (e[mid] <= v) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-}
-
 // rates of a sum record -> eps_tot, |div|, shear (the statistics' three variables), f8 as the oracle
 struct Rates { double div, shear, vort, tot; };
 __device__ __forceinline__ Rates rates_of(double ux, double uy, double vx, double vy)

@@ -238,4 +238,29 @@ cudaError_t launch_deform_grid(const GridPlan& g, const int32_t* tri, const pt* 
                                void* scratch, double* mom, int64_t* hist, float* fields, long long* nbox,
                                int upto, cudaStream_t st);
 
+// ---- pair dispersion over time lags, and its statistics (st_disperse.cu) ----
+constexpr int DS_MAX_LAGS = 64;
+constexpr int DS_MAX_CLASS_EDGES = 63;
+constexpr size_t DS_MAX_SMEM = 227 * 1024;     // opt-in dynamic shared memory per block on sm_100
+
+// The active origin rows of one call, passed by value: rows yx[o], m[o] at lag lag[o] (1..lags) before the closing row.
+struct DispOrigins {
+    int nact;
+    const pt* yx[DS_MAX_LAGS];
+    const int8_t* m[DS_MAX_LAGS];
+    int lag[DS_MAX_LAGS];
+};
+
+// Launch grid (a function of nQ only), dynamic shared memory of k_disperse for nact active origins, and the scratch
+// (block partials) a call with up to `lags` active origins needs.
+int disp_grid(long long nQ);
+size_t disp_smem(int nact, int ncedge, int nedge);
+long long disp_scratch_bytes(long long nQ, int lags, int ncedge);
+// pairs (nQ,2) buoy indices; hist (lags, ncedge+1, nedge+1) int64 and sums (lags, ncedge+1, 4) f8 [r0, dr, dr^2, dD2]
+// are zeroed and then written for the active lags; out, if not NULL (one origin only), (4, nQ) f8 r0, r1, dr, dD2.
+cudaError_t launch_dispersion(const DispOrigins& og, long long nQ, const int32_t* pairs, const pt* yx1,
+                              const int8_t* m1, double dt, int lags, int ncedge, const double* r_edges, int nedge,
+                              const double* bins, void* scratch, int64_t* hist, double* sums, double* out,
+                              cudaStream_t st);
+
 }  // namespace st

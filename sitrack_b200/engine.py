@@ -427,7 +427,7 @@ class TrackEngine:
 
     # -- the record loop ---------------------------------------------------------------
     def track(self, records, nrec, kstrt=0, pos0=None, posG0=None, rec_first=None, want_latlon=True,
-              sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None):
+              sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None, dispersion=None):
         """The record loop (si3_part_tracker.py:361-496), pipelined.
 
         records: callable k -> (u, v, ic) arrays (Nj,Ni) for record index k (0-based
@@ -456,6 +456,13 @@ class TrackEngine:
         the device (sitrack_b200.deform_grid); only the fields and statistics reach the host: grid_sink(w, fields,
         stats), or with grid_sink None the list of (fields, stats) under "deform_grid".  They do not depend on the
         order the buoys are stored in either.
+        dispersion = dict(pairs=(nQ,2) buoy pairs in the caller's order (sitrack_b200.dispersion: MeshPairs,
+        SeparationPairs), every=n, lags=m (1..MAX_LAGS), r_edges=None, bins=None, sink=callable or None), independent of
+        `deform` and combinable with it: the rows w*n are origins, kept on the device in a ring of min(m, windows) f8
+        rows and masks (17 B per buoy each); as window w closes, the pairs' dispersion between origin row (w+1-l)*n and
+        row (w+1)*n is reduced on the device for lags l = 1 .. min(m, w+1) in one launch, and only the statistics reach
+        the host: sink(w, stats), or with sink None the list of them under "dispersion".  They do not depend on the
+        order the buoys are stored in.  Not with the chunked season path either.
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -472,10 +479,13 @@ class TrackEngine:
                 raise ValueError("physics modes write f8 rows")
             chunk = None
         if chunk and chunk > 1 and sink is None:
-            if deform is not None:
-                raise ValueError("deform runs on the streaming record loop: not with chunk > 1 and sink=None")
+            if deform is not None or dispersion is not None:
+                raise ValueError("deform and dispersion run on the streaming record loop: not with chunk > 1 and sink=None")
             return self._track_chunked(get, nrec, kstrt, pos0, posG0, rec_first, want_latlon, int(chunk), rdt)
-        dfm = None if deform is None else _DeformRun(self, torch, dev, deform, rec_first, kstrt, row_f4=rdt == torch.float32)
+        wrows = None if deform is None and dispersion is None else _WindowRows(self, torch, rec_first, kstrt,
+                                                                               row_f4=rdt == torch.float32)
+        dfm = None if deform is None else _DeformRun(self, torch, dev, deform, wrows)
+        dsp = None if dispersion is None else _DispersionRun(self, torch, dev, dispersion, wrows, nrec)
         self.record_slots(2)
         stg = [self.staging(0), self.staging(1)]
         s_in, s_cmp, s_out = (torch.cuda.Stream(dev) for _ in range(3))
@@ -554,6 +564,8 @@ class TrackEngine:
                 ev_out[k] = torch.cuda.Event(); ev_out[k].record(s_out)
                 if dfm is not None:
                     dfm.after_step(k, d_yx[b], d_mk[b], s_cmp, s_out)
+                if dsp is not None:
+                    dsp.after_step(k, d_yx[b], d_mk[b], s_cmp, s_out)
             for k in range(max(0, nrec - NB), nrec):
                 if keep:
                     ev_out[k].synchronize()
@@ -561,6 +573,8 @@ class TrackEngine:
                     drain(k)
             if dfm is not None:
                 dfm.finish()
+            if dsp is not None:
+                dsp.finish()
         finally:
             if chain:
                 self.set_row_chain(False)                  # state up to date again (synchronises)
@@ -572,6 +586,8 @@ class TrackEngine:
             extra["deform_scales"] = dfm.scale_collected
         if dfm is not None and dfm.grid_collected is not None:
             extra["deform_grid"] = dfm.grid_collected
+        if dsp is not None and dsp.collected is not None:
+            extra["dispersion"] = dsp.collected
         if not keep:
             return dict(n_alive=n_alive, **extra)
         posC, posG, mask = posC.numpy(), posG.numpy(), mask.numpy()
@@ -582,38 +598,60 @@ class TrackEngine:
         return dict(posC=posC, posG=posG, mask=mask, n_alive=n_alive, **extra)
 
 
+class _WindowRows:
+    """What the per-window passes over the trajectory rows share: the buoy permutation of the engine (set_buoys or
+    set_buoys_dev with sort=True), row 0's mask in engine order (the state handed to set_buoys, masked like the returned
+    series' row 0: rec_first == kstrt) and the f8 positions of a row.  Positions are f8: with f8 rows the row itself
+    (read only, so row chaining is unaffected), with f4 rows the device state (steps with f4 rows do not chain, so it
+    is current after every step)."""
+
+    def __init__(self, eng, torch, rec_first, kstrt, row_f4):
+        nP = eng.nP
+        self.row_f4 = row_f4
+        perm = eng.perm
+        if perm is None and getattr(eng, "perm_t", None) is not None:      # set_buoys_dev(sort=True)
+            perm = eng.perm_t.cpu().numpy()
+        m0 = np.ones(nP, np.int8) if rec_first is None else (np.asarray(rec_first) - kstrt == 0).astype(np.int8)
+        self.inv = None
+        if perm is not None:                                                # caller's order -> engine slots
+            if perm.shape != (nP,):
+                raise ValueError("the engine's buoy permutation does not match its %d buoys" % nP)
+            self.inv = np.empty_like(perm); self.inv[perm] = np.arange(perm.size)
+            m0 = m0[perm]
+        self.m0 = m0
+        p = C.c_void_p()
+        check(eng.L.st_state_device_ptrs(eng.h, C.byref(p), None, None), eng.h)
+        self.state_pos = _tensor_from_ptr(torch, p.value, (nP, 2), torch.float64, 8, eng.device)
+
+    def slots(self, idx):
+        """Buoy indices in the caller's order -> engine slots (same shape, i4)."""
+        return idx if self.inv is None else self.inv[idx].astype(np.int32)
+
+    def yx(self, yx_row):
+        """The f8 positions of the row a step has just written to yx_row."""
+        return self.state_pos if self.row_f4 else yx_row
+
+
 class _DeformRun:
     """track(deform=...): the anchor row of the open window on the device, k_deform when a window closes, its
     outputs to the host on the output stream.
 
-    Positions are f8: with f8 rows the row itself (read only, so row chaining is unaffected), with f4 rows the
-    device state (steps with f4 rows do not chain, so it is current after every step).  Triangles are mapped into
-    engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs go back to the
+    Positions and row 0 as _WindowRows gives them.  Triangles are mapped into engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs go back to the
     caller's triangle order on the host.  With `scales`, the box hierarchy pass runs on the same rows after k_deform
     and before the anchor copy; its statistics go to the host on the output stream alongside the triangles'.  With
     `grid`, the Eulerian grid pass follows on the same rows, over the triangles in the caller's order (mapped to
     engine slots), and its fields and statistics go to the host the same way."""
 
-    def __init__(self, eng, torch, dev, spec, rec_first, kstrt, row_f4):
+    def __init__(self, eng, torch, dev, spec, rows):
         from . import deform as D
-        self.eng, self.torch, self.row_f4, self.D = eng, torch, row_f4, D
+        self.eng, self.torch, self.rows, self.D = eng, torch, rows, D
         self.every = int(spec["every"])
         if self.every < 1:
             raise ValueError("deform: every must be >= 1 record")
         self.sink = spec.get("sink")
         self.collected = [] if self.sink is None else None
         nP = eng.nP
-        tri = D.check_mesh(spec["tri"], nP)
-        perm = eng.perm
-        if perm is None and getattr(eng, "perm_t", None) is not None:      # set_buoys_dev(sort=True)
-            perm = eng.perm_t.cpu().numpy()
-        m0 = np.ones(nP, np.int8) if rec_first is None else (np.asarray(rec_first) - kstrt == 0).astype(np.int8)
-        if perm is not None:                                                # caller's order -> engine slots
-            if perm.shape != (nP,):
-                raise ValueError("deform: the engine's buoy permutation does not match its %d buoys" % nP)
-            inv = np.empty_like(perm); inv[perm] = np.arange(perm.size)
-            tri = inv[tri].astype(np.int32)
-            m0 = m0[perm]
+        tri = rows.slots(D.check_mesh(spec["tri"], nP))
         self.scales = None
         H = spec.get("scales")
         if H is not None:
@@ -645,12 +683,9 @@ class _DeformRun:
         self.nT = tri.shape[0]
         self.dt = self.every * eng.rdt / 86400.0
         self.tri_t = torch.from_numpy(tri).to(dev)
-        p = C.c_void_p()
-        check(eng.L.st_state_device_ptrs(eng.h, C.byref(p), None, None), eng.h)
-        self.state_pos = _tensor_from_ptr(torch, p.value, (nP, 2), torch.float64, 8, eng.device)
         # the anchor: row 0 (on torch's current stream; track's streams wait for it)
-        self.a_yx = self.state_pos.clone()
-        self.a_mk = torch.from_numpy(m0).to(dev)
+        self.a_yx = rows.state_pos.clone()
+        self.a_mk = torch.from_numpy(rows.m0).to(dev)
         self.d_out = [torch.empty((6, max(self.nT, 1)), dtype=torch.float32, device=dev) for _ in range(2)]
         self.h_out = [torch.empty((6, max(self.nT, 1)), dtype=torch.float32).pin_memory() for _ in range(2)]
         self.ev_out = []
@@ -664,7 +699,7 @@ class _DeformRun:
         b = w % 2
         if w >= 2:
             s_cmp.wait_event(self.ev_out[w - 2])                   # d_out[b] has reached the host
-        yx = self.state_pos if self.row_f4 else yx_row
+        yx = self.rows.yx(yx_row)
         self.D.launch(self.eng.L, self.eng.h, self.nT, self.tri_t, self.a_yx, self.a_mk, yx, mk_row, self.dt,
                       self.d_out[b], s_cmp)
         if self.scales is not None:
@@ -709,6 +744,79 @@ class _DeformRun:
                 self.grid_collected.append((fl, st))
             else:
                 self.grid_sink(w, fl, st)
+        self.drained = w + 1
+
+    def finish(self):
+        for w in range(self.drained, len(self.ev_out)):
+            self._drain(w)
+
+
+class _DispersionRun:
+    """track(dispersion=...): the ring of origin rows on the device, st_dispersion_dev over every active lag when a
+    window closes, its statistics to the host on the output stream.
+
+    Origin row o (= row o*every) lives in ring slot o % lags.  When window w closes the launch reads the origins
+    w+1-l, l = 1 .. min(lags, w+1), on the compute stream; only after it is the closing row, origin w+1, copied into
+    slot (w+1) % lags, the slot of origin w+1-lags that the launch has just read for the last time.  Pairs are mapped
+    to engine slots without reordering them, so the sums do not depend on `perm`."""
+
+    def __init__(self, eng, torch, dev, spec, rows, nrec):
+        from . import dispersion as P
+        self.eng, self.torch, self.rows, self.P = eng, torch, rows, P
+        self.every = int(spec["every"])
+        if self.every < 1:
+            raise ValueError("dispersion: every must be >= 1 record")
+        self.lags = P.check_lags(spec["lags"])
+        pairs = P.check_pairs(spec["pairs"], eng.nP)
+        self.plan = P._Plan(torch, dev, rows.slots(pairs), self.lags, spec.get("r_edges"), spec.get("bins"))
+        self.sink = spec.get("sink")
+        self.collected = [] if self.sink is None else None
+        self.dt = self.every * eng.rdt / 86400.0
+        self.lag_days = np.arange(1, self.lags + 1) * self.dt
+        self.nwin = nrec // self.every
+        nslot = max(1, min(self.lags, self.nwin))                   # origins 0 .. nwin-1 are the only ones read
+        nP = eng.nP
+        # slot 0: row 0 (on torch's current stream; track's streams wait for it)
+        self.r_yx = [rows.state_pos.clone()] + [torch.empty((nP, 2), dtype=torch.float64, device=dev)
+                                                 for _ in range(nslot - 1)]
+        self.r_mk = [torch.from_numpy(rows.m0).to(dev)] + [torch.empty((nP,), dtype=torch.int8, device=dev)
+                                                           for _ in range(nslot - 1)]
+        self.d_st = [self.plan.outputs() for _ in range(2)]
+        self.h_st = [self.plan.outputs(pin=True) for _ in range(2)]
+        self.ev_out = []
+        self.drained = 0
+
+    def after_step(self, k, yx_row, mk_row, s_cmp, s_out):
+        """Step k has been queued on s_cmp: row k+1 closes window w when k+1 = (w+1)*every."""
+        if (k + 1) % self.every:
+            return
+        torch, w, L = self.torch, (k + 1) // self.every - 1, self.lags
+        b = w % 2
+        if w >= 2:
+            s_cmp.wait_event(self.ev_out[w - 2])                   # d_st[b] has reached the host
+        yx = self.rows.yx(yx_row)
+        origins = [(self.r_yx[(w + 1 - l) % L], self.r_mk[(w + 1 - l) % L], l) for l in range(1, min(L, w + 1) + 1)]
+        self.plan.launch(self.eng.h, yx, mk_row, origins, self.dt, *self.d_st[b], None, s_cmp)
+        if w + 1 < self.nwin:
+            with torch.cuda.stream(s_cmp):                          # after the launch that read the slot last
+                self.r_yx[(w + 1) % L].copy_(yx)
+                self.r_mk[(w + 1) % L].copy_(mk_row)
+        ev = torch.cuda.Event(); ev.record(s_cmp)
+        if w >= 2:
+            self._drain(w - 2)                                      # h_st[b] is free again
+        s_out.wait_event(ev)
+        with torch.cuda.stream(s_out):
+            for h, d in zip(self.h_st[b], self.d_st[b]):
+                h.copy_(d, non_blocking=True)
+        self.ev_out.append(torch.cuda.Event()); self.ev_out[w].record(s_out)
+
+    def _drain(self, w):
+        self.ev_out[w].synchronize()
+        st = self.P.stats_dict(self.lag_days, self.plan.r_edges, self.plan.bins, *(h.numpy() for h in self.h_st[w % 2]))
+        if self.sink is None:
+            self.collected.append(st)
+        else:
+            self.sink(w, st)
         self.drained = w + 1
 
     def finish(self):

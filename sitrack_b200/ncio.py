@@ -22,7 +22,7 @@ from .util import epoch2clock as e2c
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
            "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter",
-           "DeformationScalingWriter", "DeformationGridWriter"]
+           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -505,6 +505,86 @@ class DeformationGridWriter:
                 for fn in sorted(os.listdir(self._tmp)):
                     z.write(os.path.join(self._tmp, fn), arcname=fn)
             shutil.rmtree(self._tmp, ignore_errors=True)
+        print('      ===> ' + self.cf_out + ' saved!')
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DispersionWriter:
+    """Window-by-window writer of the per-lag, per-class statistics of pair dispersion (sitrack_b200.dispersion,
+    TrackEngine.track's `dispersion`).  Dimensions time (windows), lag, class, bin, class_edge, bin_edge; variables
+      time_start, time_end (time) i4                 first and last date of each window [tunits]
+      lag_days (lag) f8                              time lag [day]
+      r_edges (class_edge) f8                        initial-separation class edges [km]
+      bin_edges (bin_edge) f8                        stretch-rate histogram edges [day-1]
+      n (time,lag,class) i8                          pairs that count
+      sum_r0, sum_dr, sum_dr2, sum_dD2 (time,lag,class) f8   sums of r0 [km], dr [km], dr^2 [km2], dD2 [km2]
+      hist_stretch (time,lag,class,bin) i8           counts of the stretch rate |dr| / (r0 tau) per bin
+    with `units` on every variable.  Sums, not means, so that windows add up to ensembles; no variable has a fill value
+    (a lag not reached yet has zero counts and sums).  netCDF4 when available and the name does not end in .npz;
+    otherwise an .npz with the same variables, plus `<name>_units` (0-d strings)."""
+
+    SUMS = (("sum_r0", "km"), ("sum_dr", "km"), ("sum_dr2", "km2"), ("sum_dD2", "km2"))
+
+    def __init__(self, cf_out, ntime, lag_days, r_edges, bin_edges, tunits=tunits_default, corigin=None):
+        print('\n *** [DispersionWriter]: About to generate file: ' + cf_out + ' ...')
+        lag_days, r_edges, bin_edges = (np.asarray(a, 'f8') for a in (lag_days, r_edges, bin_edges))
+        self.ntime = int(ntime)
+        units = dict(time_start=tunits, time_end=tunits, lag_days='day', r_edges='km', bin_edges='day-1', n='1',
+                     hist_stretch='1', **{n: u for n, u in self.SUMS})
+        size = dict(time=self.ntime, lag=lag_days.size, **{'class': r_edges.size + 1}, bin=bin_edges.size + 1)
+        shapes = dict(time_start=('i4', ('time',)), time_end=('i4', ('time',)), n=('i8', ('time', 'lag', 'class')),
+                      **{n: ('f8', ('time', 'lag', 'class')) for n, _ in self.SUMS},
+                      hist_stretch=('i8', ('time', 'lag', 'class', 'bin')))
+        nc = None
+        if not str(cf_out).endswith(".npz"):
+            try:
+                import netCDF4 as nc
+            except ImportError:
+                cf_out += ".npz"
+                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
+        self.cf_out, self._nc = cf_out, nc
+        if nc is None:
+            self._v = {n: np.zeros([size[d] for d in dims], dt) for n, (dt, dims) in shapes.items()}
+            self._v.update(lag_days=lag_days, r_edges=r_edges, bin_edges=bin_edges)
+            self._units = units
+        else:
+            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
+            f.createDimension('time', None)
+            for d in ('lag', 'class', 'bin'):
+                f.createDimension(d, size[d])
+            f.createDimension('class_edge', r_edges.size)
+            f.createDimension('bin_edge', bin_edges.size)
+            self._v = {n: f.createVariable(n, dt, dims) for n, (dt, dims) in shapes.items()}
+            for n, d, a in (('lag_days', 'lag', lag_days), ('r_edges', 'class_edge', r_edges),
+                            ('bin_edges', 'bin_edge', bin_edges)):
+                f.createVariable(n, 'f8', (d,))[:] = a
+            for n, u in units.items():
+                f.variables[n].units = u
+            if corigin:
+                f.Origin = corigin
+            f.About = 'Two-particle dispersion of buoy pairs over time lags, by initial separation'
+            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+
+    def write(self, jw, time_start, time_end, stats):
+        """Window jw: stats = the dict of sitrack_b200.PairDispersion / track(dispersion=...)."""
+        self._v['time_start'][jw] = time_start
+        self._v['time_end'][jw] = time_end
+        self._v['n'][jw] = np.asarray(stats['n'], 'i8')
+        for n, _ in self.SUMS:
+            self._v[n][jw] = np.asarray(stats[n], 'f8')
+        self._v['hist_stretch'][jw] = np.asarray(stats['hist_stretch'], 'i8')
+
+    def close(self):
+        if self._nc is not None:
+            self._f.close()
+        else:
+            extra = {n + '_units': np.array(u) for n, u in self._units.items()}
+            np.savez(self.cf_out, **self._v, **extra)
         print('      ===> ' + self.cf_out + ' saved!')
 
     def __enter__(self):
