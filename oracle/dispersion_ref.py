@@ -5,10 +5,10 @@ Method -- the contract of csrc/st_disperse.cu, sitrack_b200.dispersion and DESIG
 
 Pairs.     pairs (nQ,2) i4 of buoy indices in the caller's order, a != b, nQ >= 1; kept in that order.
 Windows.   As in section 10: with every = n, row (w+1)*n closes window w; row 0 is the state handed to set_buoys,
-           masked by the rec_first rule of _DeformRun.  The rows o*n, o = 0, 1, ..., are origins.  When window w
-           closes, lags l = 1 .. min(m, w+1) are evaluated between origin row (w+1-l)*n and row (w+1)*n, with
-           tau_l = l*n*rdt/86400 days.  Every (origin, lag) combination is evaluated exactly once in a run, so the sum
-           of the windows' statistics is the ensemble over all start times at every lag.
+           masked by the rec_first rule of the engine's _WindowRows.  The rows o*n, o = 0, 1, ..., are origins.
+           When window w closes, lags l = 1 .. min(m, w+1) are evaluated between origin row (w+1-l)*n and row
+           (w+1)*n, with tau_l = l*n*rdt/86400 days.  Every (origin, lag) combination is evaluated exactly once in a
+           run, so the sum of the windows' statistics is the ensemble over all start times at every lag.
 Per pair.  For one (origin, lag): valid when both buoys have mask != 0 in both rows.  In f8, in this order:
              dy0 = y_a - y_b, dx0 = x_a - x_b, r0 = sqrt(dy0*dy0 + dx0*dx0); dy1, dx1, r1 likewise at the lag row;
              dr = r1 - r0;  dD2 = (dy1-dy0)*(dy1-dy0) + (dx1-dx0)*(dx1-dx0);  s = |dr| / (r0*tau_l)  [day-1].

@@ -135,6 +135,16 @@ def record_windows(zTpos, nP, kstrt, kstop, ztime_model, iTmA, iTmB):
     return z1st, zLst
 
 
+def window_records(flag, hours):
+    """HOURS of `flag` -> records per window; ERROR and exit when it is not a positive multiple of the model time
+    step."""
+    n = hours * 3600. / rdt
+    if not (hours > 0 and abs(n - round(n)) < 1e-9 and round(n) >= 1):
+        print('ERROR: %s HOURS must be a positive multiple of the model time step (%g h), got %g' % (flag, rdt / 3600., hours))
+        exit(0)
+    return int(round(n))
+
+
 def deform_records(hours, world):
     """--deform HOURS -> records per deformation window (None without the flag); ERROR and exit when it is not a
     positive multiple of the model time step, or under torchrun (triangles would cross the ranks' shards)."""
@@ -143,45 +153,23 @@ def deform_records(hours, world):
     if world > 1:
         print('ERROR: --deform is not available with several processes (WORLD_SIZE > 1): triangles would cross ranks')
         exit(0)
-    n = hours * 3600. / rdt
-    if not (hours > 0 and abs(n - round(n)) < 1e-9 and round(n) >= 1):
-        print('ERROR: --deform HOURS must be a positive multiple of the model time step (%g h), got %g' % (rdt / 3600., hours))
-        exit(0)
-    return int(round(n))
+    return window_records('--deform', hours)
 
 
-def deform_scales_args(scales, hours):
-    """--deform-scales L0_KM LEVELS -> (L0_km, levels) or None; ERROR and exit without --deform, with L0 <= 0, or
-    with LEVELS not an integer in 1..20."""
-    if scales is None:
+def deform_levels_args(flag, levels, hours):
+    """`flag` L0_KM LEVELS (--deform-scales, --deform-grid) -> (L0_km, levels) or None; ERROR and exit without
+    --deform, with L0 <= 0, or with LEVELS not an integer in 1..20."""
+    if levels is None:
         return None
-    L0, lev = scales
+    L0, lev = levels
     if hours is None:
-        print('ERROR: --deform-scales needs --deform HOURS')
+        print('ERROR: %s needs --deform HOURS' % flag)
         exit(0)
     if not L0 > 0:
-        print('ERROR: --deform-scales L0_KM must be positive, got %g' % L0)
+        print('ERROR: %s L0_KM must be positive, got %g' % (flag, L0))
         exit(0)
     if lev != int(lev) or not 1 <= lev <= sit.MAX_LEVELS:
-        print('ERROR: --deform-scales LEVELS must be an integer in 1..%d, got %g' % (sit.MAX_LEVELS, lev))
-        exit(0)
-    return L0, int(lev)
-
-
-def deform_grid_args(grid, hours):
-    """--deform-grid L0_KM LEVELS -> (L0_km, levels) or None; ERROR and exit without --deform, with L0 <= 0, or with
-    LEVELS not an integer in 1..20."""
-    if grid is None:
-        return None
-    L0, lev = grid
-    if hours is None:
-        print('ERROR: --deform-grid needs --deform HOURS')
-        exit(0)
-    if not L0 > 0:
-        print('ERROR: --deform-grid L0_KM must be positive, got %g' % L0)
-        exit(0)
-    if lev != int(lev) or not 1 <= lev <= sit.MAX_LEVELS:
-        print('ERROR: --deform-grid LEVELS must be an integer in 1..%d, got %g' % (sit.MAX_LEVELS, lev))
+        print('ERROR: %s LEVELS must be an integer in 1..%d, got %g' % (flag, sit.MAX_LEVELS, lev))
         exit(0)
     return L0, int(lev)
 
@@ -200,10 +188,7 @@ def dispersion_args(disp, pairs, world):
     if world > 1:
         print('ERROR: --dispersion is not available with several processes (WORLD_SIZE > 1): pairs would cross ranks')
         exit(0)
-    n = hours * 3600. / rdt
-    if not (hours > 0 and abs(n - round(n)) < 1e-9 and round(n) >= 1):
-        print('ERROR: --dispersion HOURS must be a positive multiple of the model time step (%g h), got %g' % (rdt / 3600., hours))
-        exit(0)
+    n = window_records('--dispersion', hours)
     if lags != int(lags) or not 1 <= lags <= sit.MAX_LAGS:
         print('ERROR: --dispersion LAGS must be an integer in 1..%d, got %g' % (sit.MAX_LAGS, lags))
         exit(0)
@@ -214,7 +199,7 @@ def dispersion_args(disp, pairs, world):
     if not (r_min > 0 and r_max > r_min and np.isfinite(r_max)):
         print('ERROR: --dispersion-pairs needs 0 < R_MIN_KM < R_MAX_KM, got %g %g' % (r_min, r_max))
         exit(0)
-    return int(round(n)), int(lags), None if N is None else int(N), r_min, r_max
+    return n, int(lags), None if N is None else int(N), r_min, r_max
 
 
 def deform_grid_over(Yt, Xt, L0, levels):
@@ -237,8 +222,8 @@ def main():
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     args = __argument_parsing__()
     ndeform = deform_records(args.deform, world)
-    dscales = deform_scales_args(args.deform_scales, args.deform)
-    dgrid = deform_grid_args(args.deform_grid, args.deform)
+    dscales = deform_levels_args('--deform-scales', args.deform_scales, args.deform)
+    dgrid = deform_levels_args('--deform-grid', args.deform_grid, args.deform)
     dspa = dispersion_args(args.dispersion, args.dispersion_pairs, world)
     dist = None
     if world > 1:
@@ -343,12 +328,21 @@ def main():
     corgn = 'NEMO-SI3_' + ModConf + '_' + ModExp
     ext = '.npz' if str(cf_uv).endswith('.npz') else '.nc'
 
+    def nc_name(kind, t0, t1):
+        return './nc/' + corgn + '_' + kind + '_' + SeedBatch + cdtbin + '_' + hstr(t0) + '_' + hstr(t1) + csfkm + ext
+
+    writers = []                                                  # the per-window files, closed after track()
+
+    def window_sink(n, *wrs):
+        """sink(w, a, b, ...) of windows of n records: a into wrs[0], b into wrs[1], ... with the window's dates"""
+        writers.extend(wrs)
+        return lambda w, *a: [wr.write(w, vTime[w * n], vTime[(w + 1) * n], x) for wr, x in zip(wrs, a)]
+
     # Trajectory rows are written as they leave the GPU: the reference holds (Nt+1, nP, 2) arrays for the whole run
     # (:326-328), here only the two rows the `tracking12` file needs stay in memory.
     writer = None
     if rank == 0 and not lUse2DTime:
-        cf_nc_out = './nc/' + corgn + '_tracking_' + SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + hstr(vTime[Nt]) + csfkm + ext
-        writer = sit.CloudBuoyWriter(cf_nc_out, Nt + 1, IDs, with_mask=True, corigin=corgn)
+        writer = sit.CloudBuoyWriter(nc_name('tracking', vTime[0], vTime[Nt]), Nt + 1, IDs, with_mask=True, corigin=corgn)
         writer.write(0, vTime[0], xPosC0[:, 0], xPosC0[:, 1], xPosG0[:, 0], xPosG0[:, 1], mask=np.ones(nP, 'i1'))
     z2XY, z2GC, zMSK = np.zeros((2, nP, 2)), np.zeros((2, nP, 2)), np.zeros((2, nP), dtype='i1')
     z2XY[0], z2GC[0], zMSK[0] = xPosC0, xPosG0, 1                # each buoy's first row is its seed (:335-340)
@@ -396,31 +390,24 @@ def main():
             print('ERROR: --deform: no triangle left in the mesh of the buoys!')
             exit(0)
         print(' *** --deform: %d triangles, %d windows of %d records' % (tri.shape[0], nwin, ndeform))
-        cf_tail = SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + hstr(vTime[nwin * ndeform]) + csfkm + ext
-        cf_def = './nc/' + corgn + '_deformation_' + cf_tail
-        dwriter = sit.DeformationWriter(cf_def, nwin, tri, IDs, corigin=corgn)
-        deform = dict(tri=tri, every=ndeform,
-                      sink=lambda w, out: dwriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], out))
+        t1 = vTime[nwin * ndeform]
+        dwriter = sit.DeformationWriter(nc_name('deformation', vTime[0], t1), nwin, tri, IDs, corigin=corgn)
+        deform = dict(tri=tri, every=ndeform, sink=window_sink(ndeform, dwriter))
         if dscales:
             # boxes over the same mesh and seeds; only per-scale statistics leave the GPU
             H = sit.BoxHierarchy(xPosC0, tri, *dscales)
             print(' *** --deform-scales: %d levels of boxes from %g km, %s boxes' % (H.levels, H.L0_km, H.nbox.tolist()))
-            cf_sc = './nc/' + corgn + '_deformation-scaling_' + cf_tail
-            swriter = sit.DeformationScalingWriter(cf_sc, nwin, H.scale_km, H.bin_edges, corigin=corgn)
-            deform.update(scales=H, scale_sink=lambda w, st: swriter.write(w, vTime[w * ndeform],
-                                                                          vTime[(w + 1) * ndeform], st))
+            swriter = sit.DeformationScalingWriter(nc_name('deformation-scaling', vTime[0], t1), nwin, H.scale_km,
+                                                   H.bin_edges, corigin=corgn)
+            deform.update(scales=H, scale_sink=window_sink(ndeform, swriter))
         if G is not None:
             # fixed cells over the model grid, membership rebuilt every window; only fields and statistics leave the GPU
             print(' *** --deform-grid: %d levels of cells from %g km, %d x %d level-1 cells from (%g, %g) km'
                   % (G.levels, G.L0_km, G.shape[0], G.shape[1], G.origin[0], G.origin[1]))
-            gwriter = sit.DeformationGridWriter('./nc/' + corgn + '_deformation-grid_' + cf_tail, nwin, G, corigin=corgn)
-            gswriter = sit.DeformationScalingWriter('./nc/' + corgn + '_deformation-grid-scaling_' + cf_tail, nwin,
+            gwriter = sit.DeformationGridWriter(nc_name('deformation-grid', vTime[0], t1), nwin, G, corigin=corgn)
+            gswriter = sit.DeformationScalingWriter(nc_name('deformation-grid-scaling', vTime[0], t1), nwin,
                                                     G.scale_km, G.bin_edges, corigin=corgn)
-
-            def grid_sink(w, fields, st):
-                gwriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], fields)
-                gswriter.write(w, vTime[w * ndeform], vTime[(w + 1) * ndeform], st)
-            deform.update(grid=G, grid_sink=grid_sink)
+            deform.update(grid=G, grid_sink=window_sink(ndeform, gwriter, gswriter))
         small = False                                             # windows close inside the streaming record loop
     dispersion = None
     if dspa:
@@ -433,12 +420,10 @@ def main():
             exit(0)
         print(' *** --dispersion: %d pairs at %g to %g km, %d windows of %d records, lags 1..%d'
               % (pairs.shape[0], r_min, r_max, nwd, nd, lags))
-        cf_dsp = './nc/' + corgn + '_dispersion_' + SeedBatch + cdtbin + '_' + hstr(vTime[0]) + '_' + \
-            hstr(vTime[nwd * nd]) + csfkm + ext
-        pwriter = sit.DispersionWriter(cf_dsp, nwd, np.arange(1, lags + 1) * (nd * rdt / 86400.), sit.DEFAULT_R_EDGES,
+        pwriter = sit.DispersionWriter(nc_name('dispersion', vTime[0], vTime[nwd * nd]), nwd,
+                                       np.arange(1, lags + 1) * (nd * rdt / 86400.), sit.DEFAULT_R_EDGES,
                                        sit.DEFAULT_BIN_EDGES, corigin=corgn)
-        dispersion = dict(pairs=pairs, every=nd, lags=lags,
-                          sink=lambda w, st: pwriter.write(w, vTime[w * nd], vTime[(w + 1) * nd], st))
+        dispersion = dict(pairs=pairs, every=nd, lags=lags, sink=window_sink(nd, pwriter))
         small = False
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
@@ -451,15 +436,8 @@ def main():
                         row_dtype='f8' if physics else args.rows, physics=physics, deform=deform,
                         dispersion=dispersion)
     eng.close()
-    if deform:
-        dwriter.close()
-        if dscales:
-            swriter.close()
-        if G is not None:
-            gwriter.close()
-            gswriter.close()
-    if dispersion:
-        pwriter.close()
+    for w in writers:
+        w.close()
     ds.close()
     n_alive = res['n_alive']
     if world > 1:
@@ -487,9 +465,8 @@ def main():
     else:
         zTim = []
         zvt = np.array([vTime[0], vTime[Nt]])
-    cf_nc_out = './nc/' + corgn + '_tracking12_' + SeedBatch + cdtbin + '_' + hstr(zvt[0]) + '_' + hstr(zvt[1]) + csfkm + ext
-    sit.ncSaveCloudBuoys(cf_nc_out, zvt, IDs, z2XY[:, :, 0], z2XY[:, :, 1], z2GC[:, :, 0], z2GC[:, :, 1],
-                         mask=zMSK, xtime=zTim, corigin=corgn)
+    sit.ncSaveCloudBuoys(nc_name('tracking12', zvt[0], zvt[1]), zvt, IDs, z2XY[:, :, 0], z2XY[:, :, 1], z2GC[:, :, 0],
+                         z2GC[:, :, 1], mask=zMSK, xtime=zTim, corigin=corgn)
     print('        => global first and final dates in simulated trajectories:', e2c(zvt[0]), e2c(zvt[1]), '\n')
     return 0
 

@@ -83,29 +83,57 @@ def launch(L, ctx, nT, tri_t, yx0_t, m0_t, yx1_t, m1_t, dt_days, out_t, stream):
                           m1_t.data_ptr(), float(dt_days), out_t.data_ptr(), C.c_void_p(stream.cuda_stream)), ctx)
 
 
+class _Plan:
+    """The triangle pass of TrackEngine.track(deform=...) over a mesh `slots` ((nT,3) buoy indices as stored on the
+    device, caller's triangle order), sorted once by sort_mesh."""
+
+    def __init__(self, torch, dev, slots):
+        self.torch, self.L = torch, _lib.lib()
+        tri, self.inv = sort_mesh(slots)
+        self.nT = tri.shape[0]
+        self.tri_t = torch.from_numpy(tri).to(dev)
+
+    def outputs(self, pin=False):
+        """((6, max(nT,1)) f4,) on the device, or pinned on the host."""
+        kw = dict(pin_memory=True) if pin else dict(device=self.tri_t.device)
+        return (self.torch.empty((6, max(self.nT, 1)), dtype=self.torch.float32, **kw),)
+
+    def window(self, ctx, origins, yx1_t, m1_t, dt_days, outs, stream):
+        (yx0_t, m0_t, _), = origins
+        launch(self.L, ctx, self.nT, self.tri_t, yx0_t, m0_t, yx1_t, m1_t, dt_days, outs[0], stream)
+
+    def results(self, outs):
+        """(dict of (nT,) f4 DEFORM_NAMES in the caller's triangle order,)"""
+        o = outs[0].numpy()[:, :self.nT][:, self.inv]                # a copy
+        return ({n: o[j] for j, n in enumerate(DEFORM_NAMES)},)
+
+
+def _upload_rows(pYX0, pYX1, mask0, mask1, dt_days, device, nP=None):
+    """What the host entry points share: positions pYX0, pYX1 ((nP,2) [y,x] km) and masks mask0, mask1 (nP,) of the
+    same buoys (nP of them when given), dt_days apart, checked and uploaded to `device` (default config.device).
+    -> (torch, dev, nP, (yx0_t, m0_t, yx1_t, m1_t))."""
+    from .engine import _torch
+    from . import config
+    torch = _torch()
+    yx0, yx1 = as_c(pYX0, np.float64).reshape(-1, 2), as_c(pYX1, np.float64).reshape(-1, 2)
+    nP = yx0.shape[0] if nP is None else nP
+    if yx0.shape[0] != nP or yx1.shape[0] != nP or np.shape(mask0) != (nP,) or np.shape(mask1) != (nP,):
+        raise ValueError("pYX0, pYX1 (nP,2) and mask0, mask1 (nP,) must describe the same %d buoys" % nP)
+    if not dt_days > 0:
+        raise ValueError("dt_days must be positive")
+    dev = torch.device("cuda", config.device if device is None else int(device))
+    t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
+    return torch, dev, nP, (t(yx0, np.float64), t(mask0, np.int8), t(yx1, np.float64), t(mask1, np.int8))
+
+
 def DeformationRates(pYX0, pYX1, mask0, mask1, tri, dt_days, device=None):
     """-> dict of (nT,) f4 over DEFORM_NAMES for the triangles `tri` (nT,3) between positions pYX0 and pYX1
     ((nP,2) [y,x] km) with masks mask0, mask1 (nP,), dt_days apart.  Host arrays in and out; the rates are
     computed on the GPU by k_deform (no CPU fallback)."""
-    from .engine import _torch
-    from . import config
-    torch = _torch()
-    L = _lib.lib()
-    yx0, yx1 = as_c(pYX0, np.float64).reshape(-1, 2), as_c(pYX1, np.float64).reshape(-1, 2)
-    nP = yx0.shape[0]
-    if yx1.shape[0] != nP or np.shape(mask0) != (nP,) or np.shape(mask1) != (nP,):
-        raise ValueError("pYX0, pYX1 (nP,2) and mask0, mask1 (nP,) must describe the same buoys")
-    if not dt_days > 0:
-        raise ValueError("dt_days must be positive")
-    tri, inv = sort_mesh(check_mesh(tri, nP))
-    nT = tri.shape[0]
-    dev = torch.device("cuda", config.device if device is None else int(device))
+    torch, dev, nP, (yx0_t, m0_t, yx1_t, m1_t) = _upload_rows(pYX0, pYX1, mask0, mask1, dt_days, device)
     with torch.cuda.device(dev):
-        t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
-        tri_t, yx0_t, yx1_t = t(tri, np.int32), t(yx0, np.float64), t(yx1, np.float64)
-        m0_t, m1_t = t(mask0, np.int8), t(mask1, np.int8)
-        out_t = torch.empty((6, max(nT, 1)), dtype=torch.float32, device=dev)
-        s = torch.cuda.current_stream(dev)
-        launch(L, None, nT, tri_t, yx0_t, m0_t, yx1_t, m1_t, dt_days, out_t, s)
-        out = out_t[:, :nT].cpu().numpy()[:, inv]
-    return {n: as_c(out[j], np.float32) for j, n in enumerate(DEFORM_NAMES)}
+        plan = _Plan(torch, dev, check_mesh(tri, nP))
+        outs = plan.outputs()
+        plan.window(None, [(yx0_t, m0_t, 1)], yx1_t, m1_t, dt_days, outs, torch.cuda.current_stream(dev))
+        out, = plan.results([o.cpu() for o in outs])
+    return {n: as_c(o, np.float32) for n, o in out.items()}

@@ -16,15 +16,15 @@ import numpy as np
 
 from . import _lib
 from ._lib import as_c, check
-from .deform import check_mesh
-from .deform_scales import BOX_NAMES, DEFAULT_BIN_EDGES, MAX_EDGES, MAX_LEVELS, FillValue, stats_dict
+from .deform import _upload_rows, check_mesh
+from .deform_scales import BOX_NAMES, _Levels, stats_dict
 
 __all__ = ["EulerianGrid", "GriddedRates", "MAX_GRID_SIDE"]
 
 MAX_GRID_SIDE = 2 ** 20
 
 
-class EulerianGrid:
+class EulerianGrid(_Levels):
     """A fixed grid of shape = (nj, ni) level-1 cells (1..2^20 each) of side L0_km from origin_yx = (oy, ox) km, with
     `levels` (1..20) levels of sides L0_km * 2^s.  A cell counts when the area of its binned triangles is at least
     cover * L_s^2.  `bins`: histogram edges [1/day] (f8, strictly increasing; default DEFAULT_BIN_EDGES).
@@ -37,25 +37,12 @@ class EulerianGrid:
         o = np.asarray(origin_yx, np.float64).ravel()
         if o.shape != (2,) or not np.isfinite(o).all():
             raise ValueError("EulerianGrid: origin_yx must be two finite numbers (oy, ox) km, got %r" % (origin_yx,))
-        if not (np.isfinite(L0_km) and L0_km > 0):
-            raise ValueError("EulerianGrid: L0_km must be finite and positive, got %r" % (L0_km,))
         sh = tuple(shape) if np.ndim(shape) == 1 else ()
         if len(sh) != 2 or any(int(n) != n or not 1 <= n <= MAX_GRID_SIDE for n in sh):
             raise ValueError("EulerianGrid: shape must be two integers (nj, ni) in 1..%d, got %r" % (MAX_GRID_SIDE, shape))
-        if int(levels) != levels or not 1 <= levels <= MAX_LEVELS:
-            raise ValueError("EulerianGrid: levels must be an integer in 1..%d, got %r" % (MAX_LEVELS, levels))
-        if not (np.isfinite(cover) and cover > 0):
-            raise ValueError("EulerianGrid: cover must be positive, got %r" % (cover,))
-        edges = as_c(DEFAULT_BIN_EDGES if bins is None else bins, np.float64).ravel()
-        if not 1 <= edges.size <= MAX_EDGES or not np.isfinite(edges).all() or (np.diff(edges) <= 0).any():
-            raise ValueError("EulerianGrid: bins must be 1..%d finite, strictly increasing edges" % MAX_EDGES)
-        self.origin, self.L0_km, self.cover = o, float(L0_km), float(cover)
-        self.shape, self.levels = (int(sh[0]), int(sh[1])), int(levels)
-        self.bin_edges = edges
+        super().__init__("EulerianGrid", L0_km, levels, cover, bins)
+        self.origin, self.shape = o, (int(sh[0]), int(sh[1]))
         self.shapes = [(((self.shape[0] - 1) >> s) + 1, ((self.shape[1] - 1) >> s) + 1) for s in range(self.levels)]
-        self.L_km = self.L0_km * 2.0 ** np.arange(self.levels)
-        self.min_area = np.float64(self.cover) * self.L_km * self.L_km
-        self.scale_km = np.r_[FillValue, self.L_km]
 
     def centres(self, s):
         """(y_km (nj_s,), x_km (ni_s,)) cell-centre coordinates of level s (0-based)."""
@@ -107,6 +94,16 @@ class _GridPlan:
             self.scratch_bytes, mom_t.data_ptr(), hist_t.data_ptr(), fields_t.data_ptr(), nbox_t.data_ptr(),
             C.c_void_p(stream.cuda_stream)), ctx)
 
+    def window(self, ctx, origins, yx1_t, m1_t, dt_days, outs, stream):
+        """TrackEngine.track's pass over one window: origins = [(yx0_t, m0_t, 1)]."""
+        (yx0_t, m0_t, _), = origins
+        self.launch(ctx, yx0_t, m0_t, yx1_t, m1_t, dt_days, *outs, stream)
+
+    def results(self, outs):
+        """(fields, stats) of the window from its pinned outputs."""
+        mom, hist, fields, _ = (o.numpy() for o in outs)
+        return split_fields(self.G, fields), stats_dict(self.G, mom, hist)
+
 
 def split_fields(G, flat):
     """The flat f4 field buffer of one window -> per level dict of (nj_s, ni_s) f4 BOX_NAMES planes (copies) and the
@@ -132,24 +129,12 @@ def GriddedRates(pYX0, pYX1, mask0, mask1, tri, G, dt_days, device=None):
     total = eps_tot [1/day], L_eff [km], y_ctr, x_ctr [km, mid-time centroid]; FillValue where a cell has no binned
     triangle or does not count) and y_km (nj_s,), x_km (ni_s,) cell centres.  stats: as CoarseGrainedRates' (scale 0 =
     the binned triangles)."""
-    from .engine import _torch
-    from . import config
     if not isinstance(G, EulerianGrid):
         raise TypeError("G must be an EulerianGrid")
-    torch = _torch()
-    yx0, yx1 = as_c(pYX0, np.float64).reshape(-1, 2), as_c(pYX1, np.float64).reshape(-1, 2)
-    nP = yx0.shape[0]
-    if yx1.shape[0] != nP or np.shape(mask0) != (nP,) or np.shape(mask1) != (nP,):
-        raise ValueError("pYX0, pYX1 (nP,2) and mask0, mask1 (nP,) must describe the same %d buoys" % nP)
-    if not dt_days > 0:
-        raise ValueError("dt_days must be positive")
-    tri = check_mesh(tri, nP)
-    dev = torch.device("cuda", config.device if device is None else int(device))
+    torch, dev, nP, rows = _upload_rows(pYX0, pYX1, mask0, mask1, dt_days, device)
     with torch.cuda.device(dev):
-        t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
-        plan = _GridPlan(torch, dev, G, tri)
+        plan = _GridPlan(torch, dev, G, check_mesh(tri, nP))
         mom, hist, fields, nbox = plan.outputs()
-        plan.launch(None, t(yx0, np.float64), t(mask0, np.int8), t(yx1, np.float64), t(mask1, np.int8), dt_days,
-                    mom, hist, fields, nbox, torch.cuda.current_stream(dev))
+        plan.launch(None, *rows, dt_days, mom, hist, fields, nbox, torch.cuda.current_stream(dev))
         f, mom, hist = fields.cpu().numpy(), mom.cpu().numpy(), hist.cpu().numpy()
     return split_fields(G, f), stats_dict(G, mom, hist)

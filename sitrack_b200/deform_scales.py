@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import as_c, check
-from .deform import check_mesh
+from .deform import _upload_rows, check_mesh
 
 __all__ = ["BoxHierarchy", "CoarseGrainedRates", "BOX_NAMES", "DEFAULT_BIN_EDGES", "MAX_LEVELS"]
 
@@ -26,6 +26,34 @@ BOX_NAMES = ("divergence", "shear", "vorticity", "total", "L_eff", "y_ctr", "x_c
 DEFAULT_BIN_EDGES = np.array([10.0 ** (k / 10.0) for k in range(-50, 11)])   # 1e-5 ... 1e1 day-1, 10 bins per decade
 MAX_LEVELS = 20
 MAX_EDGES = 4096
+
+
+def check_edges(edges, default, limit, what):
+    """(n,) f8 histogram or class edges (`default` when None): 1..limit finite, strictly increasing values."""
+    e = as_c(default if edges is None else edges, np.float64).ravel()
+    if not 1 <= e.size <= limit or not np.isfinite(e).all() or (np.diff(e) <= 0).any():
+        raise ValueError("%s must be 1..%d finite, strictly increasing edges" % (what, limit))
+    return e
+
+
+class _Levels:
+    """What BoxHierarchy and EulerianGrid share, checked (ValueError prefixed by `who`): `levels` (1..MAX_LEVELS)
+    levels of square cells of sides L_km = L0_km * 2^s, a cell counting when its area is at least min_area =
+    cover * L_s^2, scale_km = (FillValue for the triangles, L_km...) and histogram edges bin_edges (`bins`, f8,
+    strictly increasing; default DEFAULT_BIN_EDGES)."""
+
+    def __init__(self, who, L0_km, levels, cover, bins):
+        if not (np.isfinite(L0_km) and L0_km > 0):
+            raise ValueError("%s: L0_km must be finite and positive, got %r" % (who, L0_km))
+        if int(levels) != levels or not 1 <= levels <= MAX_LEVELS:
+            raise ValueError("%s: levels must be an integer in 1..%d, got %r" % (who, MAX_LEVELS, levels))
+        if not (np.isfinite(cover) and cover > 0):
+            raise ValueError("%s: cover must be positive, got %r" % (who, cover))
+        self.bin_edges = check_edges(bins, DEFAULT_BIN_EDGES, MAX_EDGES, who + ": bins")
+        self.levels, self.L0_km, self.cover = int(levels), float(L0_km), float(cover)
+        self.L_km = self.L0_km * 2.0 ** np.arange(self.levels)
+        self.min_area = np.float64(self.cover) * self.L_km * self.L_km
+        self.scale_km = np.r_[FillValue, self.L_km]
 
 
 def _spread(v):
@@ -37,7 +65,7 @@ def _spread(v):
     return v
 
 
-class BoxHierarchy:
+class BoxHierarchy(_Levels):
     """Square material boxes over the triangles `tri` (nT,3) of buoys at positions pYX (nP,2) [y,x] km (the
     positions the mesh was built from), `levels` levels of sides L0_km * 2^s.  Host only (numpy), once per run.
 
@@ -55,23 +83,13 @@ class BoxHierarchy:
     def __init__(self, pYX, tri, L0_km, levels, cover=0.5, bins=None):
         yx = as_c(pYX, np.float64).reshape(-1, 2)
         self.nP = yx.shape[0]
-        if not (np.isfinite(L0_km) and L0_km > 0):
-            raise ValueError("BoxHierarchy: L0_km must be positive, got %r" % (L0_km,))
-        if int(levels) != levels or not 1 <= levels <= MAX_LEVELS:
-            raise ValueError("BoxHierarchy: levels must be an integer in 1..%d, got %r" % (MAX_LEVELS, levels))
-        if not (np.isfinite(cover) and cover > 0):
-            raise ValueError("BoxHierarchy: cover must be positive, got %r" % (cover,))
-        edges = as_c(DEFAULT_BIN_EDGES if bins is None else bins, np.float64).ravel()
-        if not 1 <= edges.size <= MAX_EDGES or not np.isfinite(edges).all() or (np.diff(edges) <= 0).any():
-            raise ValueError("BoxHierarchy: bins must be 1..%d finite, strictly increasing edges" % MAX_EDGES)
+        super().__init__("BoxHierarchy", L0_km, levels, cover, bins)
         self.tri = check_mesh(tri, self.nP).copy()
         nT = self.tri.shape[0]
         if nT == 0:
             raise ValueError("BoxHierarchy: the mesh has no triangle")
         if nT >= 2 ** 31:
             raise ValueError("BoxHierarchy: at most 2^31 - 1 triangles")
-        self.levels, self.L0_km, self.cover = int(levels), float(L0_km), float(cover)
-        self.bin_edges = edges
         t = self.tri
         c = np.stack([((yx[t[:, 0], k] + yx[t[:, 1], k]) + yx[t[:, 2], k]) / 3.0 for k in (0, 1)], 1)
         if not np.isfinite(c).all():
@@ -97,9 +115,6 @@ class BoxHierarchy:
             self.box_tri_off.append(np.r_[self.box_tri_off[-1][b], nT].astype(np.int64))
             self.keys.append(self.keys[-1][b] >> 1)
         self.nbox = np.array([k.shape[0] for k in self.keys], np.int64)
-        self.L_km = self.L0_km * 2.0 ** np.arange(self.levels)
-        self.min_area = np.float64(self.cover) * self.L_km * self.L_km
-        self.scale_km = np.r_[FillValue, self.L_km]
 
     def matches(self, tri, nP):
         """True when (tri, nP) is the mesh this hierarchy was built on."""
@@ -141,6 +156,15 @@ class _DevicePlan:
             self.scratch.data_ptr(), self.scratch_bytes, mom_t.data_ptr(), hist_t.data_ptr(),
             None if boxes_t is None else boxes_t.data_ptr(), C.c_void_p(stream.cuda_stream)), ctx)
 
+    def window(self, ctx, origins, yx1_t, m1_t, dt_days, outs, stream):
+        """TrackEngine.track's pass over one window: origins = [(yx0_t, m0_t, 1)]."""
+        (yx0_t, m0_t, _), = origins
+        self.launch(ctx, yx0_t, m0_t, yx1_t, m1_t, dt_days, *outs, None, stream)
+
+    def results(self, outs):
+        """(the statistics of the window,) from its pinned outputs."""
+        return (stats_dict(self.H, *(o.numpy() for o in outs)),)
+
 
 def stats_dict(H, mom, hist):
     """Host moments (S,4) and hist (S,3,nb+2) -> the statistics of one window (see CoarseGrainedRates)."""
@@ -159,25 +183,14 @@ def CoarseGrainedRates(pYX0, pYX1, mask0, mask1, H, dt_days, device=None):
     `key` (nbox,2) [bj, bi].  stats: scale_km (S,) (FillValue for the triangles), n (S,) i8 cells that count,
     sum_L_eff, sum_eps_tot, sum_eps_tot2, sum_eps_tot3 (S,) f8, hist_total, hist_divergence (of |div|), hist_shear
     (S, nb+2) i8 with underflow and overflow, bin_edges (nb+1,)."""
-    from .engine import _torch
-    from . import config
     if not isinstance(H, BoxHierarchy):
         raise TypeError("H must be a BoxHierarchy")
-    torch = _torch()
-    yx0, yx1 = as_c(pYX0, np.float64).reshape(-1, 2), as_c(pYX1, np.float64).reshape(-1, 2)
-    nP = yx0.shape[0]
-    if nP != H.nP or yx1.shape[0] != nP or np.shape(mask0) != (nP,) or np.shape(mask1) != (nP,):
-        raise ValueError("pYX0, pYX1 (nP,2) and mask0, mask1 (nP,) must describe the %d buoys of the hierarchy" % H.nP)
-    if not dt_days > 0:
-        raise ValueError("dt_days must be positive")
-    dev = torch.device("cuda", config.device if device is None else int(device))
+    torch, dev, _, rows = _upload_rows(pYX0, pYX1, mask0, mask1, dt_days, device, H.nP)
     with torch.cuda.device(dev):
-        t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
         plan = _DevicePlan(torch, dev, H, H.tri)
         mom, hist = plan.outputs()
         boxes_t = torch.empty((7, int(H.nbox.sum())), dtype=torch.float32, device=dev)
-        plan.launch(None, t(yx0, np.float64), t(mask0, np.int8), t(yx1, np.float64), t(mask1, np.int8), dt_days,
-                    mom, hist, boxes_t, torch.cuda.current_stream(dev))
+        plan.launch(None, *rows, dt_days, mom, hist, boxes_t, torch.cuda.current_stream(dev))
         o, mom, hist = boxes_t.cpu().numpy(), mom.cpu().numpy(), hist.cpu().numpy()
     b0 = np.r_[0, np.cumsum(H.nbox)]
     boxes = []

@@ -16,7 +16,8 @@ import numpy as np
 
 from . import _lib
 from ._lib import as_c, check
-from .deform_scales import DEFAULT_BIN_EDGES, MAX_EDGES
+from .deform import _upload_rows
+from .deform_scales import DEFAULT_BIN_EDGES, MAX_EDGES, check_edges
 
 __all__ = ["MeshPairs", "SeparationPairs", "PairDispersion", "check_pairs", "DEFAULT_R_EDGES", "MAX_LAGS",
            "PAIR_NAMES"]
@@ -81,13 +82,6 @@ def check_pairs(pairs, nP):
     return as_c(p, np.int32)
 
 
-def check_edges(edges, default, limit, what):
-    e = as_c(default if edges is None else edges, np.float64).ravel()
-    if not 1 <= e.size <= limit or not np.isfinite(e).all() or (np.diff(e) <= 0).any():
-        raise ValueError("%s must be 1..%d finite, strictly increasing edges" % (what, limit))
-    return e
-
-
 def check_lags(lags):
     if int(lags) != lags or not 1 <= lags <= MAX_LAGS:
         raise ValueError("lags must be an integer in 1..%d, got %r" % (MAX_LAGS, lags))
@@ -96,11 +90,12 @@ def check_lags(lags):
 
 class _Plan:
     """Device buffers of one set of pairs (buoy indices as stored on the device, caller's pair order), edges and
-    scratch for calls with up to `lags` active origins."""
+    scratch for calls with up to `lags` active origins.  Lag l is l * dt_days days in results()."""
 
-    def __init__(self, torch, dev, slots, lags, r_edges=None, bins=None):
+    def __init__(self, torch, dev, slots, lags, r_edges=None, bins=None, dt_days=None):
         self.torch, self.L = torch, _lib.lib()
         self.lags = check_lags(lags)
+        self.lag_days = None if dt_days is None else np.arange(1, self.lags + 1) * dt_days
         self.r_edges = check_edges(r_edges, DEFAULT_R_EDGES, MAX_CLASS_EDGES, "r_edges")
         self.bins = check_edges(bins, DEFAULT_BIN_EDGES, MAX_EDGES, "bins")
         t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
@@ -133,6 +128,14 @@ class _Plan:
             self.scratch_bytes, hist_t.data_ptr(), sums_t.data_ptr(),
             None if per_pair_t is None else per_pair_t.data_ptr(), C.c_void_p(stream.cuda_stream)), ctx)
 
+    def window(self, ctx, origins, yx1_t, m1_t, dt_days, outs, stream):
+        """TrackEngine.track's pass over one window: every active lag in one launch."""
+        self.launch(ctx, yx1_t, m1_t, origins, dt_days, *outs, None, stream)
+
+    def results(self, outs):
+        """(the statistics of the window,) from its pinned outputs."""
+        return (stats_dict(self.lag_days, self.r_edges, self.bins, *(o.numpy() for o in outs)),)
+
 
 def stats_dict(lag_days, r_edges, bins, hist, sums):
     """Host hist (m, C, NB) and sums (m, C, 4) -> the statistics of one window (see PairDispersion)."""
@@ -149,24 +152,12 @@ def PairDispersion(pYX0, pYX1, mask0, mask1, pairs, dt_days, r_edges=None, bins=
     -> (per_pair, stats).  per_pair: dict of (nQ,) f8 PAIR_NAMES r0, r1 [km], dr [km], dD2 [km2], FillValue where the
     pair does not count.  stats: lag_days (1,), r_edges, bin_edges, n (1, C) i8, sum_r0, sum_dr, sum_dr2, sum_dD2
     (1, C) f8 and hist_stretch (1, C, len(bins)+1) i8 of s = |dr| / (r0 dt_days), C = len(r_edges) + 1."""
-    from .engine import _torch
-    from . import config
-    torch = _torch()
-    yx0, yx1 = as_c(pYX0, np.float64).reshape(-1, 2), as_c(pYX1, np.float64).reshape(-1, 2)
-    nP = yx0.shape[0]
-    if yx1.shape[0] != nP or np.shape(mask0) != (nP,) or np.shape(mask1) != (nP,):
-        raise ValueError("pYX0, pYX1 (nP,2) and mask0, mask1 (nP,) must describe the same buoys")
-    if not dt_days > 0:
-        raise ValueError("dt_days must be positive")
-    pairs = check_pairs(pairs, nP)
-    dev = torch.device("cuda", config.device if device is None else int(device))
+    torch, dev, nP, (yx0_t, m0_t, yx1_t, m1_t) = _upload_rows(pYX0, pYX1, mask0, mask1, dt_days, device)
     with torch.cuda.device(dev):
-        t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
-        plan = _Plan(torch, dev, pairs, 1, r_edges, bins)
+        plan = _Plan(torch, dev, check_pairs(pairs, nP), 1, r_edges, bins)
         hist, sums = plan.outputs()
         pp = torch.empty((4, plan.nQ), dtype=torch.float64, device=dev)
-        plan.launch(None, t(yx1, np.float64), t(mask1, np.int8), [(t(yx0, np.float64), t(mask0, np.int8), 1)],
-                    dt_days, hist, sums, pp, torch.cuda.current_stream(dev))
+        plan.launch(None, yx1_t, m1_t, [(yx0_t, m0_t, 1)], dt_days, hist, sums, pp, torch.cuda.current_stream(dev))
         pp, hist, sums = pp.cpu().numpy(), hist.cpu().numpy(), sums.cpu().numpy()
     return ({n: pp[j].copy() for j, n in enumerate(PAIR_NAMES)},
             stats_dict([float(dt_days)], plan.r_edges, plan.bins, hist, sums))

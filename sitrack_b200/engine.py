@@ -484,8 +484,8 @@ class TrackEngine:
             return self._track_chunked(get, nrec, kstrt, pos0, posG0, rec_first, want_latlon, int(chunk), rdt)
         wrows = None if deform is None and dispersion is None else _WindowRows(self, torch, rec_first, kstrt,
                                                                                row_f4=rdt == torch.float32)
-        dfm = None if deform is None else _DeformRun(self, torch, dev, deform, wrows)
-        dsp = None if dispersion is None else _DispersionRun(self, torch, dev, dispersion, wrows, nrec)
+        runs = [run(self, torch, dev, spec, wrows, nrec)
+                for run, spec in ((_deform_run, deform), (_dispersion_run, dispersion)) if spec is not None]
         self.record_slots(2)
         stg = [self.staging(0), self.staging(1)]
         s_in, s_cmp, s_out = (torch.cuda.Stream(dev) for _ in range(3))
@@ -562,32 +562,24 @@ class TrackEngine:
                         l.copy_(d_ll[b], non_blocking=True)
                     m.copy_(d_mk[b], non_blocking=True)
                 ev_out[k] = torch.cuda.Event(); ev_out[k].record(s_out)
-                if dfm is not None:
-                    dfm.after_step(k, d_yx[b], d_mk[b], s_cmp, s_out)
-                if dsp is not None:
-                    dsp.after_step(k, d_yx[b], d_mk[b], s_cmp, s_out)
+                for run in runs:
+                    run.after_step(k, d_yx[b], d_mk[b], s_cmp, s_out)
             for k in range(max(0, nrec - NB), nrec):
                 if keep:
                     ev_out[k].synchronize()
                 else:
                     drain(k)
-            if dfm is not None:
-                dfm.finish()
-            if dsp is not None:
-                dsp.finish()
+            for run in runs:
+                run.finish()
         finally:
             if chain:
                 self.set_row_chain(False)                  # state up to date again (synchronises)
         torch.cuda.synchronize(dev)
         pool.shutdown()
         n_alive = d_na.cpu().numpy()
-        extra = {} if dfm is None or dfm.collected is None else dict(deform=dfm.collected)
-        if dfm is not None and dfm.scale_collected is not None:
-            extra["deform_scales"] = dfm.scale_collected
-        if dfm is not None and dfm.grid_collected is not None:
-            extra["deform_grid"] = dfm.grid_collected
-        if dsp is not None and dsp.collected is not None:
-            extra["dispersion"] = dsp.collected
+        extra = {}
+        for run in runs:
+            extra.update(run.collected)
         if not keep:
             return dict(n_alive=n_alive, **extra)
         posC, posG, mask = posC.numpy(), posG.numpy(), mask.numpy()
@@ -632,157 +624,81 @@ class _WindowRows:
         return self.state_pos if self.row_f4 else yx_row
 
 
-class _DeformRun:
-    """track(deform=...): the anchor row of the open window on the device, k_deform when a window closes, its
-    outputs to the host on the output stream.
-
-    Positions and row 0 as _WindowRows gives them.  Triangles are mapped into engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs go back to the
-    caller's triangle order on the host.  With `scales`, the box hierarchy pass runs on the same rows after k_deform
-    and before the anchor copy; its statistics go to the host on the output stream alongside the triangles'.  With
-    `grid`, the Eulerian grid pass follows on the same rows, over the triangles in the caller's order (mapped to
-    engine slots), and its fields and statistics go to the host the same way."""
-
-    def __init__(self, eng, torch, dev, spec, rows):
-        from . import deform as D
-        self.eng, self.torch, self.rows, self.D = eng, torch, rows, D
-        self.every = int(spec["every"])
-        if self.every < 1:
-            raise ValueError("deform: every must be >= 1 record")
-        self.sink = spec.get("sink")
-        self.collected = [] if self.sink is None else None
-        nP = eng.nP
-        tri = rows.slots(D.check_mesh(spec["tri"], nP))
-        self.scales = None
-        H = spec.get("scales")
-        if H is not None:
-            from . import deform_scales as DS
-            if not isinstance(H, DS.BoxHierarchy) or not H.matches(spec["tri"], nP):
-                raise ValueError("deform: scales must be a BoxHierarchy built on the same mesh (tri) and %d buoys" % nP)
-            # triangles keep the hierarchy's order (mapped to engine slots only): the sums do not depend on `perm`
-            self.scales = DS._DevicePlan(torch, dev, H, tri)
-            self.d_st = [self.scales.outputs() for _ in range(2)]
-            self.h_st = [self.scales.outputs(pin=True) for _ in range(2)]
-            self.DS, self.H = DS, H
-        self.scale_sink = spec.get("scale_sink")
-        self.scale_collected = [] if H is not None and self.scale_sink is None else None
-        self.grid = None
-        G = spec.get("grid")
-        if G is not None:
-            from . import deform_grid as DG
-            if not isinstance(G, DG.EulerianGrid):
-                raise ValueError("deform: grid must be an EulerianGrid")
-            # caller's triangle order (mapped to engine slots only): ties of the sort, hence the sums, do not depend
-            # on `perm`
-            self.grid = DG._GridPlan(torch, dev, G, tri)
-            self.d_gr = [self.grid.outputs() for _ in range(2)]
-            self.h_gr = [self.grid.outputs(pin=True) for _ in range(2)]
-            self.DG, self.G = DG, G
-        self.grid_sink = spec.get("grid_sink")
-        self.grid_collected = [] if G is not None and self.grid_sink is None else None
-        tri, self.inv = D.sort_mesh(tri)
-        self.nT = tri.shape[0]
-        self.dt = self.every * eng.rdt / 86400.0
-        self.tri_t = torch.from_numpy(tri).to(dev)
-        # the anchor: row 0 (on torch's current stream; track's streams wait for it)
-        self.a_yx = rows.state_pos.clone()
-        self.a_mk = torch.from_numpy(rows.m0).to(dev)
-        self.d_out = [torch.empty((6, max(self.nT, 1)), dtype=torch.float32, device=dev) for _ in range(2)]
-        self.h_out = [torch.empty((6, max(self.nT, 1)), dtype=torch.float32).pin_memory() for _ in range(2)]
-        self.ev_out = []
-        self.drained = 0
-
-    def after_step(self, k, yx_row, mk_row, s_cmp, s_out):
-        """Step k has been queued on s_cmp: row k+1 closes window w when k+1 = (w+1)*every."""
-        if (k + 1) % self.every:
-            return
-        torch, w = self.torch, (k + 1) // self.every - 1
-        b = w % 2
-        if w >= 2:
-            s_cmp.wait_event(self.ev_out[w - 2])                   # d_out[b] has reached the host
-        yx = self.rows.yx(yx_row)
-        self.D.launch(self.eng.L, self.eng.h, self.nT, self.tri_t, self.a_yx, self.a_mk, yx, mk_row, self.dt,
-                      self.d_out[b], s_cmp)
-        if self.scales is not None:
-            self.scales.launch(self.eng.h, self.a_yx, self.a_mk, yx, mk_row, self.dt, *self.d_st[b], None, s_cmp)
-        if self.grid is not None:
-            self.grid.launch(self.eng.h, self.a_yx, self.a_mk, yx, mk_row, self.dt, *self.d_gr[b], s_cmp)
-        with torch.cuda.stream(s_cmp):                              # row (w+1)*every anchors the next window
-            self.a_yx.copy_(yx)
-            self.a_mk.copy_(mk_row)
-        ev = torch.cuda.Event(); ev.record(s_cmp)
-        if w >= 2:
-            self._drain(w - 2)                                      # h_out[b] is free again
-        s_out.wait_event(ev)
-        with torch.cuda.stream(s_out):
-            self.h_out[b].copy_(self.d_out[b], non_blocking=True)
-            if self.scales is not None:
-                for h, d in zip(self.h_st[b], self.d_st[b]):
-                    h.copy_(d, non_blocking=True)
-            if self.grid is not None:
-                for h, d in zip(self.h_gr[b], self.d_gr[b]):
-                    h.copy_(d, non_blocking=True)
-        self.ev_out.append(torch.cuda.Event()); self.ev_out[w].record(s_out)
-
-    def _drain(self, w):
-        self.ev_out[w].synchronize()
-        o = self.h_out[w % 2].numpy()[:, :self.nT][:, self.inv]     # a copy, in the caller's triangle order
-        out = {n: o[j] for j, n in enumerate(self.D.DEFORM_NAMES)}
-        if self.sink is None:
-            self.collected.append(out)
-        else:
-            self.sink(w, out)
-        if self.scales is not None:
-            st = self.DS.stats_dict(self.H, *(h.numpy() for h in self.h_st[w % 2]))
-            if self.scale_sink is None:
-                self.scale_collected.append(st)
-            else:
-                self.scale_sink(w, st)
-        if self.grid is not None:
-            mom, hist, fields, _ = (h.numpy() for h in self.h_gr[w % 2])
-            fl, st = self.DG.split_fields(self.G, fields), self.DG.stats_dict(self.G, mom, hist)
-            if self.grid_sink is None:
-                self.grid_collected.append((fl, st))
-            else:
-                self.grid_sink(w, fl, st)
-        self.drained = w + 1
-
-    def finish(self):
-        for w in range(self.drained, len(self.ev_out)):
-            self._drain(w)
+def _window_every(spec, what):
+    """spec["every"]: records per window, >= 1."""
+    every = int(spec["every"])
+    if every < 1:
+        raise ValueError("%s: every must be >= 1 record" % what)
+    return every
 
 
-class _DispersionRun:
-    """track(dispersion=...): the ring of origin rows on the device, st_dispersion_dev over every active lag when a
-    window closes, its statistics to the host on the output stream.
+def _deform_run(eng, torch, dev, spec, rows, nrec):
+    """track(deform=...): triangles, then the box hierarchy (`scales`), then the Eulerian grid (`grid`), over the
+    window's anchor row and its closing row.
 
-    Origin row o (= row o*every) lives in ring slot o % lags.  When window w closes the launch reads the origins
-    w+1-l, l = 1 .. min(lags, w+1), on the compute stream; only after it is the closing row, origin w+1, copied into
-    slot (w+1) % lags, the slot of origin w+1-lags that the launch has just read for the last time.  Pairs are mapped
-    to engine slots without reordering them, so the sums do not depend on `perm`."""
+    Triangles are mapped into engine order (set_buoys sort=True) and sorted once by their smallest vertex; the outputs
+    go back to the caller's triangle order on the host.  The hierarchy keeps its own triangle order and the grid the
+    caller's (both mapped to engine slots only), so neither's sums depend on `perm`."""
+    from . import deform as D
+    every = _window_every(spec, "deform")
+    nP = eng.nP
+    tri = rows.slots(D.check_mesh(spec["tri"], nP))
+    passes = [("deform", spec.get("sink"), D._Plan(torch, dev, tri))]
+    H = spec.get("scales")
+    if H is not None:
+        from . import deform_scales as DS
+        if not isinstance(H, DS.BoxHierarchy) or not H.matches(spec["tri"], nP):
+            raise ValueError("deform: scales must be a BoxHierarchy built on the same mesh (tri) and %d buoys" % nP)
+        passes.append(("deform_scales", spec.get("scale_sink"), DS._DevicePlan(torch, dev, H, tri)))
+    G = spec.get("grid")
+    if G is not None:
+        from . import deform_grid as DG
+        if not isinstance(G, DG.EulerianGrid):
+            raise ValueError("deform: grid must be an EulerianGrid")
+        passes.append(("deform_grid", spec.get("grid_sink"), DG._GridPlan(torch, dev, G, tri)))
+    return _WindowRun(eng, torch, dev, rows, every, nrec, 1, passes)
 
-    def __init__(self, eng, torch, dev, spec, rows, nrec):
-        from . import dispersion as P
-        self.eng, self.torch, self.rows, self.P = eng, torch, rows, P
-        self.every = int(spec["every"])
-        if self.every < 1:
-            raise ValueError("dispersion: every must be >= 1 record")
-        self.lags = P.check_lags(spec["lags"])
-        pairs = P.check_pairs(spec["pairs"], eng.nP)
-        self.plan = P._Plan(torch, dev, rows.slots(pairs), self.lags, spec.get("r_edges"), spec.get("bins"))
-        self.sink = spec.get("sink")
-        self.collected = [] if self.sink is None else None
-        self.dt = self.every * eng.rdt / 86400.0
-        self.lag_days = np.arange(1, self.lags + 1) * self.dt
-        self.nwin = nrec // self.every
-        nslot = max(1, min(self.lags, self.nwin))                   # origins 0 .. nwin-1 are the only ones read
+
+def _dispersion_run(eng, torch, dev, spec, rows, nrec):
+    """track(dispersion=...): every active lag in one pass.  Pairs are mapped to engine slots without reordering
+    them, so the sums do not depend on `perm`."""
+    from . import dispersion as P
+    every = _window_every(spec, "dispersion")
+    lags = P.check_lags(spec["lags"])
+    pairs = P.check_pairs(spec["pairs"], eng.nP)
+    plan = P._Plan(torch, dev, rows.slots(pairs), lags, spec.get("r_edges"), spec.get("bins"),
+                   dt_days=every * eng.rdt / 86400.0)
+    return _WindowRun(eng, torch, dev, rows, every, nrec, lags, [("dispersion", spec.get("sink"), plan)])
+
+
+class _WindowRun:
+    """The windows of one analysis of track(): a ring of origin rows on the device, its passes when a window closes,
+    their outputs to the host on the output stream.
+
+    passes: [(result key, sink or None, plan)]; a plan has outputs(pin), window(ctx, origins, yx1, m1, dt_days, outs,
+    stream) and results(host outs) -> the sink's arguments after the window index.  Origin row o (= row o*every)
+    lives in ring slot o % nslot, nslot = min(lags, windows) (row 0 in slot 0, as _WindowRows gives it).  When window
+    w closes every pass reads the origins w+1-l, l = 1 .. min(lags, w+1), on the compute stream; only after them is
+    the closing row, origin w+1, copied into slot (w+1) % nslot, the slot of origin w+1-lags that they have just read
+    for the last time (no slot index reaches nslot < lags; origins 0 .. windows-1 are the only ones read).  Outputs
+    are double-buffered: window w's reach the sinks, or the lists under their keys in `collected`, when window w+2
+    closes or at finish()."""
+
+    def __init__(self, eng, torch, dev, rows, every, nrec, lags, passes):
+        self.ctx, self.torch, self.rows, self.passes = eng.h, torch, rows, passes
+        self.every, self.lags = every, lags
+        self.dt = every * eng.rdt / 86400.0
+        self.nwin = nrec // every
+        nslot = max(1, min(lags, self.nwin))
         nP = eng.nP
         # slot 0: row 0 (on torch's current stream; track's streams wait for it)
         self.r_yx = [rows.state_pos.clone()] + [torch.empty((nP, 2), dtype=torch.float64, device=dev)
                                                  for _ in range(nslot - 1)]
         self.r_mk = [torch.from_numpy(rows.m0).to(dev)] + [torch.empty((nP,), dtype=torch.int8, device=dev)
                                                            for _ in range(nslot - 1)]
-        self.d_st = [self.plan.outputs() for _ in range(2)]
-        self.h_st = [self.plan.outputs(pin=True) for _ in range(2)]
+        self.d_out = [[plan.outputs() for _, _, plan in passes] for _ in range(2)]
+        self.h_out = [[plan.outputs(pin=True) for _, _, plan in passes] for _ in range(2)]
+        self.collected = {key: [] for key, sink, _ in passes if sink is None}
         self.ev_out = []
         self.drained = 0
 
@@ -790,33 +706,37 @@ class _DispersionRun:
         """Step k has been queued on s_cmp: row k+1 closes window w when k+1 = (w+1)*every."""
         if (k + 1) % self.every:
             return
-        torch, w, L = self.torch, (k + 1) // self.every - 1, self.lags
+        torch, w, n = self.torch, (k + 1) // self.every - 1, len(self.r_yx)
         b = w % 2
         if w >= 2:
-            s_cmp.wait_event(self.ev_out[w - 2])                   # d_st[b] has reached the host
+            s_cmp.wait_event(self.ev_out[w - 2])                   # d_out[b] has reached the host
         yx = self.rows.yx(yx_row)
-        origins = [(self.r_yx[(w + 1 - l) % L], self.r_mk[(w + 1 - l) % L], l) for l in range(1, min(L, w + 1) + 1)]
-        self.plan.launch(self.eng.h, yx, mk_row, origins, self.dt, *self.d_st[b], None, s_cmp)
+        origins = [(self.r_yx[(w + 1 - l) % n], self.r_mk[(w + 1 - l) % n], l)
+                   for l in range(1, min(self.lags, w + 1) + 1)]
+        for (_, _, plan), outs in zip(self.passes, self.d_out[b]):
+            plan.window(self.ctx, origins, yx, mk_row, self.dt, outs, s_cmp)
         if w + 1 < self.nwin:
-            with torch.cuda.stream(s_cmp):                          # after the launch that read the slot last
-                self.r_yx[(w + 1) % L].copy_(yx)
-                self.r_mk[(w + 1) % L].copy_(mk_row)
+            with torch.cuda.stream(s_cmp):                          # after the passes that read the slot last
+                self.r_yx[(w + 1) % n].copy_(yx)
+                self.r_mk[(w + 1) % n].copy_(mk_row)
         ev = torch.cuda.Event(); ev.record(s_cmp)
         if w >= 2:
-            self._drain(w - 2)                                      # h_st[b] is free again
+            self._drain(w - 2)                                      # h_out[b] is free again
         s_out.wait_event(ev)
         with torch.cuda.stream(s_out):
-            for h, d in zip(self.h_st[b], self.d_st[b]):
-                h.copy_(d, non_blocking=True)
+            for hs, ds in zip(self.h_out[b], self.d_out[b]):
+                for h, d in zip(hs, ds):
+                    h.copy_(d, non_blocking=True)
         self.ev_out.append(torch.cuda.Event()); self.ev_out[w].record(s_out)
 
     def _drain(self, w):
         self.ev_out[w].synchronize()
-        st = self.P.stats_dict(self.lag_days, self.plan.r_edges, self.plan.bins, *(h.numpy() for h in self.h_st[w % 2]))
-        if self.sink is None:
-            self.collected.append(st)
-        else:
-            self.sink(w, st)
+        for (key, sink, plan), h in zip(self.passes, self.h_out[w % 2]):
+            r = plan.results(h)
+            if sink is None:
+                self.collected[key].append(r[0] if len(r) == 1 else r)
+            else:
+                sink(w, *r)
         self.drained = w + 1
 
     def finish(self):

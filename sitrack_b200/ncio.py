@@ -12,7 +12,10 @@ The km coordinates of the grid come from the device projection kernel
 import math
 import os
 import re
+import shutil
 import sys
+import tempfile
+import zipfile
 
 import numpy as np
 
@@ -144,28 +147,19 @@ def GetModelSeaIceConc(fNCsi3, name='siconc', krec=0, expected_shape=[]):
     return sic
 
 
-# (variable, dtype, dims, units, use fill value) of the buoy-cloud file, ncio.py:153-172
-_CLOUD_VARS = [
-    ('latitude', 'f4', 'degrees north'), ('longitude', 'f4', 'degrees south'),      # sic (ncio.py:164)
-    ('y_pos', 'f4', 'km'), ('x_pos', 'f4', 'km'),
-]
+class _OutFile:
+    """One output file of the writers below, created with its dimensions `dims` (name -> size; `time` is unlimited
+    on netCDF4) and global attributes About, Author, Origin (corigin, if given) and `attrs`.
 
+    netCDF4 when it imports and the name does not end in .npz; otherwise `<name>.npz` with the same variables, each an
+    on-disk .npy member (numpy memmap) in a temporary directory next to the output, zipped (deflate) at close, never
+    held in memory.  The .npz also holds the `attrs` as members, a 0-d string member `<name>_units` for every variable
+    with units and, with `fill` given, a `FillValue` member of fill's type; npz_attrs=False (the cloud-of-buoys file,
+    which mirrors the reference's file that LoadNCdata reads back) leaves out all of these.  Variables are `_v[name]`,
+    written by index like netCDF4 variables."""
 
-class CloudBuoyWriter:
-    """Record-by-record writer of a cloud-of-buoys file: the variables, dtypes and attributes of ncSaveCloudBuoys
-    (reference ncio.py:131-197), one `write(jt, ...)` per trajectory row, so that a run never has to hold the
-    (Nt+1, nP, 2) series the reference allocates (si3_part_tracker.py:326-328; SURVEY section 5 "output volume").
-    netCDF4 when available and the name does not end in .npz (unlimited `time` dimension, rows appended as they
-    come); otherwise an .npz with the same variables, assembled from on-disk .npy members (numpy memmaps), never
-    from arrays in memory."""
-
-    def __init__(self, cf_out, ntime, pIDs, with_mask=False, with_time_pos=False, tunits=tunits_default,
-                 fillVal=FillValue, corigin=None):
-        print('\n *** [ncSaveCloudBuoys]: About to generate file: ' + cf_out + ' ...')
-        self.ntime, self.nP = int(ntime), int(np.shape(pIDs)[0])
-        self.names = [n for n, _, _ in _CLOUD_VARS] + (['mask'] if with_mask else []) + (['time_pos'] if with_time_pos else [])
-        self._dt = {n: dt for n, dt, _ in _CLOUD_VARS}
-        self._dt.update(mask='i1', time_pos='i4')
+    def __init__(self, cf_out, who, dims, about, corigin=None, fill=None, npz_attrs=True, **attrs):
+        print('\n *** [%s]: About to generate file: %s ...' % (who, cf_out))
         nc = None
         if not str(cf_out).endswith(".npz"):
             try:
@@ -173,37 +167,92 @@ class CloudBuoyWriter:
             except ImportError:
                 cf_out += ".npz"
                 print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
-        self.cf_out, self._nc = cf_out, nc
+        self.cf_out, self._nc, self.dims, self.fill, self._npz_attrs = cf_out, nc, dims, fill, npz_attrs
+        self._v = {}
         if nc is None:
-            import tempfile
-            self._tmp = tempfile.mkdtemp(prefix=".cloud_", dir=os.path.dirname(os.path.abspath(cf_out)) or ".")
-            mm = lambda n, dt, shp: np.lib.format.open_memmap(os.path.join(self._tmp, n + ".npy"), mode='w+', dtype=dt, shape=shp)
-            self._v = {n: mm(n, self._dt[n], (self.ntime, self.nP)) for n in self.names}
-            self._v['time'] = mm('time', 'i4', (self.ntime,))
-            mm('buoy', 'i4', (self.nP,))[:] = np.arange(self.nP, dtype='i4')
-            mm('id_buoy', 'i8', (self.nP,))[:] = np.asarray(pIDs).astype('i8')
+            self._tmp = tempfile.mkdtemp(prefix=".sitrack_", dir=os.path.dirname(os.path.abspath(cf_out)) or ".")
+            if npz_attrs:
+                if fill is not None:
+                    attrs['FillValue'] = fill
+                for n, a in attrs.items():
+                    np.save(os.path.join(self._tmp, n + ".npy"), a)
         else:
             f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
-            f.createDimension('time', None)
-            f.createDimension('buoy', self.nP)
-            vt = f.createVariable('time', 'i4', ('time',)); vt.units = tunits
-            f.createVariable('buoy', 'i4', ('buoy',))[:] = np.arange(self.nP, dtype='i8')
-            vid = f.createVariable('id_buoy', 'i8', ('buoy',)); vid.units = 'ID of buoy'
-            vid[:] = np.asarray(pIDs)[:]
-            zkw = dict(zlib=True, complevel=9)
-            self._v = {'time': vt}
-            for name, dt, units in _CLOUD_VARS:
-                self._v[name] = f.createVariable(name, dt, ('time', 'buoy'), fill_value=fillVal, **zkw)
-                self._v[name].units = units
-            if with_mask:
-                self._v['mask'] = f.createVariable('mask', 'i1', ('time', 'buoy'), **zkw)
-            if with_time_pos:
-                self._v['time_pos'] = f.createVariable('time_pos', 'i4', ('time', 'buoy'), fill_value=fillVal, **zkw)
-                self._v['time_pos'].units = tunits
+            for d, n in dims.items():
+                f.createDimension(d, None if d == 'time' else n)
+            for n, a in attrs.items():
+                setattr(f, n, a)
             if corigin:
                 f.Origin = corigin
-            f.About = 'Lagrangian sea-ice drift'
+            f.About = about
             f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+
+    def var(self, name, dtype, dims, units=None, fill=False, zlib=False, data=None):
+        """Variable `name` over the dimensions `dims`; fill: with the file's fill value; zlib: compressed on netCDF4
+        (every .npz member is); data: its whole content."""
+        if self._nc is None:
+            v = np.lib.format.open_memmap(os.path.join(self._tmp, name + ".npy"), mode='w+', dtype=dtype,
+                                          shape=tuple(self.dims[d] for d in dims))
+            if units is not None and self._npz_attrs:
+                np.save(os.path.join(self._tmp, name + "_units.npy"), np.array(units))
+        else:
+            kw = dict(fill_value=self.fill) if fill else {}
+            v = self._f.createVariable(name, dtype, dims, **kw, **(dict(zlib=True, complevel=9) if zlib else {}))
+            if units is not None:
+                v.units = units
+        if data is not None:
+            v[:] = data
+        self._v[name] = v
+
+    def close(self):
+        if self._nc is not None:
+            self._f.close()
+        else:
+            for v in self._v.values():
+                v.flush()
+            self._v = {}
+            with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
+                for fn in sorted(os.listdir(self._tmp)):
+                    z.write(os.path.join(self._tmp, fn), arcname=fn)         # streamed from disk
+            shutil.rmtree(self._tmp, ignore_errors=True)
+        print('      ===> ' + self.cf_out + ' saved!')
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+# (variable, dtype, units) of the buoy-cloud file, ncio.py:153-172
+_CLOUD_VARS = [
+    ('latitude', 'f4', 'degrees north'), ('longitude', 'f4', 'degrees south'),      # sic (ncio.py:164)
+    ('y_pos', 'f4', 'km'), ('x_pos', 'f4', 'km'),
+]
+
+
+class CloudBuoyWriter(_OutFile):
+    """Record-by-record writer of a cloud-of-buoys file: the variables, dtypes and attributes of ncSaveCloudBuoys
+    (reference ncio.py:131-197), one `write(jt, ...)` per trajectory row, so that a run never has to hold the
+    (Nt+1, nP, 2) series the reference allocates (si3_part_tracker.py:326-328; SURVEY section 5 "output volume").
+    netCDF4 (unlimited `time` dimension, rows appended as they come) or an .npz with the same variables and no other
+    member (see _OutFile)."""
+
+    def __init__(self, cf_out, ntime, pIDs, with_mask=False, with_time_pos=False, tunits=tunits_default,
+                 fillVal=FillValue, corigin=None):
+        self.ntime, self.nP = int(ntime), int(np.shape(pIDs)[0])
+        super().__init__(cf_out, 'ncSaveCloudBuoys', dict(time=self.ntime, buoy=self.nP), 'Lagrangian sea-ice drift',
+                         corigin, fill=fillVal, npz_attrs=False)
+        self.names = [n for n, _, _ in _CLOUD_VARS] + (['mask'] if with_mask else []) + (['time_pos'] if with_time_pos else [])
+        self.var('time', 'i4', ('time',), units=tunits)
+        self.var('buoy', 'i4', ('buoy',), data=np.arange(self.nP, dtype='i8'))
+        self.var('id_buoy', 'i8', ('buoy',), units='ID of buoy', data=np.asarray(pIDs))
+        for name, dt, units in _CLOUD_VARS:
+            self.var(name, dt, ('time', 'buoy'), units=units, fill=True, zlib=True)
+        if with_mask:
+            self.var('mask', 'i1', ('time', 'buoy'), zlib=True)
+        if with_time_pos:
+            self.var('time_pos', 'i4', ('time', 'buoy'), units=tunits, fill=True, zlib=True)
 
     def write(self, jt, time, y, x, lat, lon, mask=None, time_pos=None):
         """Row jt of every variable ((nP,) arrays, any float dtype: stored as f4 like the reference's file)."""
@@ -212,85 +261,31 @@ class CloudBuoyWriter:
         for n in self.names:
             self._v[n][jt, :] = np.asarray(row[n])
 
-    def close(self):
-        if self._nc is not None:
-            self._f.close()
-        else:
-            import shutil
-            import zipfile
-            for v in self._v.values():
-                v.flush()
-            self._v = {}
-            with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
-                for fn in sorted(os.listdir(self._tmp)):
-                    z.write(os.path.join(self._tmp, fn), arcname=fn)         # streamed from disk, like np.savez's members
-            shutil.rmtree(self._tmp, ignore_errors=True)
-        print('      ===> ' + self.cf_out + ' saved!')
 
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-
-class DeformationWriter:
+class DeformationWriter(_OutFile):
     """Window-by-window writer of the strain rates of buoy triangles (sitrack_b200.deform, TrackEngine.track's
     `deform`).  Dimensions time (windows), triangle, vertex = 3; variables
       time_start, time_end (time) i4          first and last date of each window [tunits]
       vertices (triangle,vertex) i4           indices into the `buoy` axis of the tracking file
       id_vertices (triangle,vertex) i8        IDs of those buoys
       divergence, shear, vorticity (time,triangle) f4 [day-1]; area f4 [km2]; y_ctr, x_ctr f4 [km]
-    each output with `units` and the fill value `fillVal` for invalid triangles.  netCDF4 when available and the
-    name does not end in .npz; otherwise an .npz with the same variables, plus `<name>_units` (0-d strings) and
-    `FillValue` members for the attributes, assembled from on-disk .npy members like CloudBuoyWriter's."""
+    each output with `units` and the fill value `fillVal` for invalid triangles.  netCDF4 or an .npz with the same
+    variables, `<name>_units` and an f4 `FillValue` (see _OutFile)."""
 
     def __init__(self, cf_out, ntime, tri, pIDs, tunits=tunits_default, fillVal=FillValue, corigin=None):
         from .deform import DEFORM_NAMES, DEFORM_UNITS
-        print('\n *** [DeformationWriter]: About to generate file: ' + cf_out + ' ...')
         tri = np.asarray(tri).reshape(-1, 3)
         self.ntime, self.nT = int(ntime), tri.shape[0]
         self.names = DEFORM_NAMES
         ids = np.asarray(pIDs).astype('i8')[tri] if self.nT else np.zeros((0, 3), 'i8')
-        nc = None
-        if not str(cf_out).endswith(".npz"):
-            try:
-                import netCDF4 as nc
-            except ImportError:
-                cf_out += ".npz"
-                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
-        self.cf_out, self._nc = cf_out, nc
-        if nc is None:
-            import tempfile
-            self._tmp = tempfile.mkdtemp(prefix=".deform_", dir=os.path.dirname(os.path.abspath(cf_out)) or ".")
-            mm = lambda n, dt, shp: np.lib.format.open_memmap(os.path.join(self._tmp, n + ".npy"), mode='w+', dtype=dt, shape=shp)
-            self._v = {n: mm(n, 'f4', (self.ntime, self.nT)) for n in self.names}
-            self._v['time_start'] = mm('time_start', 'i4', (self.ntime,))
-            self._v['time_end'] = mm('time_end', 'i4', (self.ntime,))
-            mm('vertices', 'i4', (self.nT, 3))[:] = tri
-            mm('id_vertices', 'i8', (self.nT, 3))[:] = ids
-            for n in self.names:
-                np.save(os.path.join(self._tmp, n + "_units.npy"), np.array(DEFORM_UNITS[n]))
-            np.save(os.path.join(self._tmp, "FillValue.npy"), np.float32(fillVal))
-        else:
-            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
-            f.createDimension('time', None)
-            f.createDimension('triangle', self.nT)
-            f.createDimension('vertex', 3)
-            self._v = {}
-            for n in ('time_start', 'time_end'):
-                self._v[n] = f.createVariable(n, 'i4', ('time',)); self._v[n].units = tunits
-            f.createVariable('vertices', 'i4', ('triangle', 'vertex'))[:] = tri
-            vid = f.createVariable('id_vertices', 'i8', ('triangle', 'vertex')); vid.units = 'ID of buoy'
-            vid[:] = ids
-            zkw = dict(zlib=True, complevel=9)
-            for n in self.names:
-                self._v[n] = f.createVariable(n, 'f4', ('time', 'triangle'), fill_value=fillVal, **zkw)
-                self._v[n].units = DEFORM_UNITS[n]
-            if corigin:
-                f.Origin = corigin
-            f.About = 'Sea-ice deformation rates of buoy triangles'
-            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+        super().__init__(cf_out, 'DeformationWriter', dict(time=self.ntime, triangle=self.nT, vertex=3),
+                         'Sea-ice deformation rates of buoy triangles', corigin, fill=np.float32(fillVal))
+        for n in ('time_start', 'time_end'):
+            self.var(n, 'i4', ('time',), units=tunits)
+        self.var('vertices', 'i4', ('triangle', 'vertex'), data=tri)
+        self.var('id_vertices', 'i8', ('triangle', 'vertex'), units='ID of buoy', data=ids)
+        for n in self.names:
+            self.var(n, 'f4', ('time', 'triangle'), units=DEFORM_UNITS[n], fill=True, zlib=True)
 
     def write(self, jw, time_start, time_end, out):
         """Window jw: out = dict of (nT,) arrays over the six outputs."""
@@ -299,29 +294,8 @@ class DeformationWriter:
         for n in self.names:
             self._v[n][jw, :] = np.asarray(out[n], dtype=np.float32)
 
-    def close(self):
-        if self._nc is not None:
-            self._f.close()
-        else:
-            import shutil
-            import zipfile
-            for v in self._v.values():
-                v.flush()
-            self._v = {}
-            with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
-                for fn in sorted(os.listdir(self._tmp)):
-                    z.write(os.path.join(self._tmp, fn), arcname=fn)
-            shutil.rmtree(self._tmp, ignore_errors=True)
-        print('      ===> ' + self.cf_out + ' saved!')
 
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-
-class DeformationScalingWriter:
+class DeformationScalingWriter(_OutFile):
     """Window-by-window writer of the per-scale statistics of coarse-grained deformation (sitrack_b200.deform_scales,
     TrackEngine.track's `deform` with `scales`).  Dimensions time (windows), scale, bin, bin_edge; variables
       time_start, time_end (time) i4                       first and last date of each window [tunits]
@@ -332,53 +306,29 @@ class DeformationScalingWriter:
                                                            fillVal where n = 0
       hist_total, hist_divergence, hist_shear (time,scale,bin) i8   counts of eps_tot, |div|, shear per bin,
                                                            bin k = [edge k-1, edge k), underflow and overflow first/last
-    with `units` on every variable.  netCDF4 when available and the name does not end in .npz; otherwise an .npz
-    with the same variables, plus `<name>_units` (0-d strings) and `FillValue` members for the attributes."""
+    with `units` on every variable.  netCDF4 or an .npz with the same variables, `<name>_units` and an f8
+    `FillValue` (see _OutFile)."""
 
     MEANS = (("L_eff", "sum_L_eff", "km"), ("eps_tot", "sum_eps_tot", "day-1"), ("eps_tot2", "sum_eps_tot2", "day-2"),
              ("eps_tot3", "sum_eps_tot3", "day-3"))
     HISTS = ("hist_total", "hist_divergence", "hist_shear")
 
     def __init__(self, cf_out, ntime, scale_km, bin_edges, tunits=tunits_default, fillVal=FillValue, corigin=None):
-        print('\n *** [DeformationScalingWriter]: About to generate file: ' + cf_out + ' ...')
         scale_km, bin_edges = np.asarray(scale_km, 'f8'), np.asarray(bin_edges, 'f8')
         self.ntime, self.ns, self.nbin = int(ntime), scale_km.size, bin_edges.size + 1
-        self.fill = fillVal
-        units = dict(time_start=tunits, time_end=tunits, scale_km='km', bin_edges='day-1', n='1',
-                     **{n: u for n, _, u in self.MEANS}, **{h: '1' for h in self.HISTS})
-        nc = None
-        if not str(cf_out).endswith(".npz"):
-            try:
-                import netCDF4 as nc
-            except ImportError:
-                cf_out += ".npz"
-                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
-        self.cf_out, self._nc = cf_out, nc
-        shapes = dict(time_start=('i4', ('time',)), time_end=('i4', ('time',)), n=('i8', ('time', 'scale')),
-                      **{n: ('f8', ('time', 'scale')) for n, _, _ in self.MEANS},
-                      **{h: ('i8', ('time', 'scale', 'bin')) for h in self.HISTS})
-        if nc is None:
-            size = dict(time=self.ntime, scale=self.ns, bin=self.nbin)
-            self._v = {n: np.zeros([size[d] for d in dims], dt) for n, (dt, dims) in shapes.items()}
-            self._v['scale_km'], self._v['bin_edges'] = scale_km, bin_edges
-            self._units = units
-        else:
-            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
-            f.createDimension('time', None)
-            f.createDimension('scale', self.ns)
-            f.createDimension('bin', self.nbin)
-            f.createDimension('bin_edge', bin_edges.size)
-            self._v = {}
-            for n, (dt, dims) in shapes.items():
-                self._v[n] = f.createVariable(n, dt, dims, **(dict(fill_value=fillVal) if dt == 'f8' else {}))
-            f.createVariable('scale_km', 'f8', ('scale',))[:] = scale_km
-            f.createVariable('bin_edges', 'f8', ('bin_edge',))[:] = bin_edges
-            for n, u in units.items():
-                f.variables[n].units = u
-            if corigin:
-                f.Origin = corigin
-            f.About = 'Per-scale statistics of sea-ice deformation coarse-grained over material boxes of buoy triangles'
-            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+        super().__init__(cf_out, 'DeformationScalingWriter',
+                         dict(time=self.ntime, scale=self.ns, bin=self.nbin, bin_edge=bin_edges.size),
+                         'Per-scale statistics of sea-ice deformation coarse-grained over material boxes of buoy '
+                         'triangles', corigin, fill=np.float64(fillVal))
+        for n in ('time_start', 'time_end'):
+            self.var(n, 'i4', ('time',), units=tunits)
+        self.var('n', 'i8', ('time', 'scale'), units='1')
+        for n, _, u in self.MEANS:
+            self.var(n, 'f8', ('time', 'scale'), units=u, fill=True)
+        for h in self.HISTS:
+            self.var(h, 'i8', ('time', 'scale', 'bin'), units='1')
+        self.var('scale_km', 'f8', ('scale',), units='km', data=scale_km)
+        self.var('bin_edges', 'f8', ('bin_edge',), units='day-1', data=bin_edges)
 
     def write(self, jw, time_start, time_end, stats):
         """Window jw: stats = the dict of sitrack_b200.CoarseGrainedRates / track(deform=dict(scales=...))."""
@@ -392,22 +342,8 @@ class DeformationScalingWriter:
         for h in self.HISTS:
             self._v[h][jw, :, :] = np.asarray(stats[h], 'i8')
 
-    def close(self):
-        if self._nc is not None:
-            self._f.close()
-        else:
-            extra = {n + '_units': np.array(u) for n, u in self._units.items()}
-            np.savez(self.cf_out, FillValue=np.float64(self.fill), **self._v, **extra)
-        print('      ===> ' + self.cf_out + ' saved!')
 
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-
-class DeformationGridWriter:
+class DeformationGridWriter(_OutFile):
     """Window-by-window writer of deformation coarse-grained over the cells of a fixed Eulerian grid
     (sitrack_b200.deform_grid, TrackEngine.track's `deform` with `grid`).  Dimensions time (windows) and, per level
     s = 1..levels, y<s>, x<s>; variables
@@ -416,73 +352,34 @@ class DeformationGridWriter:
       <name>_<s> (time,y<s>,x<s>) f4                       divergence, shear, vorticity, total [day-1], L_eff [km],
                                                            y_ctr, x_ctr [km]; fillVal where the cell does not count
     with `units` on every variable and the attributes L_km (cell side per level), cover and origin ([y, x] km of the
-    grid's corner); corigin, if given, as `Origin`.  netCDF4 when available and the name does not end in .npz;
-    otherwise an .npz with the same variables, plus `L_km`, `cover`, `origin`, `<name>_units` (0-d strings) and
-    `FillValue` members, assembled from on-disk .npy members like DeformationWriter's."""
+    grid's corner); corigin, if given, as `Origin`.  netCDF4 or an .npz with the same variables, `L_km`, `cover`,
+    `origin`, `<name>_units` and an f4 `FillValue` (see _OutFile)."""
 
     UNITS = dict(divergence='day-1', shear='day-1', vorticity='day-1', total='day-1', L_eff='km', y_ctr='km',
                  x_ctr='km')
 
     def __init__(self, cf_out, ntime, G, tunits=tunits_default, fillVal=FillValue, corigin=None):
         from .deform_scales import BOX_NAMES
-        print('\n *** [DeformationGridWriter]: About to generate file: ' + cf_out + ' ...')
         self.ntime, self.levels, self.names = int(ntime), G.levels, BOX_NAMES
-        self.var = lambda n, s: '%s_%d' % (n, s + 1)
-        nc = None
-        if not str(cf_out).endswith(".npz"):
-            try:
-                import netCDF4 as nc
-            except ImportError:
-                cf_out += ".npz"
-                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
-        self.cf_out, self._nc = cf_out, nc
-        units = dict(time_start=tunits, time_end=tunits)
-        for s in range(G.levels):
-            units['y%d' % (s + 1)] = units['x%d' % (s + 1)] = 'km'
-            units.update({self.var(n, s): self.UNITS[n] for n in self.names})
-        if nc is None:
-            import tempfile
-            self._tmp = tempfile.mkdtemp(prefix=".deform_grid_", dir=os.path.dirname(os.path.abspath(cf_out)) or ".")
-            mm = lambda n, dt, shp: np.lib.format.open_memmap(os.path.join(self._tmp, n + ".npy"), mode='w+', dtype=dt, shape=shp)
-            self._v = {'time_start': mm('time_start', 'i4', (self.ntime,)), 'time_end': mm('time_end', 'i4', (self.ntime,))}
-            for s, (nj, ni) in enumerate(G.shapes):
-                y, x = G.centres(s)
-                np.save(os.path.join(self._tmp, 'y%d.npy' % (s + 1)), y)
-                np.save(os.path.join(self._tmp, 'x%d.npy' % (s + 1)), x)
-                for n in self.names:
-                    self._v[self.var(n, s)] = mm(self.var(n, s), 'f4', (self.ntime, nj, ni))
-            for n, u in units.items():
-                np.save(os.path.join(self._tmp, n + "_units.npy"), np.array(u))
-            np.save(os.path.join(self._tmp, "L_km.npy"), np.asarray(G.L_km, 'f8'))
-            np.save(os.path.join(self._tmp, "cover.npy"), np.float64(G.cover))
-            np.save(os.path.join(self._tmp, "origin.npy"), np.asarray(G.origin, 'f8'))
-            np.save(os.path.join(self._tmp, "FillValue.npy"), np.float32(fillVal))
-        else:
-            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
-            f.createDimension('time', None)
-            self._v = {}
-            for n in ('time_start', 'time_end'):
-                self._v[n] = f.createVariable(n, 'i4', ('time',))
-            zkw = dict(zlib=True, complevel=9)
-            for s, (nj, ni) in enumerate(G.shapes):
-                dy, dx = 'y%d' % (s + 1), 'x%d' % (s + 1)
-                f.createDimension(dy, nj)
-                f.createDimension(dx, ni)
-                y, x = G.centres(s)
-                self._v[dy] = f.createVariable(dy, 'f8', (dy,)); self._v[dy][:] = y
-                self._v[dx] = f.createVariable(dx, 'f8', (dx,)); self._v[dx][:] = x
-                for n in self.names:
-                    self._v[self.var(n, s)] = f.createVariable(self.var(n, s), 'f4', ('time', dy, dx),
-                                                               fill_value=fillVal, **zkw)
-            for n, u in units.items():
-                self._v[n].units = u
-            f.L_km = np.asarray(G.L_km, 'f8')
-            f.cover = float(G.cover)
-            f.origin = np.asarray(G.origin, 'f8')
-            if corigin:
-                f.Origin = corigin
-            f.About = 'Sea-ice deformation of buoy triangles coarse-grained over the cells of a fixed grid'
-            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+        dims = dict(time=self.ntime)
+        for s, (nj, ni) in enumerate(G.shapes):
+            dims['y%d' % (s + 1)], dims['x%d' % (s + 1)] = nj, ni
+        super().__init__(cf_out, 'DeformationGridWriter', dims,
+                         'Sea-ice deformation of buoy triangles coarse-grained over the cells of a fixed grid', corigin,
+                         fill=np.float32(fillVal), L_km=np.asarray(G.L_km, 'f8'), cover=float(G.cover),
+                         origin=np.asarray(G.origin, 'f8'))
+        for n in ('time_start', 'time_end'):
+            self.var(n, 'i4', ('time',), units=tunits)
+        for s, (y, x) in enumerate(G.centres(s) for s in range(G.levels)):
+            dy, dx = 'y%d' % (s + 1), 'x%d' % (s + 1)
+            self.var(dy, 'f8', (dy,), units='km', data=y)
+            self.var(dx, 'f8', (dx,), units='km', data=x)
+            for n in self.names:
+                self.var(self.field(n, s), 'f4', ('time', dy, dx), units=self.UNITS[n], fill=True, zlib=True)
+
+    @staticmethod
+    def field(n, s):
+        return '%s_%d' % (n, s + 1)
 
     def write(self, jw, time_start, time_end, fields):
         """Window jw: fields = per level dicts of (nj_s, ni_s) planes (sitrack_b200.GriddedRates, track's grid_sink)."""
@@ -490,31 +387,10 @@ class DeformationGridWriter:
         self._v['time_end'][jw] = time_end
         for s in range(self.levels):
             for n in self.names:
-                self._v[self.var(n, s)][jw, :, :] = np.asarray(fields[s][n], dtype=np.float32)
-
-    def close(self):
-        if self._nc is not None:
-            self._f.close()
-        else:
-            import shutil
-            import zipfile
-            for v in self._v.values():
-                v.flush()
-            self._v = {}
-            with zipfile.ZipFile(self.cf_out, 'w', zipfile.ZIP_DEFLATED, allowZip64=True) as z:
-                for fn in sorted(os.listdir(self._tmp)):
-                    z.write(os.path.join(self._tmp, fn), arcname=fn)
-            shutil.rmtree(self._tmp, ignore_errors=True)
-        print('      ===> ' + self.cf_out + ' saved!')
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
+                self._v[self.field(n, s)][jw, :, :] = np.asarray(fields[s][n], dtype=np.float32)
 
 
-class DispersionWriter:
+class DispersionWriter(_OutFile):
     """Window-by-window writer of the per-lag, per-class statistics of pair dispersion (sitrack_b200.dispersion,
     TrackEngine.track's `dispersion`).  Dimensions time (windows), lag, class, bin, class_edge, bin_edge; variables
       time_start, time_end (time) i4                 first and last date of each window [tunits]
@@ -525,50 +401,27 @@ class DispersionWriter:
       sum_r0, sum_dr, sum_dr2, sum_dD2 (time,lag,class) f8   sums of r0 [km], dr [km], dr^2 [km2], dD2 [km2]
       hist_stretch (time,lag,class,bin) i8           counts of the stretch rate |dr| / (r0 tau) per bin
     with `units` on every variable.  Sums, not means, so that windows add up to ensembles; no variable has a fill value
-    (a lag not reached yet has zero counts and sums).  netCDF4 when available and the name does not end in .npz;
-    otherwise an .npz with the same variables, plus `<name>_units` (0-d strings)."""
+    (a lag not reached yet has zero counts and sums).  netCDF4 or an .npz with the same variables and `<name>_units`
+    (see _OutFile)."""
 
     SUMS = (("sum_r0", "km"), ("sum_dr", "km"), ("sum_dr2", "km2"), ("sum_dD2", "km2"))
 
     def __init__(self, cf_out, ntime, lag_days, r_edges, bin_edges, tunits=tunits_default, corigin=None):
-        print('\n *** [DispersionWriter]: About to generate file: ' + cf_out + ' ...')
         lag_days, r_edges, bin_edges = (np.asarray(a, 'f8') for a in (lag_days, r_edges, bin_edges))
         self.ntime = int(ntime)
-        units = dict(time_start=tunits, time_end=tunits, lag_days='day', r_edges='km', bin_edges='day-1', n='1',
-                     hist_stretch='1', **{n: u for n, u in self.SUMS})
-        size = dict(time=self.ntime, lag=lag_days.size, **{'class': r_edges.size + 1}, bin=bin_edges.size + 1)
-        shapes = dict(time_start=('i4', ('time',)), time_end=('i4', ('time',)), n=('i8', ('time', 'lag', 'class')),
-                      **{n: ('f8', ('time', 'lag', 'class')) for n, _ in self.SUMS},
-                      hist_stretch=('i8', ('time', 'lag', 'class', 'bin')))
-        nc = None
-        if not str(cf_out).endswith(".npz"):
-            try:
-                import netCDF4 as nc
-            except ImportError:
-                cf_out += ".npz"
-                print('      (netCDF4 not available: writing ' + cf_out + ' with the same variables)')
-        self.cf_out, self._nc = cf_out, nc
-        if nc is None:
-            self._v = {n: np.zeros([size[d] for d in dims], dt) for n, (dt, dims) in shapes.items()}
-            self._v.update(lag_days=lag_days, r_edges=r_edges, bin_edges=bin_edges)
-            self._units = units
-        else:
-            f = self._f = nc.Dataset(cf_out, 'w', format='NETCDF4')
-            f.createDimension('time', None)
-            for d in ('lag', 'class', 'bin'):
-                f.createDimension(d, size[d])
-            f.createDimension('class_edge', r_edges.size)
-            f.createDimension('bin_edge', bin_edges.size)
-            self._v = {n: f.createVariable(n, dt, dims) for n, (dt, dims) in shapes.items()}
-            for n, d, a in (('lag_days', 'lag', lag_days), ('r_edges', 'class_edge', r_edges),
-                            ('bin_edges', 'bin_edge', bin_edges)):
-                f.createVariable(n, 'f8', (d,))[:] = a
-            for n, u in units.items():
-                f.variables[n].units = u
-            if corigin:
-                f.Origin = corigin
-            f.About = 'Two-particle dispersion of buoy pairs over time lags, by initial separation'
-            f.Author = 'Generated with `%s` of `sitrack` (L. Brodeau, 2023)' % os.path.basename(sys.argv[0])
+        super().__init__(cf_out, 'DispersionWriter',
+                         dict(time=self.ntime, lag=lag_days.size, **{'class': r_edges.size + 1}, bin=bin_edges.size + 1,
+                              class_edge=r_edges.size, bin_edge=bin_edges.size),
+                         'Two-particle dispersion of buoy pairs over time lags, by initial separation', corigin)
+        for n in ('time_start', 'time_end'):
+            self.var(n, 'i4', ('time',), units=tunits)
+        self.var('n', 'i8', ('time', 'lag', 'class'), units='1')
+        for n, u in self.SUMS:
+            self.var(n, 'f8', ('time', 'lag', 'class'), units=u)
+        self.var('hist_stretch', 'i8', ('time', 'lag', 'class', 'bin'), units='1')
+        self.var('lag_days', 'f8', ('lag',), units='day', data=lag_days)
+        self.var('r_edges', 'f8', ('class_edge',), units='km', data=r_edges)
+        self.var('bin_edges', 'f8', ('bin_edge',), units='day-1', data=bin_edges)
 
     def write(self, jw, time_start, time_end, stats):
         """Window jw: stats = the dict of sitrack_b200.PairDispersion / track(dispersion=...)."""
@@ -578,20 +431,6 @@ class DispersionWriter:
         for n, _ in self.SUMS:
             self._v[n][jw] = np.asarray(stats[n], 'f8')
         self._v['hist_stretch'][jw] = np.asarray(stats['hist_stretch'], 'i8')
-
-    def close(self):
-        if self._nc is not None:
-            self._f.close()
-        else:
-            extra = {n + '_units': np.array(u) for n, u in self._units.items()}
-            np.savez(self.cf_out, **self._v, **extra)
-        print('      ===> ' + self.cf_out + ' saved!')
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
 
 def ncSaveCloudBuoys(cf_out, ptime, pIDs, pY, pX, pLat, pLon, mask=[], xtime=[],
