@@ -357,6 +357,38 @@ int  st_dispersion_dev(st_ctx *ctx, int64_t nQ, const int32_t *pairs_dev, const 
                        void *scratch_dev, int64_t scratch_bytes, int64_t *hist_dev, double *sums_dev,
                        double *per_pair_dev, void *stream);
 
+/* ---- finite-size Lyapunov exponents of pairs: exit times between separation thresholds ----
+ * nQ (1..2^31-1) pairs pairs_dev (nQ,2) int32 of buoy indices (8-byte aligned; not range-checked on the device), one
+ * sample t (1..65535) per call: the row yx_dev, m_dev (DESIGN.md section 14, oracle/fsle_ref.py).  Per pair and sample,
+ * in f8 and in this order: dy = y_a - y_b, dx = x_a - x_b, r = sqrt(dy*dy + dx*dx); the sample is valid when both
+ * masks are != 0 and r is finite; b = searchsorted(deltas, r, side="right") over nthr (2..64) positive, strictly
+ * increasing f8 thresholds deltas_dev, so a tie reaches the threshold.
+ * state_dev (nQ,2) int32 {level, anchor} in the caller's pair order (8-byte aligned): level -1 not started, -2 ended,
+ * 0..nthr thresholds reached; anchor the sample at which that level was first reached, -1 when unknown.  Update:
+ *   not started, valid:    level = b, anchor = -1, n_start[b] += 1 (a pair starting above delta_j is not timed there);
+ *   not started, invalid:  nothing;
+ *   started, invalid:      level = -2; n_censored[level-1] += 1 when anchor >= 0 and level < nthr;
+ *   started, valid, b > level: record tau = t - anchor for transition level-1 when level >= 1 and anchor >= 0, record
+ *                          tau = 0 for transitions level .. b-2, then anchor = t, level = b (levels never go down).
+ * Recording tau for transition j (0..nthr-2) adds 1 to hist_tau[j][searchsorted(tau_edges, tau, side="right")], tau to
+ * sum_tau[j] and tau^2 to sum_tau2[j]; tau_edges_dev holds ntau_edges (1..512) ascending f8 edges in samples.
+ * With yx_start_dev, m_start_dev (both or neither) the call first resets every pair to not started and evaluates the
+ * start row as sample t-1, then the row as sample t: the first call of a run, with row 0 as the start row.
+ * stats_dev, one int64 buffer (8-byte aligned), zeroed and then written with the events of this call, in this order:
+ *   n_start (nthr+1) | hist_tau (nthr-1, ntau_edges+1) | sum_tau (nthr-1) | sum_tau2 (nthr-1) | n_censored (nthr-1),
+ * nthr+1 + (nthr-1)(ntau_edges+4) words.  Integer atomics only: exact, independent of the launch grid, the device and
+ * the buoy storage order.  Sample indices up to 65535 keep sum_tau2 below 2^63.  The shared-memory counters need
+ * 8 (nthr + ntau_edges + 2 (nthr-1)) + 4 (nthr+1 + (nthr-1)(ntau_edges+2)) B of the 227 KB a block may have.
+ * st_fsle_state_bytes checks (nQ, nthr, ntau_edges) on the host before any CUDA call and gives the size of state_dev.
+ * ASYNC st_fsle_dev: no host synchronisation, no allocation; refuses nQ < 1, t outside 1..65535, shapes past the
+ * limits, a NULL pointer, rows not 16-byte aligned and pairs, state, edges or stats not 8-byte aligned, and writes
+ * nothing then.                                                                                                       */
+int  st_fsle_state_bytes(int64_t nQ, int nthr, int ntau_edges, int64_t *bytes);
+int  st_fsle_dev(st_ctx *ctx, int64_t nQ, const int32_t *pairs_dev, int32_t *state_dev, const double *yx_dev,
+                 const int8_t *m_dev, int t, const double *yx_start_dev, const int8_t *m_start_dev, int nthr,
+                 const double *deltas_dev, int ntau_edges, const double *tau_edges_dev, int64_t *stats_dev,
+                 void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

@@ -76,6 +76,15 @@ def __argument_parsing__():
     parser.add_argument('--dispersion-pairs', type=float, nargs=3, default=None, metavar=('N', 'R_MIN_KM', 'R_MAX_KM'),
                         help='with --dispersion: N random draws of pairs at log-uniform separations in [R_MIN_KM, R_MAX_KM] '
                              '(default: one draw per buoy, 10 to 1000 km)')
+    parser.add_argument('--fsle', type=float, default=None, metavar='HOURS',
+                        help='also compute finite-size Lyapunov exponents of buoy pairs on the GPU: the pairs are sampled '
+                             'every HOURS (a multiple of the model time step) and the exit times between separation '
+                             'thresholds of every window go into ./nc/..._fsle_...')
+    parser.add_argument('--fsle-deltas', type=float, nargs=3, default=None, metavar=('D0_KM', 'ALPHA', 'K'),
+                        help='with --fsle: K (2..64) thresholds D0_KM * ALPHA^j (default: 2 km, sqrt(2), 19)')
+    parser.add_argument('--fsle-pairs', type=float, nargs=3, default=None, metavar=('N', 'R_MIN_KM', 'R_MAX_KM'),
+                        help='with --fsle: N random draws of pairs at log-uniform separations in [R_MIN_KM, R_MAX_KM] '
+                             '(default: one draw per buoy, 10 to 1000 km)')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -202,6 +211,44 @@ def dispersion_args(disp, pairs, world):
     return n, int(lags), None if N is None else int(N), r_min, r_max
 
 
+def fsle_args(hours, deltas, pairs, world):
+    """--fsle HOURS [--fsle-deltas D0_KM ALPHA K] [--fsle-pairs N R_MIN_KM R_MAX_KM] -> (records per sample, the
+    thresholds, N or None, r_min, r_max) or None; ERROR and exit when HOURS is not a positive multiple of the model
+    time step, K is not an integer in 2..64, D0 <= 0, ALPHA <= 1 or the thresholds are not finite and increasing,
+    N < 1, R_MIN <= 0 or R_MAX <= R_MIN, an option comes without --fsle, or under torchrun (pairs would cross the
+    ranks' shards)."""
+    if hours is None:
+        for flag, v in (('--fsle-deltas', deltas), ('--fsle-pairs', pairs)):
+            if v is not None:
+                print('ERROR: %s needs --fsle HOURS' % flag)
+                exit(0)
+        return None
+    if world > 1:
+        print('ERROR: --fsle is not available with several processes (WORLD_SIZE > 1): pairs would cross ranks')
+        exit(0)
+    n = window_records('--fsle', hours)
+    D0, alpha, K = (2.0, np.sqrt(2.0), 19) if deltas is None else deltas
+    if K != int(K) or not 2 <= K <= sit.MAX_THRESHOLDS:
+        print('ERROR: --fsle-deltas K must be an integer in 2..%d, got %g' % (sit.MAX_THRESHOLDS, K))
+        exit(0)
+    if not (D0 > 0 and alpha > 1):
+        print('ERROR: --fsle-deltas needs D0_KM > 0 and ALPHA > 1, got %g %g' % (D0, alpha))
+        exit(0)
+    with np.errstate(over='ignore'):
+        d = np.float64(D0) * np.float64(alpha) ** np.arange(int(K), dtype=np.float64)
+    if not (np.isfinite(d).all() and (np.diff(d) > 0).all()):
+        print('ERROR: --fsle-deltas: the thresholds D0_KM * ALPHA^j are not finite and increasing (last %g)' % d[-1])
+        exit(0)
+    N, r_min, r_max = (None, 10.0, 1000.0) if pairs is None else pairs
+    if N is not None and (N != int(N) or N < 1):
+        print('ERROR: --fsle-pairs N must be a positive integer, got %g' % N)
+        exit(0)
+    if not (r_min > 0 and r_max > r_min and np.isfinite(r_max)):
+        print('ERROR: --fsle-pairs needs 0 < R_MIN_KM < R_MAX_KM, got %g %g' % (r_min, r_max))
+        exit(0)
+    return n, d, None if N is None else int(N), r_min, r_max
+
+
 def deform_grid_over(Yt, Xt, L0, levels):
     """The EulerianGrid of side L0 covering the T-points (Yt, Xt) km: origin floor(min / L0) L0 and
     floor((max - origin) / L0) + 1 cells per axis; ERROR and exit when that is more than 2^20 cells a side."""
@@ -225,6 +272,7 @@ def main():
     dscales = deform_levels_args('--deform-scales', args.deform_scales, args.deform)
     dgrid = deform_levels_args('--deform-grid', args.deform_grid, args.deform)
     dspa = dispersion_args(args.dispersion, args.dispersion_pairs, world)
+    fsla = fsle_args(args.fsle, args.fsle_deltas, args.fsle_pairs, world)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
@@ -253,6 +301,10 @@ def main():
         exit(0)
     if dspa and Nt // dspa[0] < 1:
         print('ERROR: --dispersion window (%d records) is longer than the run (%d records)!' % (dspa[0], Nt))
+        exit(0)
+    if fsla and not 1 <= Nt // fsla[0] <= sit.MAX_SAMPLES:
+        print('ERROR: --fsle gives %d windows of %d records over the run (%d records): need 1..%d'
+              % (Nt // fsla[0], fsla[0], Nt, sit.MAX_SAMPLES))
         exit(0)
     for cd in ['seed', 'nc', 'npz']:
         makedirs(cd, exist_ok=True)
@@ -425,6 +477,22 @@ def main():
                                        sit.DEFAULT_BIN_EDGES, corigin=corgn)
         dispersion = dict(pairs=pairs, every=nd, lags=lags, sink=window_sink(nd, pwriter))
         small = False
+    fsle = None
+    if fsla:
+        # pairs over the seeds in the order the files use (after --sort), drawn as for --dispersion; the pairs' state
+        # stays on the GPU and only statistics leave it
+        nf, deltas, npair, r_min, r_max = fsla
+        nwf = Nt // nf
+        pairs = sit.SeparationPairs(xPosC0, r_min, r_max, nP if npair is None else npair, seed=0)
+        if pairs.shape[0] == 0:
+            print('ERROR: --fsle: no pair of distinct buoys was drawn!')
+            exit(0)
+        print(' *** --fsle: %d pairs at %g to %g km, %d thresholds from %g to %g km, %d samples of %d records'
+              % (pairs.shape[0], r_min, r_max, deltas.size, deltas[0], deltas[-1], nwf, nf))
+        fwriter = sit.FsleWriter(nc_name('fsle', vTime[0], vTime[nwf * nf]), nwf, deltas, sit.DEFAULT_TAU_EDGES,
+                                 nf * rdt / 86400., corigin=corgn)
+        fsle = dict(pairs=pairs, every=nf, deltas=deltas, sink=window_sink(nf, fwriter))
+        small = False
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
         res = eng.track(record, Nt, kstrt=kstrt, pos0=xPosC0, posG0=xPosG0, rec_first=z1st, chunk=nchunk,
@@ -434,7 +502,7 @@ def main():
     else:
         res = eng.track(record, Nt, kstrt=kstrt, rec_first=cut(z1st), sink=sink,
                         row_dtype='f8' if physics else args.rows, physics=physics, deform=deform,
-                        dispersion=dispersion)
+                        dispersion=dispersion, fsle=fsle)
     eng.close()
     for w in writers:
         w.close()

@@ -1317,6 +1317,45 @@ int st_dispersion_dev(st_ctx* c, int64_t nQ, const int32_t* pairs, const double*
     return ST_OK;
 }
 
+// ---- finite-size Lyapunov exponents of pairs (st_fsle.cu) ---------------------------------------
+static const char* fsle_check(int64_t nQ, int nthr, int ntau_edges)
+{
+    if (nQ < 1 || nQ > INT32_MAX) return "nQ must be in 1..2^31-1";
+    if (nthr < 2 || nthr > FS_MAX_THRESHOLDS) return "nthr must be in 2..64";
+    if (ntau_edges < 1 || ntau_edges > FS_MAX_TAU_EDGES) return "ntau_edges must be in 1..512";
+    if (fsle_smem(nthr, ntau_edges) > DS_MAX_SMEM)
+        return "thresholds x exit-time bins need more than the 227 KB of shared memory a block may have";
+    return nullptr;
+}
+
+int st_fsle_state_bytes(int64_t nQ, int nthr, int ntau_edges, int64_t* bytes)
+{
+    if (!bytes) return fail(nullptr, ST_EINVAL, "st_fsle_state_bytes: NULL argument");
+    if (const char* why = fsle_check(nQ, nthr, ntau_edges))
+        return fail(nullptr, ST_EINVAL, std::string("st_fsle_state_bytes: ") + why);
+    *bytes = nQ * 2 * (int64_t)sizeof(int32_t);
+    return ST_OK;
+}
+
+int st_fsle_dev(st_ctx* c, int64_t nQ, const int32_t* pairs, int32_t* state, const double* yx, const int8_t* m, int t,
+                const double* yx0, const int8_t* m0, int nthr, const double* deltas, int ntau_edges,
+                const double* tau_edges, int64_t* stats, void* stream)
+{
+    if (const char* why = fsle_check(nQ, nthr, ntau_edges))
+        return fail(c, ST_EINVAL, std::string("st_fsle_dev: ") + why);
+    if (t < 1 || t > FS_MAX_SAMPLES) return fail(c, ST_EINVAL, "st_fsle_dev: t must be in 1..65535");
+    if (!pairs || !state || !yx || !m || !deltas || !tau_edges || !stats)
+        return fail(c, ST_EINVAL, "st_fsle_dev: NULL argument");
+    if (!yx0 != !m0) return fail(c, ST_EINVAL, "st_fsle_dev: give both yx_start and m_start, or neither");
+    if ((uintptr_t)yx % 16 || (uintptr_t)yx0 % 16 || (uintptr_t)pairs % 8 || (uintptr_t)state % 8 ||
+        (uintptr_t)deltas % 8 || (uintptr_t)tau_edges % 8 || (uintptr_t)stats % 8)
+        return fail(c, ST_EINVAL, "st_fsle_dev: rows must be 16-byte aligned, pairs, state, edges and stats 8-byte");
+    if (c) CU(c, cudaSetDevice(c->device));
+    CU(c, launch_fsle(nQ, pairs, state, (const pt*)yx, m, t, (const pt*)yx0, m0, nthr, deltas, ntau_edges, tau_edges,
+                      stats, (cudaStream_t)stream));
+    return ST_OK;
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

@@ -263,4 +263,19 @@ cudaError_t launch_dispersion(const DispOrigins& og, long long nQ, const int32_t
                               const double* bins, void* scratch, int64_t* hist, double* sums, double* out,
                               cudaStream_t st);
 
+// ---- finite-size Lyapunov exponents of pairs: exit times between separation thresholds (st_fsle.cu) ----
+constexpr int FS_MAX_THRESHOLDS = 64;
+constexpr int FS_MAX_TAU_EDGES = 512;
+constexpr int FS_MAX_SAMPLES = 65535;
+
+// Dynamic shared memory of k_fsle and the length (int64 words) of its statistics buffer for K thresholds and ntau
+// exit-time edges.
+size_t fsle_smem(int K, int ntau);
+long long fsle_stats_len(int K, int ntau);
+// pairs (nQ,2) buoy indices; state (nQ,2) int32 {level, anchor}; sample t of the row yx, m; with yx0 != NULL the
+// state is reset and the row yx0, m0 is sample t-1 first.  stats (fsle_stats_len) int64 is zeroed and then written.
+cudaError_t launch_fsle(long long nQ, const int32_t* pairs, int32_t* state, const pt* yx, const int8_t* m, int t,
+                        const pt* yx0, const int8_t* m0, int K, const double* deltas, int ntau,
+                        const double* tau_edges, int64_t* stats, cudaStream_t st);
+
 }  // namespace st

@@ -427,7 +427,8 @@ class TrackEngine:
 
     # -- the record loop ---------------------------------------------------------------
     def track(self, records, nrec, kstrt=0, pos0=None, posG0=None, rec_first=None, want_latlon=True,
-              sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None, dispersion=None):
+              sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None, dispersion=None,
+              fsle=None):
         """The record loop (si3_part_tracker.py:361-496), pipelined.
 
         records: callable k -> (u, v, ic) arrays (Nj,Ni) for record index k (0-based
@@ -463,6 +464,13 @@ class TrackEngine:
         row (w+1)*n is reduced on the device for lags l = 1 .. min(m, w+1) in one launch, and only the statistics reach
         the host: sink(w, stats), or with sink None the list of them under "dispersion".  They do not depend on the
         order the buoys are stored in.  Not with the chunked season path either.
+        fsle = dict(pairs=(nQ,2) buoy pairs in the caller's order, every=n, deltas=None, tau_edges=None, sink=callable or
+        None), independent of `deform` and `dispersion` and combinable with both: the rows s*n are the samples of the
+        pairs' finite-size Lyapunov exponents (sitrack_b200.fsle); each pair's first-passage state {level, anchor}
+        stays on the device for the whole run and is updated at every sample, and only each window's integer
+        statistics (the events of sample w+1, window 0 also those of row 0) reach the host: sink(w, stats), or with
+        sink None the list of them under "fsle".  They do not depend on the order the buoys are stored in.  At most
+        MAX_SAMPLES windows; not with the chunked season path either.
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -479,13 +487,13 @@ class TrackEngine:
                 raise ValueError("physics modes write f8 rows")
             chunk = None
         if chunk and chunk > 1 and sink is None:
-            if deform is not None or dispersion is not None:
+            if deform is not None or dispersion is not None or fsle is not None:
                 raise ValueError("deform and dispersion run on the streaming record loop: not with chunk > 1 and sink=None")
             return self._track_chunked(get, nrec, kstrt, pos0, posG0, rec_first, want_latlon, int(chunk), rdt)
-        wrows = None if deform is None and dispersion is None else _WindowRows(self, torch, rec_first, kstrt,
-                                                                               row_f4=rdt == torch.float32)
-        runs = [run(self, torch, dev, spec, wrows, nrec)
-                for run, spec in ((_deform_run, deform), (_dispersion_run, dispersion)) if spec is not None]
+        specs = ((_deform_run, deform), (_dispersion_run, dispersion), (_fsle_run, fsle))
+        wrows = None if all(spec is None for _, spec in specs) else _WindowRows(self, torch, rec_first, kstrt,
+                                                                                row_f4=rdt == torch.float32)
+        runs = [run(self, torch, dev, spec, wrows, nrec) for run, spec in specs if spec is not None]
         self.record_slots(2)
         stg = [self.staging(0), self.staging(1)]
         s_in, s_cmp, s_out = (torch.cuda.Stream(dev) for _ in range(3))
@@ -669,6 +677,20 @@ def _dispersion_run(eng, torch, dev, spec, rows, nrec):
     plan = P._Plan(torch, dev, rows.slots(pairs), lags, spec.get("r_edges"), spec.get("bins"),
                    dt_days=every * eng.rdt / 86400.0)
     return _WindowRun(eng, torch, dev, rows, every, nrec, lags, [("dispersion", spec.get("sink"), plan)])
+
+
+def _fsle_run(eng, torch, dev, spec, rows, nrec):
+    """track(fsle=...): one sample per window on the one-slot ring (row 0 is read in window 0 only).  Pairs are mapped
+    to engine slots without reordering them, so the state stays in the caller's pair order."""
+    from . import fsle as F
+    from .dispersion import check_pairs
+    every = _window_every(spec, "fsle")
+    if nrec // every > F.MAX_SAMPLES:
+        raise ValueError("fsle: %d windows, more than the %d samples a run may have" % (nrec // every, F.MAX_SAMPLES))
+    pairs = check_pairs(spec["pairs"], eng.nP)
+    plan = F._Plan(torch, dev, rows.slots(pairs), spec.get("deltas"), spec.get("tau_edges"),
+                   sample_days=every * eng.rdt / 86400.0)
+    return _WindowRun(eng, torch, dev, rows, every, nrec, 1, [("fsle", spec.get("sink"), plan)])
 
 
 class _WindowRun:

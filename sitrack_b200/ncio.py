@@ -25,7 +25,7 @@ from .util import epoch2clock as e2c
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
            "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter",
-           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter"]
+           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter", "FsleWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -431,6 +431,48 @@ class DispersionWriter(_OutFile):
         for n, _ in self.SUMS:
             self._v[n][jw] = np.asarray(stats[n], 'f8')
         self._v['hist_stretch'][jw] = np.asarray(stats['hist_stretch'], 'i8')
+
+
+class FsleWriter(_OutFile):
+    """Window-by-window writer of the exit-time statistics of finite-size Lyapunov exponents (sitrack_b200.fsle,
+    TrackEngine.track's `fsle`).  Dimensions time (windows), threshold (K), transition (K-1), tau_bin, plus level
+    (K+1) and tau_edge; variables
+      time_start, time_end (time) i4                 first and last date of each window [tunits]
+      delta_km (threshold) f8                        separation thresholds [km]
+      tau_edges (tau_edge) f8                        exit-time histogram edges [sample]
+      n_start (time,level) i8                        pairs that started with that many thresholds reached
+      n, n_censored (time,transition) i8             exit times recorded; timed transitions cut by a pair's end
+      sum_tau, sum_tau2 (time,transition) i8         sums of the exit times [sample] and of their squares [sample2]
+      hist_tau (time,transition,tau_bin) i8          counts of the exit times per bin
+    with `units` on every variable and the global attribute sample_days (the length of one sample in days).  Sums,
+    not means, so that windows add up to the run; no variable has a fill value.  netCDF4 or an .npz with the same
+    variables, `<name>_units` and `sample_days` (see _OutFile)."""
+
+    COUNTS = (("n", "1"), ("sum_tau", "sample"), ("sum_tau2", "sample2"), ("n_censored", "1"))
+
+    def __init__(self, cf_out, ntime, deltas_km, tau_edges, sample_days, tunits=tunits_default, corigin=None):
+        deltas_km, tau_edges = np.asarray(deltas_km, 'f8'), np.asarray(tau_edges, 'f8')
+        self.ntime, K = int(ntime), deltas_km.size
+        super().__init__(cf_out, 'FsleWriter',
+                         dict(time=self.ntime, threshold=K, transition=K - 1, tau_bin=tau_edges.size + 1,
+                              level=K + 1, tau_edge=tau_edges.size),
+                         'Finite-size Lyapunov exponents of buoy pairs: exit times between separation thresholds',
+                         corigin, sample_days=float(sample_days))
+        for n in ('time_start', 'time_end'):
+            self.var(n, 'i4', ('time',), units=tunits)
+        self.var('n_start', 'i8', ('time', 'level'), units='1')
+        for n, u in self.COUNTS:
+            self.var(n, 'i8', ('time', 'transition'), units=u)
+        self.var('hist_tau', 'i8', ('time', 'transition', 'tau_bin'), units='1')
+        self.var('delta_km', 'f8', ('threshold',), units='km', data=deltas_km)
+        self.var('tau_edges', 'f8', ('tau_edge',), units='sample', data=tau_edges)
+
+    def write(self, jw, time_start, time_end, stats):
+        """Window jw: stats = a window's dict of sitrack_b200.FiniteSizeLyapunov / track(fsle=...)."""
+        self._v['time_start'][jw] = time_start
+        self._v['time_end'][jw] = time_end
+        for n in ('n_start', 'hist_tau') + tuple(n for n, _ in self.COUNTS):
+            self._v[n][jw] = np.asarray(stats[n], 'i8')
 
 
 def ncSaveCloudBuoys(cf_out, ptime, pIDs, pY, pX, pLat, pLon, mask=[], xtime=[],
