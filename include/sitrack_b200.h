@@ -389,6 +389,28 @@ int  st_fsle_dev(st_ctx *ctx, int64_t nQ, const int32_t *pairs_dev, int32_t *sta
                  const double *deltas_dev, int ntau_edges, const double *tau_edges_dev, int64_t *stats_dev,
                  void *stream);
 
+/* ---- SI3 T-cell fields sampled along the buoy trajectories (DESIGN.md section 15, oracle/sample_ref.py) ----
+ * One row of the trajectory: for every buoy p of the context, its host cell (jT, iT) from the cell state (bit 31
+ * stripped), its f8 position from yx_dev (nP,2) [y,x] km, or from the state when yx_dev is NULL (the chained row after
+ * a chained step), and its row mask mask_dev (nP,) int8.  fields_dev holds nF (1..16) planes of Nj*Ni f4 (the T-cell
+ * values of one record, e.g. siconc as plane 2 of a record slot), plane f at fields_dev + f * plane_stride floats
+ * (plane_stride >= Nj*Ni).  out_dev (nF, nP) f4 gets, per field and buoy, in the caller's buoy order of the state:
+ *   FillValue (-9999) when the mask is 0 or the cell lies outside 1..Nj-2 x 1..Ni-2;
+ *   interp 0 (cell):      F[jT,iT], an exact copy;
+ *   interp 1 (bilinear):  the T-quad on P's side of the grid lines T[jT-1,iT]->T[jT+1,iT] and T[jT,iT-1]->T[jT,iT+1]
+ *     (f8 orientation tests, a point on a line goes to the higher index), the closed-form inverse bilinear (xi, eta)
+ *     of P in it (k2 == 0: the parallelogram's linear root), clamped to [0,1]; corners SW, SE, NE, NW weighted
+ *     (1-xi)(1-eta), xi(1-eta), xi eta, (1-xi) eta, those with tmask 0 or a non-finite value dropped and the rest
+ *     renormalised in that order; no weight kept: the cell value.  f8 without FMA, rounded once to f4.
+ *     tyx_dev (Nj*Ni,2) f8 [y,x] km are the T-points of a right-handed grid (i eastward, j northward: the quad pick
+ *     reads "west" and "south" from the signs of the two orientation tests); the stencil reaches T[jT+-1, iT+-1].
+ *   a non-finite result: FillValue.
+ * ASYNC st_sample_dev: no host synchronisation, no allocation; refuses (before any CUDA call, writing nothing) a NULL
+ * context, fields, mask or out, tyx NULL with interp 1, nF outside 1..16, plane_stride < Nj*Ni, interp other than 0
+ * or 1, fields or out not 4-byte aligned and yx or tyx not 16-byte aligned.                                        */
+int  st_sample_dev(st_ctx *ctx, int nF, const float *fields_dev, int64_t plane_stride, const double *yx_dev,
+                   const int8_t *mask_dev, int interp, const double *tyx_dev, float *out_dev, void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

@@ -85,6 +85,14 @@ def __argument_parsing__():
     parser.add_argument('--fsle-pairs', type=float, nargs=3, default=None, metavar=('N', 'R_MIN_KM', 'R_MAX_KM'),
                         help='with --fsle: N random draws of pairs at log-uniform separations in [R_MIN_KM, R_MAX_KM] '
                              '(default: one draw per buoy, 10 to 1000 km)')
+    parser.add_argument('--sample', nargs='+', default=None, metavar='VAR',
+                        help='also sample these SI3 T-cell variables (e.g. siconc sithic) along the trajectories on the GPU '
+                             'and write them, per sampled row and buoy, into ./nc/..._sampled_...')
+    parser.add_argument('--sample-every', type=float, default=None, metavar='HOURS',
+                        help='with --sample: sample every HOURS (a multiple of the model time step; default: every record)')
+    parser.add_argument('--sample-interp', default=None, choices=['cell', 'bilinear'],
+                        help='with --sample: the host cell\'s value (cell, default) or the bilinear interpolation '
+                             'between the four T-points around the buoy (bilinear)')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -249,6 +257,42 @@ def fsle_args(hours, deltas, pairs, world):
     return n, d, None if N is None else int(N), r_min, r_max
 
 
+def sample_args(names, hours, interp):
+    """--sample VAR [VAR ...] [--sample-every HOURS] [--sample-interp cell|bilinear] -> (names, records between sampled
+    rows, interp) or None; ERROR and exit when HOURS is not a positive multiple of the model time step, a variable is
+    named twice or more than MAX_SAMPLE_FIELDS are named, or an option comes without --sample."""
+    if names is None:
+        for flag, v in (('--sample-every', hours), ('--sample-interp', interp)):
+            if v is not None:
+                print('ERROR: %s needs --sample VAR [VAR ...]' % flag)
+                exit(0)
+        return None
+    if len(set(names)) != len(names) or len(names) > sit.MAX_SAMPLE_FIELDS:
+        print('ERROR: --sample needs 1..%d distinct variables, got %s' % (sit.MAX_SAMPLE_FIELDS, ' '.join(names)))
+        exit(0)
+    n = 1 if hours is None else window_records('--sample-every', hours)
+    return list(names), n, interp or 'cell'
+
+
+def check_sample_vars(ds, names):
+    """ERROR and exit when a --sample variable is missing from the SI3 file or is not a (t,y,x) variable of the shape
+    of u_ice; -> {name: units} of those that have units."""
+    ref = tuple(ds.variables['u_ice'].shape)
+    units = {}
+    for n in names:
+        if n not in ds.variables:
+            print('ERROR: --sample: variable %s is not in the SI3 file' % n)
+            exit(0)
+        v = ds.variables[n]
+        if tuple(v.shape) != ref:
+            print('ERROR: --sample: %s has shape %s, not the (t,y,x) shape %s of u_ice' % (n, tuple(v.shape), ref))
+            exit(0)
+        u = getattr(v, 'units', None)
+        if u is not None:
+            units[n] = str(u)
+    return units
+
+
 def deform_grid_over(Yt, Xt, L0, levels):
     """The EulerianGrid of side L0 covering the T-points (Yt, Xt) km: origin floor(min / L0) L0 and
     floor((max - origin) / L0) + 1 cells per axis; ERROR and exit when that is more than 2^20 cells a side."""
@@ -273,6 +317,7 @@ def main():
     dgrid = deform_levels_args('--deform-grid', args.deform_grid, args.deform)
     dspa = dispersion_args(args.dispersion, args.dispersion_pairs, world)
     fsla = fsle_args(args.fsle, args.fsle_deltas, args.fsle_pairs, world)
+    smpa = sample_args(args.sample, args.sample_every, args.sample_interp)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
@@ -306,6 +351,10 @@ def main():
         print('ERROR: --fsle gives %d windows of %d records over the run (%d records): need 1..%d'
               % (Nt // fsla[0], fsla[0], Nt, sit.MAX_SAMPLES))
         exit(0)
+    sunits = {}
+    if smpa:
+        with sit.open_dataset(cf_uv) as ds0:
+            sunits = check_sample_vars(ds0, smpa[0])
     for cd in ['seed', 'nc', 'npz']:
         makedirs(cd, exist_ok=True)
 
@@ -409,14 +458,20 @@ def main():
         sel = np.flatnonzero(kN == k + 1)
         z2XY[1, sel], z2GC[1, sel], zMSK[1, sel] = yx[sel], ll[sel], m[sel]
 
+    sample_stash = []                                             # torchrun: samples that go with the next row
+
     def sink(k, yx, ll, m):
         if world == 1:
             keep_row(k, yx, ll, m)
         else:                                                     # one small gather per record, rank 0 writes
             parts = [None] * world if rank == 0 else None
-            dist.gather_object((yx.copy(), ll.copy(), m.copy()), parts, dst=0)
+            dist.gather_object((yx.copy(), ll.copy(), m.copy(), sample_stash[:]), parts, dst=0)
+            sample_stash.clear()
             if rank == 0:
                 keep_row(k, *[np.concatenate([p[i] for p in parts]) for i in range(3)])
+                for i, (js, vals) in enumerate(parts[0][3]):      # every rank samples the same rows
+                    smwriter.write(js, vTime[js * smpa[1]],
+                                  {n: np.concatenate([p[3][i][1][n] for p in parts]) for n in vals})
 
     eng = sit.TrackEngine(xYf, xXf, xYu, xXu, xYv, xXv, tmask=imaskt, uv_strategy=args.uvstrategy, rdt=rdt,
                           rmin_conc=sit.rmin_conc, device=sit.config.device)
@@ -493,6 +548,27 @@ def main():
                                  nf * rdt / 86400., corigin=corgn)
         fsle = dict(pairs=pairs, every=nf, deltas=deltas, sink=window_sink(nf, fwriter))
         small = False
+    sample = None
+    if smpa:
+        # the SI3 fields along the trajectories, in the order the files use (after --sort); under torchrun each rank
+        # samples its block and the samples travel to rank 0 with the rows
+        snames, ns, sinterp = smpa
+        nws = Nt // ns
+        print(' *** --sample: %s (%s) at %d rows, every %d records' % (' '.join(snames), sinterp, nws + 1, ns))
+        smwriter = None
+        if rank == 0:
+            smwriter = sit.SampleWriter(nc_name('sampled', vTime[0], vTime[Nt]), nws + 1, IDs, snames, sinterp, ns,
+                                        units=sunits, corigin=corgn)
+            writers.append(smwriter)
+
+        def sample_sink(js, vals):
+            if world == 1:
+                smwriter.write(js, vTime[js * ns], vals)
+            else:
+                sample_stash.append((js, vals))
+        sample = dict(names=snames, every=ns, interp=sinterp, tyx=(xYt, xXt), sink=sample_sink,
+                      get=lambda k, n: ds.variables[n][k + kstrt, :, :])
+        small = False                                             # rows are sampled inside the streaming record loop
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
         res = eng.track(record, Nt, kstrt=kstrt, pos0=xPosC0, posG0=xPosG0, rec_first=z1st, chunk=nchunk,
@@ -502,7 +578,7 @@ def main():
     else:
         res = eng.track(record, Nt, kstrt=kstrt, rec_first=cut(z1st), sink=sink,
                         row_dtype='f8' if physics else args.rows, physics=physics, deform=deform,
-                        dispersion=dispersion, fsle=fsle)
+                        dispersion=dispersion, fsle=fsle, sample=sample)
     eng.close()
     for w in writers:
         w.close()

@@ -13,6 +13,7 @@ from .deform_scales import *  # noqa: F401,F403
 from .deform_grid import *    # noqa: F401,F403
 from .dispersion import *     # noqa: F401,F403
 from .fsle import *           # noqa: F401,F403
+from .sample import *         # noqa: F401,F403
 from . import config                      # noqa: F401
 from .engine import TrackEngine          # noqa: F401
 from ._lib import SitrackCudaError       # noqa: F401

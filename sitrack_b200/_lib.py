@@ -88,6 +88,7 @@ SIGNATURES = {
                                   c_i64, vp, vp, vp, vp]),
     "st_fsle_state_bytes": (c_int, [c_i64, c_int, c_int, vp]),
     "st_fsle_dev": (c_int, [vp, c_i64, vp, vp, vp, vp, c_int, vp, vp, c_int, vp, c_int, vp, vp, vp]),
+    "st_sample_dev": (c_int, [vp, c_int, vp, c_i64, vp, vp, c_int, vp, vp, vp]),
     "st_xy2latlon": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_latlon2xy": (c_int, [c_int, c_i64, vp, vp, c_dbl, c_dbl]),
     "st_xy2latlon_dev": (c_int, [c_i64, vp, vp, c_dbl, c_dbl, vp]),

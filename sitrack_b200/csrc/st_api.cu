@@ -1356,6 +1356,28 @@ int st_fsle_dev(st_ctx* c, int64_t nQ, const int32_t* pairs, int32_t* state, con
     return ST_OK;
 }
 
+// ---- SI3 T-cell fields sampled along the buoy trajectories (st_sample.cu) ---------------------------------
+int st_sample_dev(st_ctx* c, int nF, const float* fields, int64_t plane_stride, const double* yx, const int8_t* mask,
+                  int interp, const double* tyx, float* out, void* stream)
+{
+    if (!c) return fail(nullptr, ST_EINVAL, "st_sample_dev: ctx is NULL");
+    if (nF < 1 || nF > SP_MAX_FIELDS) return fail(c, ST_EINVAL, "st_sample_dev: nF must be in 1..16");
+    if (interp != 0 && interp != 1) return fail(c, ST_EINVAL, "st_sample_dev: interp must be 0 (cell) or 1 (bilinear)");
+    if (!fields || !mask || !out || (interp == 1 && !tyx))
+        return fail(c, ST_EINVAL, "st_sample_dev: NULL argument (fields, mask, out; tyx with interp 1)");
+    if (plane_stride < (int64_t)c->Nj * c->Ni)
+        return fail(c, ST_EINVAL, "st_sample_dev: plane_stride must be at least Nj*Ni");
+    if ((uintptr_t)fields % 4 || (uintptr_t)out % 4 || (uintptr_t)yx % 16 || (uintptr_t)tyx % 16)
+        return fail(c, ST_EINVAL, "st_sample_dev: fields and out must be 4-byte aligned, yx and tyx 16-byte");
+    if (c->nP == 0) return ST_OK;
+    CU(c, cudaSetDevice(c->device));
+    // NULL: the state's positions, which after chained steps live in the last chained row
+    const pt* pos = yx ? (const pt*)yx : (c->pos_src ? c->pos_src : c->pos);
+    CU(c, launch_sample(c->nP, c->Nj, c->Ni, c->cell, mask, pos, (const pt*)tyx, c->tmask, fields, plane_stride, nF,
+                        interp, out, (cudaStream_t)stream));
+    return ST_OK;
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

@@ -278,4 +278,13 @@ cudaError_t launch_fsle(long long nQ, const int32_t* pairs, int32_t* state, cons
                         const pt* yx0, const int8_t* m0, int K, const double* deltas, int ntau,
                         const double* tau_edges, int64_t* stats, cudaStream_t st);
 
+// ---- SI3 T-cell fields sampled along the buoy trajectories (st_sample.cu) ----
+constexpr int SP_MAX_FIELDS = 16;
+
+// cell (nP) the state's cells, mask (nP) the row mask, yx (nP) the f8 positions (bilinear only); T (Nj*Ni) the T-points
+// [y,x] km (bilinear only); F nF planes of Nj*Ni f4 at `stride` floats; interp 0 cell, 1 bilinear; out (nF, nP) f4.
+cudaError_t launch_sample(long long nP, int Nj, int Ni, const int2* cell, const int8_t* mask, const pt* yx,
+                          const pt* T, const int8_t* tmask, const float* F, long long stride, int nF, int interp,
+                          float* out, cudaStream_t st);
+
 }  // namespace st

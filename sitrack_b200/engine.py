@@ -428,7 +428,7 @@ class TrackEngine:
     # -- the record loop ---------------------------------------------------------------
     def track(self, records, nrec, kstrt=0, pos0=None, posG0=None, rec_first=None, want_latlon=True,
               sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None, dispersion=None,
-              fsle=None):
+              fsle=None, sample=None):
         """The record loop (si3_part_tracker.py:361-496), pipelined.
 
         records: callable k -> (u, v, ic) arrays (Nj,Ni) for record index k (0-based
@@ -471,6 +471,13 @@ class TrackEngine:
         statistics (the events of sample w+1, window 0 also those of row 0) reach the host: sink(w, stats), or with
         sink None the list of them under "fsle".  They do not depend on the order the buoys are stored in.  At most
         MAX_SAMPLES windows; not with the chunked season path either.
+        sample = dict(names=[...], get=callable(k, name) -> (Nj,Ni) or None, every=n, interp="cell"|"bilinear",
+        tyx=(Yt, Xt), sink=callable or None), combinable with all of the above: SI3 T-cell fields sampled along the
+        trajectories on the device (sitrack_b200.sample, DESIGN.md section 15) at rows 0, n, 2n, ...; row 0 with record
+        0, row k+1 with record k.  "siconc" is read from the record itself; every other name with get(k, name), only
+        for the records that are sampled.  sink(s, {name: (nP,) f4}) in the caller's buoy order (called before the
+        row sink of the same row), or with sink None {name: (nsample, nP) f4} under "sample".  "bilinear" needs tyx,
+        the T-points [km].  Not with the chunked season path either.
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -487,13 +494,18 @@ class TrackEngine:
                 raise ValueError("physics modes write f8 rows")
             chunk = None
         if chunk and chunk > 1 and sink is None:
-            if deform is not None or dispersion is not None or fsle is not None:
-                raise ValueError("deform and dispersion run on the streaming record loop: not with chunk > 1 and sink=None")
+            if deform is not None or dispersion is not None or fsle is not None or sample is not None:
+                raise ValueError("deform, dispersion, fsle and sample run on the streaming record loop: not with chunk > 1 "
+                                 "and sink=None")
             return self._track_chunked(get, nrec, kstrt, pos0, posG0, rec_first, want_latlon, int(chunk), rdt)
         specs = ((_deform_run, deform), (_dispersion_run, dispersion), (_fsle_run, fsle))
-        wrows = None if all(spec is None for _, spec in specs) else _WindowRows(self, torch, rec_first, kstrt,
-                                                                                row_f4=rdt == torch.float32)
+        wrows = None if all(spec is None for _, spec in specs) and sample is None else \
+            _WindowRows(self, torch, rec_first, kstrt, row_f4=rdt == torch.float32)
         runs = [run(self, torch, dev, spec, wrows, nrec) for run, spec in specs if spec is not None]
+        smp = None
+        if sample is not None:
+            from .sample import _SampleRun
+            smp = _SampleRun(self, torch, dev, sample, wrows, nrec)
         self.record_slots(2)
         stg = [self.staging(0), self.staging(1)]
         s_in, s_cmp, s_out = (torch.cuda.Stream(dev) for _ in range(3))
@@ -520,6 +532,8 @@ class TrackEngine:
 
         def drain(k):
             ev_out[k].synchronize()
+            if smp is not None:
+                smp.deliver(k + 1, ev_out)                 # the samples of rows <= k+1 before the row sink of k
             if not keep:
                 y, l, m = rows(k)
                 sink(k, y.numpy(), None if l is None else l.numpy(), m.numpy())
@@ -534,6 +548,8 @@ class TrackEngine:
                 ev_in[k - 2].synchronize()                 # staging slot b has left the host
             u, v, ic = get(k)
             stg[b][0], stg[b][1], stg[b][2] = u, v, ic     # f4 copy into pinned memory
+            if smp is not None:
+                smp.load(k)                                # the extra fields of a sampled record, same reader
         pool = ThreadPoolExecutor(1)
         nxt = pool.submit(load, 0) if nrec > 0 else None
         # f8 rows: the row of record k is the position input of record k+1 (st_set_row_chain); both row buffers
@@ -550,19 +566,30 @@ class TrackEngine:
                 if k >= 2:
                     s_in.wait_event(ev_step[k - 2])            # device slot b no longer read
                 self.submit_record(b, s_in)
+                if smp is not None:
+                    smp.upload(k, s_in)
                 ev_in[k] = torch.cuda.Event(); ev_in[k].record(s_in)
                 s_cmp.wait_event(ev_in[k])
                 if k >= NB:
                     s_cmp.wait_event(ev_out[k - NB])           # device out buffer b drained
+                if smp is not None and k == 0:
+                    smp.row(0, 0, b, None, smp.m0, s_cmp)     # row 0: the state handed to set_buoys, record 0
                 if physics:
                     self.step_ext(b, k + kstrt, physics.get("scheme", 1), physics.get("interp", 0),
                                   physics.get("max_hops", 1), d_yx[b], d_ll[b], d_mk[b], d_na[k:k + 1], s_cmp)
                 else:
                     self.step(b, k + kstrt, d_yx[b], d_ll[b], d_mk[b], d_na[k:k + 1], s_cmp)
+                if smp is not None and (k + 1) % smp.every == 0:
+                    # row k+1 with record k, before ev_step[k]: the slot is not overwritten before this has read it
+                    smp.row(k + 1, k, b, d_yx[b] if rdt == torch.float64 else None, d_mk[b], s_cmp)
                 ev_step[k] = torch.cuda.Event(); ev_step[k].record(s_cmp)
                 s_out.wait_event(ev_step[k])
                 if not keep and k >= NB:
                     drain(k - NB)                              # pinned row buffer b is free again
+                elif keep and smp is not None and k >= NB:
+                    smp.deliver(k - 1, ev_out)                 # as drain(k - NB) would: the sample ring is free again
+                if smp is not None:
+                    smp.copy_out(k, s_out)
                 y, l, m = rows(k)
                 with torch.cuda.stream(s_out):
                     y.copy_(d_yx[b], non_blocking=True)
@@ -579,6 +606,8 @@ class TrackEngine:
                     drain(k)
             for run in runs:
                 run.finish()
+            if smp is not None:
+                smp.deliver(nrec, ev_out)
         finally:
             if chain:
                 self.set_row_chain(False)                  # state up to date again (synchronises)
@@ -588,6 +617,8 @@ class TrackEngine:
         extra = {}
         for run in runs:
             extra.update(run.collected)
+        if smp is not None:
+            extra.update(smp.collected)
         if not keep:
             return dict(n_alive=n_alive, **extra)
         posC, posG, mask = posC.numpy(), posG.numpy(), mask.numpy()

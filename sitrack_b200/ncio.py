@@ -25,7 +25,7 @@ from .util import epoch2clock as e2c
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
            "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter",
-           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter", "FsleWriter"]
+           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter", "FsleWriter", "SampleWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -473,6 +473,35 @@ class FsleWriter(_OutFile):
         self._v['time_end'][jw] = time_end
         for n in ('n_start', 'hist_tau') + tuple(n for n, _ in self.COUNTS):
             self._v[n][jw] = np.asarray(stats[n], 'i8')
+
+
+class SampleWriter(_OutFile):
+    """Row-by-row writer of SI3 fields sampled along the trajectories (sitrack_b200.sample, TrackEngine.track's
+    `sample`).  Dimensions time (sampled rows), buoy (the tracking file's buoy axis); variables
+      time (time) i4                 the date of each sampled row [tunits]
+      id_buoy (buoy) i8              IDs of the buoys
+      <name> (time,buoy) f4          one per field, named like the SI3 variable, with its units when given and the
+                                     fill value fillVal where the buoy is masked or the value is missing
+    and the global attributes interp ("cell" or "bilinear") and every (records between sampled rows).  netCDF4 or an
+    .npz with the same variables, `<name>_units`, `interp`, `every` and an f4 `FillValue` (see _OutFile)."""
+
+    def __init__(self, cf_out, ntime, pIDs, names, interp, every, units=None, tunits=tunits_default,
+                 fillVal=FillValue, corigin=None):
+        self.ntime, self.nP, self.names = int(ntime), int(np.shape(pIDs)[0]), list(names)
+        units = units or {}
+        super().__init__(cf_out, 'SampleWriter', dict(time=self.ntime, buoy=self.nP),
+                         'SI3 fields sampled along Lagrangian sea-ice trajectories', corigin, fill=np.float32(fillVal),
+                         interp=str(interp), every=int(every))
+        self.var('time', 'i4', ('time',), units=tunits)
+        self.var('id_buoy', 'i8', ('buoy',), units='ID of buoy', data=np.asarray(pIDs))
+        for n in self.names:
+            self.var(n, 'f4', ('time', 'buoy'), units=units.get(n), fill=True, zlib=True)
+
+    def write(self, js, time, values):
+        """Sampled row js: values = {name: (nP,) f4} (sitrack_b200.SampleFields / track(sample=...))."""
+        self._v['time'][js] = time
+        for n in self.names:
+            self._v[n][js, :] = np.asarray(values[n], 'f4')
 
 
 def ncSaveCloudBuoys(cf_out, ptime, pIDs, pY, pX, pLat, pLon, mask=[], xtime=[],
