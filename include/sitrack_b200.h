@@ -411,6 +411,41 @@ int  st_fsle_dev(st_ctx *ctx, int64_t nQ, const int32_t *pairs_dev, int32_t *sta
 int  st_sample_dev(st_ctx *ctx, int nF, const float *fields_dev, int64_t plane_stride, const double *yx_dev,
                    const int8_t *mask_dev, int interp, const double *tyx_dev, float *out_dev, void *stream);
 
+/* ---- buoy transits between regions: connectivity (DESIGN.md section 16, oracle/connect_ref.py) ----
+ * labels_dev (Nj*Ni) u8 on the T-grid: 0 = in no region, 1..nreg (1..31) regions; a label above nreg counts as 0.
+ * One sample t (0..65535) per call.  Per buoy p of nP (1..2^31-1): its cell (jT, iT) from cell_dev (nP,2) int32 (bit
+ * 31 of the jT word, the discontinued flag, stripped), or from the context's cell state when cell_dev is NULL (nP, Nj
+ * and Ni must then match the context; with cell_dev given ctx may be NULL); its row mask mask_dev (nP) int8.  The
+ * sample is valid when the mask is != 0 and 1 <= jT <= Nj-2, 1 <= iT <= Ni-2; cur = labels[jT*Ni + iT] then.
+ * state_dev (nP,2) int32, 8-byte aligned, in the storage order of the cells: word 0 `visited` (bit r-1 = region r
+ * entered), word 1 start | src << 16 | prev << 21 | status << 26 (start sample 16 bits; src, prev regions; status 0
+ * not started, 1 started, 2 ended).  t = 0 first resets every buoy to not started.  Update at sample t:
+ *   not started, valid:   start: src = prev = cur, start = t, visited = bit(cur) when cur >= 1; n_start[src] += 1 and,
+ *                         when t > 0, count[src][cur] += 1;
+ *   not started, invalid: nothing;
+ *   started, invalid:     ended for good: n_end[src] += 1;
+ *   started, valid:       trans[prev][cur] += 1, count[src][cur] += 1; when cur >= 1 and bit(cur) is not in visited,
+ *                         a first arrival, tau = t - start >= 1: n_arrive[src][cur-1] += 1, sum_tau += tau,
+ *                         sum_tau2 += tau^2, hist_tau[src][cur-1][searchsorted(tau_edges, tau, side="right")] += 1,
+ *                         and the bit is set; then prev = cur.
+ * tau_edges_dev holds ntau_edges (1..512) ascending f8 edges in samples (8-byte aligned).  stats_dev, one int64
+ * buffer (8-byte aligned) that the call ADDS to (the caller zeroes it), with R = nreg, R1 = R+1, NB = ntau_edges+1:
+ *   n_start (R1) | n_end (R1) | count (R1,R1) | trans (R1,R1) | n_arrive (R1,R) | sum_tau (R1,R) | sum_tau2 (R1,R) |
+ *   hist_tau (R1,R,NB),  2 R1 + 2 R1^2 + 3 R1 R + R1 R NB words.
+ * Integer atomics only: exact, independent of the launch grid, the device, the buoy storage order and of how the
+ * buoys are split between calls.  The shared-memory counters need 16 R1 R + 4 (2 R1 + 2 R1^2 + R1 R) B of the 48 KB a
+ * block has without opting in (28 288 B at R = 31).  With t <= 65535 and nP < 2^31, sum_tau2 stays below 2^63 over a run.
+ * st_connect_state_bytes checks (nP, nreg, ntau_edges) on the host before any CUDA call and gives the size of
+ * state_dev, 8 nP.
+ * ASYNC st_connect_dev: no host synchronisation, no allocation; refuses (before any CUDA call, writing nothing) t
+ * outside 0..65535, shapes past the limits (and Nj, Ni < 1 or Nj*Ni >= 2^31), a NULL labels, mask, state, tau_edges or
+ * stats, a NULL cell_dev without a context or with nP, Nj, Ni other than the context's, and cell, state, tau_edges or
+ * stats not 8-byte aligned.                                                                                           */
+int  st_connect_state_bytes(int64_t nP, int nreg, int ntau_edges, int64_t *bytes);
+int  st_connect_dev(st_ctx *ctx, int Nj, int Ni, const uint8_t *labels_dev, int nreg, int64_t nP,
+                    const int32_t *cell_dev, const int8_t *mask_dev, int t, int32_t *state_dev, int ntau_edges,
+                    const double *tau_edges_dev, int64_t *stats_dev, void *stream);
+
 /* ---- projections (util.py:394-472 via cartopy NorthPolarStereo) ------------------------ */
 int  st_xy2latlon(int device, int64_t n, const double *yx, double *latlon, double lat_ts, double lon0);
 int  st_latlon2xy(int device, int64_t n, const double *latlon, double *yx, double lat_ts, double lon0);

@@ -93,6 +93,14 @@ def __argument_parsing__():
     parser.add_argument('--sample-interp', default=None, choices=['cell', 'bilinear'],
                         help='with --sample: the host cell\'s value (cell, default) or the bilinear interpolation '
                              'between the four T-points around the buoy (bilinear)')
+    parser.add_argument('--connect', type=float, default=None, metavar='HOURS',
+                        help='also count buoy transits between the regions of a label map on the GPU: the buoys\' host '
+                             'cells are sampled every HOURS (a multiple of the model time step) and per-window starts, '
+                             'ends, transitions, source-to-region counts and first-arrival times go into '
+                             './nc/..._connectivity_...')
+    parser.add_argument('--connect-regions', nargs=2, default=None, metavar=('FILE', 'VAR'),
+                        help='with --connect: the (y,x) variable VAR of FILE (netCDF or .npz) labels the T-cells with '
+                             'regions 1..31 (0 or a masked value: in no region)')
     args = parser.parse_args()
     print('')
     print(' *** SI3 file to get ice velocities from => ', args.fsi3)
@@ -293,6 +301,41 @@ def check_sample_vars(ds, names):
     return units
 
 
+def connect_args(hours, regions):
+    """--connect HOURS --connect-regions FILE VAR -> (records per sample, FILE, VAR) or None; ERROR and exit when one
+    comes without the other or HOURS is not a positive multiple of the model time step."""
+    if (hours is None) != (regions is None):
+        print('ERROR: --connect HOURS and --connect-regions FILE VAR go together')
+        exit(0)
+    if hours is None:
+        return None
+    return window_records('--connect', hours), regions[0], regions[1]
+
+
+def connect_labels(fn, var, shape):
+    """The region map VAR of FILE as (u8 labels, R); ERROR and exit when the file or the variable is missing, the
+    variable is not `shape` (the model's (y,x)) after taking its first (y,x) plane, or its labels are refused."""
+    from sitrack_b200.ncio import _plane
+    if not path.exists(fn):
+        print('ERROR: --connect-regions: file %s not found' % fn)
+        exit(0)
+    with sit.open_dataset(fn) as ds:
+        if var not in ds.variables:
+            print('ERROR: --connect-regions: variable %s is not in %s' % (var, fn))
+            exit(0)
+        v = ds.variables[var]
+        a = _plane(v) if len(v.shape) >= 2 else None
+    if a is None or a.shape != tuple(shape):
+        print('ERROR: --connect-regions: %s has shape %s, not the (y,x) shape %s of the model grid'
+              % (var, tuple(v.shape), tuple(shape)))
+        exit(0)
+    try:
+        return sit.connect.check_labels(a, *shape)
+    except ValueError as e:
+        print('ERROR: --connect-regions: %s' % e)
+        exit(0)
+
+
 def deform_grid_over(Yt, Xt, L0, levels):
     """The EulerianGrid of side L0 covering the T-points (Yt, Xt) km: origin floor(min / L0) L0 and
     floor((max - origin) / L0) + 1 cells per axis; ERROR and exit when that is more than 2^20 cells a side."""
@@ -318,6 +361,7 @@ def main():
     dspa = dispersion_args(args.dispersion, args.dispersion_pairs, world)
     fsla = fsle_args(args.fsle, args.fsle_deltas, args.fsle_pairs, world)
     smpa = sample_args(args.sample, args.sample_every, args.sample_interp)
+    cona = connect_args(args.connect, args.connect_regions)
     dist = None
     if world > 1:
         import torch.distributed as dist                      # host-side plumbing only: gloo over CPU arrays
@@ -351,6 +395,14 @@ def main():
         print('ERROR: --fsle gives %d windows of %d records over the run (%d records): need 1..%d'
               % (Nt // fsla[0], fsla[0], Nt, sit.MAX_SAMPLES))
         exit(0)
+    if cona and not 1 <= Nt // cona[0] <= sit.MAX_SAMPLES:
+        print('ERROR: --connect gives %d windows of %d records over the run (%d records): need 1..%d'
+              % (Nt // cona[0], cona[0], Nt, sit.MAX_SAMPLES))
+        exit(0)
+    labels = None
+    if cona:
+        with sit.open_dataset(cf_uv) as ds0:
+            labels, nreg = connect_labels(cona[1], cona[2], ds0.variables['u_ice'].shape[-2:])
     sunits = {}
     if smpa:
         with sit.open_dataset(cf_uv) as ds0:
@@ -569,6 +621,30 @@ def main():
         sample = dict(names=snames, every=ns, interp=sinterp, tyx=(xYt, xXt), sink=sample_sink,
                       get=lambda k, n: ds.variables[n][k + kstrt, :, :])
         small = False                                             # rows are sampled inside the streaming record loop
+    connect = None
+    if cona:
+        # the buoys' host cells against the region map, on the GPU; under torchrun each rank counts its block and the
+        # windows' integer statistics are summed on rank 0 (every rank drains its windows in the same order)
+        nc = cona[0]
+        nwc = Nt // nc
+        print(' *** --connect: %d regions of %s in %s, %d samples of %d records' % (nreg, cona[2], cona[1], nwc, nc))
+        cwriter = None
+        if rank == 0:
+            cwriter = sit.ConnectivityWriter(nc_name('connectivity', vTime[0], vTime[nwc * nc]), nwc, nreg,
+                                             sit.DEFAULT_TAU_EDGES, nc * rdt / 86400., corigin=corgn)
+            writers.append(cwriter)
+
+        def connect_sink(w, st):
+            if world > 1:
+                import torch
+                t = torch.from_numpy(np.concatenate([np.ravel(st[k]) for k in sit.CONNECT_STATS]))
+                dist.reduce(t, dst=0)
+                if rank != 0:
+                    return
+                st = sit.connect.stats_dict(st['tau_edges'], st['sample_days'], st['nreg'], t.numpy())
+            cwriter.write(w, vTime[w * nc], vTime[(w + 1) * nc], st)
+        connect = dict(labels=labels, every=nc, sink=connect_sink)
+        small = False                                             # windows close inside the streaming record loop
     if small:
         nchunk = max(2, min(Nt, 48, int(256e6 // (3 * Nj * Ni * 4))))      # <= 256 MB of pinned records per slot
         res = eng.track(record, Nt, kstrt=kstrt, pos0=xPosC0, posG0=xPosG0, rec_first=z1st, chunk=nchunk,
@@ -578,7 +654,7 @@ def main():
     else:
         res = eng.track(record, Nt, kstrt=kstrt, rec_first=cut(z1st), sink=sink,
                         row_dtype='f8' if physics else args.rows, physics=physics, deform=deform,
-                        dispersion=dispersion, fsle=fsle, sample=sample)
+                        dispersion=dispersion, fsle=fsle, sample=sample, connect=connect)
     eng.close()
     for w in writers:
         w.close()

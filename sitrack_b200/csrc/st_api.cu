@@ -1378,6 +1378,49 @@ int st_sample_dev(st_ctx* c, int nF, const float* fields, int64_t plane_stride, 
     return ST_OK;
 }
 
+// ---- buoy transits between regions (st_connect.cu) ---------------------------------------------------------
+static const char* connect_check(int64_t nP, int nreg, int ntau_edges)
+{
+    if (nP < 1 || nP > INT32_MAX) return "nP must be in 1..2^31-1";
+    if (nreg < 1 || nreg > CN_MAX_REGIONS) return "nreg must be in 1..31";
+    if (ntau_edges < 1 || ntau_edges > CN_MAX_TAU_EDGES) return "ntau_edges must be in 1..512";
+    if (connect_smem(nreg) > CN_MAX_SMEM) return "the region counters need more than 48 KB of shared memory";
+    return nullptr;
+}
+
+int st_connect_state_bytes(int64_t nP, int nreg, int ntau_edges, int64_t* bytes)
+{
+    if (!bytes) return fail(nullptr, ST_EINVAL, "st_connect_state_bytes: NULL argument");
+    if (const char* why = connect_check(nP, nreg, ntau_edges))
+        return fail(nullptr, ST_EINVAL, std::string("st_connect_state_bytes: ") + why);
+    *bytes = nP * 2 * (int64_t)sizeof(int32_t);
+    return ST_OK;
+}
+
+int st_connect_dev(st_ctx* c, int Nj, int Ni, const uint8_t* labels, int nreg, int64_t nP, const int32_t* cell,
+                   const int8_t* mask, int t, int32_t* state, int ntau_edges, const double* tau_edges, int64_t* stats,
+                   void* stream)
+{
+    if (const char* why = connect_check(nP, nreg, ntau_edges))
+        return fail(c, ST_EINVAL, std::string("st_connect_dev: ") + why);
+    if (Nj < 1 || Ni < 1 || (int64_t)Nj * Ni > INT32_MAX)
+        return fail(c, ST_EINVAL, "st_connect_dev: Nj and Ni must be >= 1 with Nj*Ni < 2^31");
+    if (t < 0 || t > CN_MAX_SAMPLES) return fail(c, ST_EINVAL, "st_connect_dev: t must be in 0..65535");
+    if (!labels || !mask || !state || !tau_edges || !stats)
+        return fail(c, ST_EINVAL, "st_connect_dev: NULL argument");
+    if (!cell) {
+        if (!c) return fail(nullptr, ST_EINVAL, "st_connect_dev: cell is NULL and so is ctx (whose cells it means)");
+        if (nP != c->nP || Nj != c->Nj || Ni != c->Ni)
+            return fail(c, ST_EINVAL, "st_connect_dev: nP, Nj and Ni must match the context's cell state");
+    }
+    if ((uintptr_t)cell % 8 || (uintptr_t)state % 8 || (uintptr_t)tau_edges % 8 || (uintptr_t)stats % 8)
+        return fail(c, ST_EINVAL, "st_connect_dev: cell, state, tau_edges and stats must be 8-byte aligned");
+    if (c) CU(c, cudaSetDevice(c->device));
+    CU(c, launch_connect(nP, Nj, Ni, labels, nreg, cell ? (const int2*)cell : c->cell, mask, t, state, ntau_edges,
+                         tau_edges, stats, (cudaStream_t)stream));
+    return ST_OK;
+}
+
 // ---- projections and batched predicates (host in/out) -------------------------------------------
 #define CUS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(nullptr, e_, #call); } while (0)
 

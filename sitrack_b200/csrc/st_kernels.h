@@ -287,4 +287,19 @@ cudaError_t launch_sample(long long nP, int Nj, int Ni, const int2* cell, const 
                           const pt* T, const int8_t* tmask, const float* F, long long stride, int nF, int interp,
                           float* out, cudaStream_t st);
 
+// ---- buoy transits between regions: connectivity state and statistics (st_connect.cu) ----
+constexpr int CN_MAX_REGIONS = 31;
+constexpr int CN_MAX_TAU_EDGES = 512;
+constexpr int CN_MAX_SAMPLES = 65535;
+constexpr size_t CN_MAX_SMEM = 48 * 1024;      // dynamic shared memory a block may have without opting in
+
+// Dynamic shared memory of k_connect for R regions, and the length (int64 words) of its statistics buffer.
+size_t connect_smem(int R);
+long long connect_stats_len(int R, int ntau);
+// labels (Nj*Ni) u8; cell (nP) cell words (bit 31 stripped on read); mask (nP) the row mask of sample t; state (nP,2)
+// int32, reset when t = 0; stats (connect_stats_len) int64 is added to, never zeroed.
+cudaError_t launch_connect(long long nP, int Nj, int Ni, const uint8_t* labels, int R, const int2* cell,
+                           const int8_t* mask, int t, int32_t* state, int ntau, const double* tau_edges,
+                           int64_t* stats, cudaStream_t st);
+
 }  // namespace st

@@ -428,7 +428,7 @@ class TrackEngine:
     # -- the record loop ---------------------------------------------------------------
     def track(self, records, nrec, kstrt=0, pos0=None, posG0=None, rec_first=None, want_latlon=True,
               sink=None, chunk=None, verbose=None, row_dtype="f8", physics=None, deform=None, dispersion=None,
-              fsle=None, sample=None):
+              fsle=None, sample=None, connect=None):
         """The record loop (si3_part_tracker.py:361-496), pipelined.
 
         records: callable k -> (u, v, ic) arrays (Nj,Ni) for record index k (0-based
@@ -478,6 +478,13 @@ class TrackEngine:
         for the records that are sampled.  sink(s, {name: (nP,) f4}) in the caller's buoy order (called before the
         row sink of the same row), or with sink None {name: (nsample, nP) f4} under "sample".  "bilinear" needs tyx,
         the T-points [km].  Not with the chunked season path either.
+        connect = dict(labels=(Nj,Ni) region map, every=n, tau_edges=None, sink=callable or None), combinable with all
+        of the above: buoy transits between the regions 1..R of the label map (sitrack_b200.connect, DESIGN.md section
+        16) at the rows s*n, from the host cells on the device; each buoy's state {status, src, prev, start, visited}
+        stays on the device for the whole run, and only each window's integer statistics (the events of sample w+1,
+        window 0 also the starts of row 0, and the count snapshot of sample w+1) reach the host: sink(w, stats), or
+        with sink None the list of them under "connect".  They do not depend on the order the buoys are stored in.  At
+        most MAX_SAMPLES windows; not with the chunked season path either.
         """
         torch = _torch()
         dev = torch.device("cuda", self.device)
@@ -494,11 +501,11 @@ class TrackEngine:
                 raise ValueError("physics modes write f8 rows")
             chunk = None
         if chunk and chunk > 1 and sink is None:
-            if deform is not None or dispersion is not None or fsle is not None or sample is not None:
-                raise ValueError("deform, dispersion, fsle and sample run on the streaming record loop: not with chunk > 1 "
-                                 "and sink=None")
+            if any(a is not None for a in (deform, dispersion, fsle, sample, connect)):
+                raise ValueError("deform, dispersion, fsle, sample and connect run on the streaming record loop: not with "
+                                 "chunk > 1 and sink=None")
             return self._track_chunked(get, nrec, kstrt, pos0, posG0, rec_first, want_latlon, int(chunk), rdt)
-        specs = ((_deform_run, deform), (_dispersion_run, dispersion), (_fsle_run, fsle))
+        specs = ((_deform_run, deform), (_dispersion_run, dispersion), (_fsle_run, fsle), (_connect_run, connect))
         wrows = None if all(spec is None for _, spec in specs) and sample is None else \
             _WindowRows(self, torch, rec_first, kstrt, row_f4=rdt == torch.float32)
         runs = [run(self, torch, dev, spec, wrows, nrec) for run, spec in specs if spec is not None]
@@ -724,12 +731,28 @@ def _fsle_run(eng, torch, dev, spec, rows, nrec):
     return _WindowRun(eng, torch, dev, rows, every, nrec, 1, [("fsle", spec.get("sink"), plan)])
 
 
+def _connect_run(eng, torch, dev, spec, rows, nrec):
+    """track(connect=...): one sample per window from the context's cells and the closing row's mask; no origin ring
+    (lags = 0), row 0 is evaluated by the plan's start() before step 0."""
+    from . import connect as K
+    from . import fsle as F
+    every = _window_every(spec, "connect")
+    if nrec // every > F.MAX_SAMPLES:
+        raise ValueError("connect: %d windows, more than the %d samples a run may have" % (nrec // every, F.MAX_SAMPLES))
+    labels, R = K.check_labels(spec["labels"], eng.Nj, eng.Ni)
+    plan = K._Plan(torch, dev, labels, R, eng.Nj, eng.Ni, eng.nP, spec.get("tau_edges"),
+                   sample_days=every * eng.rdt / 86400.0)
+    return _WindowRun(eng, torch, dev, rows, every, nrec, 0, [("connect", spec.get("sink"), plan)])
+
+
 class _WindowRun:
     """The windows of one analysis of track(): a ring of origin rows on the device, its passes when a window closes,
     their outputs to the host on the output stream.
 
     passes: [(result key, sink or None, plan)]; a plan has outputs(pin), window(ctx, origins, yx1, m1, dt_days, outs,
-    stream) and results(host outs) -> the sink's arguments after the window index.  Origin row o (= row o*every)
+    stream) and results(host outs) -> the sink's arguments after the window index, and may have start(ctx, m0, outs,
+    stream), called once with window 0's outputs on torch's current stream when the run is set up (row 0's cells are
+    gone by the time window 0 closes).  With lags = 0 there is no ring and no closing-row copy.  Origin row o (= row o*every)
     lives in ring slot o % nslot, nslot = min(lags, windows) (row 0 in slot 0, as _WindowRows gives it).  When window
     w closes every pass reads the origins w+1-l, l = 1 .. min(lags, w+1), on the compute stream; only after them is
     the closing row, origin w+1, copied into slot (w+1) % nslot, the slot of origin w+1-lags that they have just read
@@ -742,14 +765,19 @@ class _WindowRun:
         self.every, self.lags = every, lags
         self.dt = every * eng.rdt / 86400.0
         self.nwin = nrec // every
-        nslot = max(1, min(lags, self.nwin))
+        nslot = max(1, min(lags, self.nwin)) if lags else 0
         nP = eng.nP
         # slot 0: row 0 (on torch's current stream; track's streams wait for it)
         self.r_yx = [rows.state_pos.clone()] + [torch.empty((nP, 2), dtype=torch.float64, device=dev)
-                                                 for _ in range(nslot - 1)]
+                                                 for _ in range(nslot - 1)] if nslot else []
         self.r_mk = [torch.from_numpy(rows.m0).to(dev)] + [torch.empty((nP,), dtype=torch.int8, device=dev)
-                                                           for _ in range(nslot - 1)]
+                                                           for _ in range(nslot - 1)] if nslot else []
         self.d_out = [[plan.outputs() for _, _, plan in passes] for _ in range(2)]
+        starts = [(plan, outs) for (_, _, plan), outs in zip(passes, self.d_out[0]) if hasattr(plan, "start")]
+        if starts:
+            self.m0 = self.r_mk[0] if nslot else torch.from_numpy(rows.m0).to(dev)
+            for plan, outs in starts:
+                plan.start(self.ctx, self.m0, outs, torch.cuda.current_stream(dev))
         self.h_out = [[plan.outputs(pin=True) for _, _, plan in passes] for _ in range(2)]
         self.collected = {key: [] for key, sink, _ in passes if sink is None}
         self.ev_out = []
@@ -768,7 +796,7 @@ class _WindowRun:
                    for l in range(1, min(self.lags, w + 1) + 1)]
         for (_, _, plan), outs in zip(self.passes, self.d_out[b]):
             plan.window(self.ctx, origins, yx, mk_row, self.dt, outs, s_cmp)
-        if w + 1 < self.nwin:
+        if n and w + 1 < self.nwin:
             with torch.cuda.stream(s_cmp):                          # after the passes that read the slot last
                 self.r_yx[(w + 1) % n].copy_(yx)
                 self.r_mk[(w + 1) % n].copy_(mk_row)

@@ -25,7 +25,8 @@ from .util import epoch2clock as e2c
 __all__ = ["tunits_default", "FillValue", "GetModelGrid", "GetModelUVGrid", "GetSeedMask",
            "GetModelSeaIceConc", "ncSaveCloudBuoys", "LoadNCtime", "LoadNCdata", "SeedFileTimeInfo",
            "ModelFileTimeInfo", "open_dataset", "CloudBuoyWriter", "DeformationWriter",
-           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter", "FsleWriter", "SampleWriter"]
+           "DeformationScalingWriter", "DeformationGridWriter", "DispersionWriter", "FsleWriter", "SampleWriter",
+           "ConnectivityWriter"]
 
 tunits_default = 'seconds since 1970-01-01 00:00:00'     # ncio.py:15
 FillValue = -9999.                                       # ncio.py:19
@@ -502,6 +503,51 @@ class SampleWriter(_OutFile):
         self._v['time'][js] = time
         for n in self.names:
             self._v[n][js, :] = np.asarray(values[n], 'f4')
+
+
+class ConnectivityWriter(_OutFile):
+    """Window-by-window writer of the buoy connectivity between regions (sitrack_b200.connect, TrackEngine.track's
+    `connect`).  Dimensions time (windows), region (R+1: 0 = in no region, then 1..R), dest (R: regions 1..R),
+    tau_bin and tau_edge; variables
+      time_start, time_end (time) i4                 first and last date of each window [tunits]
+      tau_edges (tau_edge) f8                        first-arrival time histogram edges [sample]
+      n_start, n_end (time,region) i8                buoys that started / ended, by source region
+      count (time,region,region) i8                  started buoys by [source][current region] at the window's
+                                                     closing sample: a SNAPSHOT, not a sum
+      trans (time,region,region) i8                  transitions [previous][current region] between consecutive samples
+      n_arrive (time,region,dest) i8                 first arrivals [source][destination]
+      sum_tau, sum_tau2 (time,region,dest) i8        sums of their arrival times [sample] and of their squares [sample2]
+      hist_tau (time,region,dest,tau_bin) i8         counts of the arrival times per bin
+    with `units` on every variable and the global attribute sample_days (the length of one sample in days).  Every
+    variable but count is a sum over the window's sample (window 0 also holds the starts of row 0), so that windows
+    add up to the run; no variable has a fill value.  netCDF4 or an .npz with the same variables, `<name>_units` and
+    `sample_days` (see _OutFile)."""
+
+    VARS = (("n_start", ('region',), "1"), ("n_end", ('region',), "1"), ("count", ('region', 'region'), "1"),
+            ("trans", ('region', 'region'), "1"), ("n_arrive", ('region', 'dest'), "1"),
+            ("sum_tau", ('region', 'dest'), "sample"), ("sum_tau2", ('region', 'dest'), "sample2"),
+            ("hist_tau", ('region', 'dest', 'tau_bin'), "1"))
+
+    def __init__(self, cf_out, ntime, nreg, tau_edges, sample_days, tunits=tunits_default, corigin=None):
+        tau_edges = np.asarray(tau_edges, 'f8')
+        self.ntime, R = int(ntime), int(nreg)
+        super().__init__(cf_out, 'ConnectivityWriter',
+                         dict(time=self.ntime, region=R + 1, dest=R, tau_bin=tau_edges.size + 1,
+                              tau_edge=tau_edges.size),
+                         'Connectivity of Lagrangian sea-ice buoys between regions: transitions and first-arrival times',
+                         corigin, sample_days=float(sample_days))
+        for n in ('time_start', 'time_end'):
+            self.var(n, 'i4', ('time',), units=tunits)
+        for n, dims, u in self.VARS:
+            self.var(n, 'i8', ('time',) + dims, units=u)
+        self.var('tau_edges', 'f8', ('tau_edge',), units='sample', data=tau_edges)
+
+    def write(self, jw, time_start, time_end, stats):
+        """Window jw: stats = a window's dict of sitrack_b200.RegionConnectivity / track(connect=...)."""
+        self._v['time_start'][jw] = time_start
+        self._v['time_end'][jw] = time_end
+        for n, _, _ in self.VARS:
+            self._v[n][jw] = np.asarray(stats[n], 'i8')
 
 
 def ncSaveCloudBuoys(cf_out, ptime, pIDs, pY, pX, pLat, pLon, mask=[], xtime=[],
