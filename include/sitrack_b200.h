@@ -491,6 +491,11 @@ int  st_selftest_div1000(int device, int64_t n, const double *a, double *q_fast,
  * kernel's nine-operation sequence, q_div = IEEE division, for n host pairs a/b.            */
 int  st_selftest_divide(int device, int64_t n, const double *a, const double *b, double *q_fast, double *q_div);
 
+/* The cell bits (csrc/st_advect.cu: k_cell_bits) that every cell of [2,Nj-3] x [2,Ni-3] carries, or -1 when they
+ * differ there.  With 6 (every cell a convex anticlockwise quadrangle, the usual U/V staggering) the default chained
+ * step takes them as a constant instead of reading them per buoy; the results are the same either way.             */
+int  st_cell_bits_uniform(st_ctx *ctx, int *bits);
+
 /* Diagnostics of the certified fast path of step variant 4 (csrc/st_cert.cuh).  The kernel decides the
  * U/V pick (si3_part_tracker.py:430-441) and "still inside its cell" (locate.py:49-78) from a per-cell affine
  * frame in f32 whenever the buoy is farther than proven margins from every line involved, and runs the

@@ -34,6 +34,7 @@ SIGNATURES = {
     "st_selftest_proj": (c_int, [c_int, c_int, c_i64, vp, vp, c_dbl, c_dbl, c_dbl, c_dbl]),
     "st_selftest_div1000": (c_int, [c_int, c_i64, vp, vp, vp]),
     "st_selftest_divide": (c_int, [c_int, c_i64, vp, vp, vp, vp]),
+    "st_cell_bits_uniform": (c_int, [vp, C.POINTER(c_int)]),
     "st_cert_stats": (c_int, [vp, C.POINTER(c_i64), C.POINTER(c_i64)]),
     "st_cert_frames": (c_int, [vp, vp, vp]),
     "st_selftest_cert": (c_int, [vp, c_i64, vp, vp, vp, vp]),

@@ -283,17 +283,18 @@ int st_create(st_ctx** out, int device, int Nj, int Ni, const double* Yf, const 
     c->grid.atab = c->atab;
     if (e == cudaSuccess) e = refresh_fill(c);
     if (e == cudaSuccess) {
-        int* d_bad = nullptr; int bad = 0;
+        int* d_w = nullptr; int w[3] = {0, -1, 0};                           // bad coordinates, AND and OR of the bits
         e = cudaMalloc(&c->cellbits, n);
-        if (e == cudaSuccess) e = cudaMalloc(&d_bad, sizeof(int));
-        if (e == cudaSuccess) e = cudaMemsetAsync(d_bad, 0, sizeof(int), c->stream);
-        if (e == cudaSuccess) e = launch_cell_bits(c->grid, c->cellbits, d_bad, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaMalloc(&d_w, sizeof(w));
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d_w, w, sizeof(w), cudaMemcpyHostToDevice, c->stream);
+        if (e == cudaSuccess) e = launch_cell_bits(c->grid, c->cellbits, d_w, d_w + 1, c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(w, d_w, sizeof(w), cudaMemcpyDeviceToHost, c->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        cudaFree(d_bad);
+        cudaFree(d_w);
         c->grid.cellbits = c->cellbits;
         // the orientation filter's error bound assumes km coordinates within 2^17 (inside_margin)
-        c->grid.filter_ok = (bad == 0) && !getenv("SITRACK_B200_NO_FILTER");
+        c->grid.filter_ok = (w[0] == 0) && !getenv("SITRACK_B200_NO_FILTER");
+        c->grid.cellbits_uniform = w[1] == w[2] ? w[1] : -1;
     }
     if (e != cudaSuccess) { rc = cuda_fail(nullptr, e, "st_create(projection tables, cell bits)"); st_destroy(c); return rc; }
     { const char* ev = getenv("SITRACK_B200_KERNEL"); if (ev && ev[0] == 'v' && ev[1] == '1') c->variant = 1; }
@@ -1509,6 +1510,13 @@ int st_selftest_divide(int device, int64_t n, const double* a, const double* b, 
     CUS(launch_divcore(da, db, f, r, n, 0));
     CUS(cudaMemcpy(q_fast, f, sizeof(double) * n, cudaMemcpyDeviceToHost));
     CUS(cudaMemcpy(q_div, r, sizeof(double) * n, cudaMemcpyDeviceToHost));
+    return ST_OK;
+}
+
+int st_cell_bits_uniform(st_ctx* c, int* bits)
+{
+    if (!c || !bits) return fail(c, ST_EINVAL, "st_cell_bits_uniform: ctx and bits are required");
+    *bits = c->grid.cellbits_uniform;
     return ST_OK;
 }
 

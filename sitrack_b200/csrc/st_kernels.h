@@ -20,6 +20,7 @@ struct AdvectGrid {
                                 //  -- the buoy-independent orientation of the two U/V-pick segment tests (k_cell_bits);
                                 //  bit 2 = the cell is a convex anticlockwise quadrangle with edges shorter than 1024 km
     int filter_ok;              // the grid qualifies for the orientation filter of k_advect_warp (st_create checks)
+    int cellbits_uniform;       // the bits every cell of [2,Nj-3] x [2,Ni-3] carries, -1 when they differ (st_create)
     // certified fast path (st_cert.cuh, k_cell_frames): per host cell an affine frame and two margins, 32 B
     const float4* frames;       // (2*Nj*Ni) {oy, ox, a, b}, {c, d, bf16(hin) << 16 | bf16(msep), bf16(es) << 16 | bf16(et)};
                                 // hin = -1: nothing is certified in this cell
@@ -101,7 +102,8 @@ cudaError_t launch_advect_step(const AdvectGrid& g, const float* u, const float*
 cudaError_t launch_advect_ext(const AdvectGrid& g, const float* u, const float* v, const float* ic,
                               const BuoyState& s, int jrec, const StepOut& o, int scheme, int interp, int max_hops,
                               cudaStream_t st);
-cudaError_t launch_cell_bits(const AdvectGrid& g, int8_t* bits, int* n_bad_coord, cudaStream_t st);
+// span (2 ints, preset {-1, 0}): AND and OR of the bits over the cells a live buoy can occupy
+cudaError_t launch_cell_bits(const AdvectGrid& g, int8_t* bits, int* n_bad_coord, int* span, cudaStream_t st);
 cudaError_t launch_cell_frames(const AdvectGrid& g, float4* frames, unsigned long long* stats, cudaStream_t st);
 cudaError_t launch_cert_selftest(const AdvectGrid& g, long long n, const pt* yx, const int2* cell, const float4* vel,
                                  uint8_t* flags, cudaStream_t st);

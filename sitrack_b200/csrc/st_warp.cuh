@@ -9,6 +9,8 @@
 //   * FILT 1: the inside test of the common path is an orientation filter (inside_margin, st_advect.cu) that
 //     certifies "inside" for lanes clear of every edge; the others are queued and the dense pass applies the
 //     reference's own test before walking -- the exact test runs on ~15 % of the buoys instead of all;
+//   * CB >= 0: every cell a live buoy can occupy carries the cell bits CB (st_create: cellbits_uniform), so the pick
+//     and the filter take them from the instruction stream instead of gathering g.cellbits[c] per lane;
 //   * the row-store mode is a template parameter (ROWS 0: f8 rows into local HBM; 1: f4 rows and/or
 //     remote rows of the fused all-gather; 2: f8 rows that are also the position state, see BuoyState::pos_in),
 //     so the default path carries no per-row mode branches.
@@ -29,7 +31,7 @@ __device__ __forceinline__ float4 ldg_frame(const float4* a)
     return r;
 }
 
-template <int UV, bool WIN, int ROWS, int FILT, int BLK, int MINB>
+template <int UV, bool WIN, int ROWS, int FILT, int CB, int BLK, int MINB>
 __global__ void __launch_bounds__(BLK, MINB)
 k_advect_warp(const AdvectGrid g, const float* __restrict__ u, const float* __restrict__ v,
               const float* __restrict__ ic, BuoyState s, int jrec, StepOut o, int ntiles)
@@ -80,14 +82,14 @@ k_advect_warp(const AdvectGrid g, const float* __restrict__ u, const float* __re
             pt A, B;
             { const double2 q = *reinterpret_cast<const double2*>(&qP[wid][e]); A.y = q.x; A.x = q.y; }
             { const double2 q = *reinterpret_cast<const double2*>(&qPn[wid][e]); B.y = q.x; B.x = q.y; }
-            bool out = true;
-            if (FILT) {                                           // queued as "not certainly inside": the reference's test decides
-                const int c = cc.x * g.Ni + cc.y;
-                out = !inside_quad_flat(B.y, B.x, ldg_pt(g.F, c - g.Ni - 1), ldg_pt(g.F, c - g.Ni), ldg_pt(g.F, c),
-                                       ldg_pt(g.F, c - 1));
-            }
+            const int Ni = g.Ni, c = cc.x * Ni + cc.y;
+            ST_CHECK_CELL(c, 2 * Ni + 2, g.Nj, Ni);
+            const pt bl = ldg_pt(g.F, c - Ni - 1), br = ldg_pt(g.F, c - Ni);
+            const pt ul = ldg_pt(g.F, c - 1),      ur = ldg_pt(g.F, c);
+            // queued as "not certainly inside" (FILT): the reference's test decides; the walk reuses its corners
+            const bool out = !FILT || !inside_quad_flat(B.y, B.x, bl, br, ur, ul);
             if (out) {
-                walk_cell(g, ic, A, B, cc.x, cc.y, a2);
+                walk_cell_at(g, ic, A, B, c, bl, br, ur, ul, cc.x, cc.y, a2);
                 const unsigned p = qI[wid][e];
                 if (!a2) cc.x |= ST_DEAD_BIT;
                 if (cc.x != j0 || cc.y != i0) __stcg(s.cell + p, cc);
@@ -157,7 +159,7 @@ k_advect_warp(const AdvectGrid g, const float* __restrict__ u, const float* __re
             const pt u0 = ldg_pt(g.U, c - 1),  u1 = ldg_pt(g.U, c);
             const float uL = __ldg(u + c - 1), uR = __ldg(u + c);
             const float vB = __ldg(v + c - Ni), vT = __ldg(v + c);
-            const int cb = __ldg(g.cellbits + c);                 // orientation of (ur,v0,v1) and (ur,u0,u1)
+            const int cb = CB >= 0 ? CB : __ldg(g.cellbits + c);  // orientation of (ur,v0,v1) and (ur,u0,u1)
             const bool llum1 = intersect2seg_pre(P, ur, v0, v1, cb & 1);      // si3_part_tracker.py:430
             const bool llvm1 = intersect2seg_pre(P, ur, u0, u1, cb & 2);      // :431
             zU = (double)(llum1 ? uL : uR);
@@ -171,7 +173,7 @@ k_advect_warp(const AdvectGrid g, const float* __restrict__ u, const float* __re
         Pn.y = __dadd_rn(P.y, div1000(__dmul_rn(zV, g.rdt)));
         bool in;
         if (FILT == 2 && UV == 1) in = inside_margin(Pn.y, Pn.x, bl, br, ur, ul) && convex;
-        else if (FILT) in = inside_margin(Pn.y, Pn.x, bl, br, ur, ul) && (__ldg(g.cellbits + c) & 4);   // same byte as the pick's
+        else if (FILT) in = inside_margin(Pn.y, Pn.x, bl, br, ur, ul) && ((CB >= 0 ? CB : __ldg(g.cellbits + c)) & 4);   // same byte as the pick's
         else      in = inside_quad2(Pn.y, Pn.x, bl, br, ur, ul, active);
         const bool cross = active && !in;
         pt outp = {ST_FILL, ST_FILL};

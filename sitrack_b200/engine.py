@@ -109,6 +109,13 @@ class TrackEngine:
         (straightforward A/B reference), 4 = the certified two-kernel step; see include/sitrack_b200.h."""
         check(self.L.st_set_kernel_variant(self.h, int(variant)), self.h)
 
+    def cell_bits_uniform(self):
+        """-> the cell bits every cell a live buoy can occupy carries, or -1 when they differ (6: the default chained
+        step takes them as a constant)."""
+        b = C.c_int(0)
+        check(self.L.st_cell_bits_uniform(self.h, C.byref(b)), self.h)
+        return b.value
+
     # -- diagnostics of the certified fast path (csrc/st_cert.cuh) ----------------------------
     def cert_stats(self):
         """-> (cells admitted to the certified fast path, cells examined)."""
